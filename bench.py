@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config C1..C5]      # this repo's CUDA path
     python bench.py --impl reference [...]                                       # the reference's CPU path
+    python bench.py --dump-outputs DIR [...]      # also write the outputs of the last timed step to DIR (OutputDump)
 
 The line's headline (`metric`, `value`, `e2e`, `roofline`, `cpu_baseline`) is the workload `--config` names; the default
 is C2 = BASELINE.json configs[1], the configuration the metric is quoted on:
@@ -199,6 +200,55 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": 0}
         return {"sm_mhz": float(np.median(self.samples)), "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons),
                 "samples": len(self.samples)}
+
+
+class OutputDump:
+    """--dump-outputs DIR: the arrays the timed path returned in its last step, written after the timed steps as
+    DIR/<name>.npy in float32 (the uint8 results are exact in it; the tracker's records stay float64), so that two builds
+    can be compared output for output: the inputs are seeded and identical from run to run.  The run declares up front
+    the arrays it will write, and each one may take an equal share of what TOTAL_BYTES has left.  An array larger than
+    its share keeps a fixed, seeded sample of its entries along the first axis (frames of a stack of masks, rows of an
+    image), whose positions go to DIR/<name>_index.npy (float64).
+
+    Rank 0 alone writes.  A median is the whole image at any world size; a highlight stack is rank 0's share of the
+    frames, so its sample is the same only between runs on the same number of GPUs."""
+
+    TOTAL_BYTES = 64 << 20
+
+    def __init__(self, path, names):
+        self.dir = Path(path) if path else None
+        self.pending = list(names)
+        self.written = 0
+        if self.dir is not None:
+            self.dir.mkdir(parents=True, exist_ok=True)
+
+    def add(self, name: str, arr) -> None:
+        """arr: a numpy array or a torch tensor on any device, indexed along its first axis before any copy to the host."""
+        if self.dir is None:
+            return
+        self.pending.remove(name)  # a name the run did not declare is an error: it would take a share nobody left it
+        share = (self.TOTAL_BYTES - self.written) // (len(self.pending) + 1)
+        n = arr.shape[0]
+        entry_bytes = int(np.prod(arr.shape[1:])) * (8 if arr.dtype == np.float64 else 4)
+        index = None
+        if n * entry_bytes > share:
+            k = share // (entry_bytes + 8)
+            if k < 1:
+                raise RuntimeError(f"--dump-outputs: one entry of {name} is larger than its share of {share} bytes")
+            index = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+            if hasattr(arr, "cpu"):
+                import torch
+
+                arr = arr[torch.as_tensor(index, device=arr.device)]
+            else:
+                arr = arr[index]
+        host = arr.cpu().numpy() if hasattr(arr, "cpu") else np.asarray(arr)
+        host = host.astype(np.float64 if host.dtype == np.float64 else np.float32)
+        np.save(self.dir / f"{name}.npy", host)
+        self.written += host.nbytes
+        if index is not None:
+            np.save(self.dir / f"{name}_index.npy", index.astype(np.float64))
+            self.written += index.size * 8
 
 
 def bind_near_gpu(device_index: int) -> int:
@@ -425,6 +475,7 @@ class Env:
             self.dist = dist
         self.ctx = _cabi.Context(local_rank)
         self.lib = _cabi.load()
+        self.dump = OutputDump(args.dump_outputs if rank == 0 else None, dump_names(args, world))
         self.stream = torch.cuda.ExternalStream(self.ctx.stream, device=self.dev)
 
     def barrier(self):
@@ -474,7 +525,7 @@ def push_all(E: Env, host, n0, n_rank, nelem, per_call=125):
             E.ctx.median_push_raw(host[i].ctypes.data, min(per_call, m - i), nelem)
 
 
-def median_single(E: Env, cfg, steps, warmup, sampler, e2e_steps, with_cpu, row_band=None):
+def median_single(E: Env, cfg, steps, warmup, sampler, e2e_steps, with_cpu, dump_name, row_band=None):
     """Median of a stack resident on ONE device (all frames; optionally a band of rows of every frame)."""
     torch, ctx = E.torch, E.ctx
     W, H, N = cfg["width"], cfg["height"], cfg["nframes"]
@@ -516,6 +567,11 @@ def median_single(E: Env, cfg, steps, warmup, sampler, e2e_steps, with_cpu, row_
         E.barrier()
         sampler.active = False
         launches = ctx.launch_count - l0
+    if gathered is None:
+        E.dump.add(dump_name, out[:nelem].view(nrows, W))
+    elif E.dump.dir is not None:  # the bands of all ranks, as the all-gather of the last step left them
+        bands = gathered.view(E.world, band_max)
+        E.dump.add(dump_name, torch.cat([bands[r, : shard_plan(H, r, E.world)[1] * W] for r in range(E.world)]).view(H, W))
     total_ms, kern_ms = E.max_over_ranks([ev0.elapsed_time(ev1), float(np.mean([a.elapsed_time(b) for a, b in kern]))])
     ms = kern_ms if flush is not None else total_ms / steps  # with a flush in the loop only the kernel events count
     job_mpxf = W * H * N / 1e6
@@ -591,7 +647,7 @@ def median_single(E: Env, cfg, steps, warmup, sampler, e2e_steps, with_cpu, row_
     return res
 
 
-def median_sharded(E: Env, cfg, n_rank, first_frame, total_frames, steps, warmup, sampler, e2e_steps):
+def median_sharded(E: Env, cfg, n_rank, first_frame, total_frames, steps, warmup, sampler, e2e_steps, dump_name):
     """Frame-sharded median: this rank holds frames [first_frame, first_frame + n_rank) of the stream; the job is the
     median of all `total_frames`.  One step = ShardedMedian.run: window counting (phase 4), barrier, owner kernel
     (phase 5), barrier, the undecided-element count fetched from the device, and the two-round exchange only if it is not
@@ -647,6 +703,7 @@ def median_sharded(E: Env, cfg, n_rank, first_frame, total_frames, steps, warmup
                                    "barriers_and_host_check": max(0.0, ms - p4 - p5)}
     res["barrier"] = job.barrier_kind
     result_dev = ctx.copy_to_host(job.result_ptr(), nelem)
+    E.dump.add(dump_name, result_dev.reshape(H, W))
     # ---- end to end through the host-buffer C ABI: cvvp_median_push of this rank's pinned frames, the exchange on the
     # pushed stack (cvvp_median_stack_device), the full result image back in host memory
     pinned, host, n0 = pinned_prefix(E, stack, max(n_rank, 1), nelem)
@@ -713,7 +770,7 @@ def _gather_ragged(dist, outs, mine, E):
         dist.broadcast(outs[r], src=r)
 
 
-def highlight_bench(E: Env, cfg, frames_rank, first_frame, total_frames, steps, sampler, with_cpu, traffic_file=None,
+def highlight_bench(E: Env, cfg, frames_rank, first_frame, total_frames, steps, sampler, with_cpu, dump_name, traffic_file=None,
                     frames_per_launch=None):
     """Highlight of this rank's frames [first_frame, first_frame + frames_rank) of the config's stream, resident in HBM
     (`value`, CUDA events, max over ranks) and from pinned host memory through cvvp_highlight_frames (`e2e`).  Frames
@@ -756,6 +813,7 @@ def highlight_bench(E: Env, cfg, frames_rank, first_frame, total_frames, steps, 
         E.barrier()
         sampler.active = False
         launches = ctx.launch_count - l0
+    E.dump.add(dump_name, masks.view(nfr, H, W))
     (ms,) = E.max_over_ranks([e0.elapsed_time(e1) / steps])
     # end to end from pinned host memory through cvvp_highlight_frames (bounded pinned buffers: a prefix of the frames,
     # processed ceil(n / n0) times per step when the rank's share is larger)
@@ -839,6 +897,7 @@ def frame_source_bench(E: Env, steps):
         e1.record(E.stream)
         torch.cuda.synchronize()
         launches = ctx.launch_count - l0
+    E.dump.add("frame_source_gray", dst.view(n, H, W))
     ms = e0.elapsed_time(e1) / steps
     out = {
         "metric": "megapixel-frames/sec (frame source: 1080p decoded 3-channel -> grey)", "unit": UNIT,
@@ -1000,6 +1059,7 @@ def track_e2e_bench(E: Env, nframes):
         run(noop)  # warm-up: scratch allocation, module load
         t_noop, _ = run(noop)
         t_ccl, arch_gpu = run(ccl)
+        E.dump.add("track_e2e_objects", np.array([(f, *obj) for f in sorted(arch_gpu) for obj in arch_gpu[f]], np.float64).reshape(-1, 4))
         mpx = nframes * W * H / 1e6
         out["value"] = mpx / t_ccl
         out["ms_per_frame"] = {"noop_callback": t_noop / nframes * 1e3, "ccl_tracker": t_ccl / nframes * 1e3}
@@ -1017,6 +1077,17 @@ def track_e2e_bench(E: Env, nframes):
 # ------------------------------------------------------------------------------------------------
 # the GPU arm
 # ------------------------------------------------------------------------------------------------
+def dump_names(args, world):
+    """The arrays run_gpu_arm hands to OutputDump, in its order and under its conditions."""
+    names = ["background" if CONFIGS[args.config]["kind"] == "median" else "masks"]
+    if args.config == "C2" and not args.no_highlight:
+        names += ["highlight_masks"] + (["frame_source_gray"] if world == 1 else [])
+        if not args.no_extra_configs:
+            names += ["c5_median_background", "c4_highlight_masks"]
+            names += ["track_e2e_objects"] if world == 1 and not args.no_track else []
+    return names
+
+
 def run_gpu_arm(args, rank, local_rank, world):
     E = Env(args, rank, local_rank, world)
     cfg = CONFIGS[args.config]
@@ -1027,25 +1098,26 @@ def run_gpu_arm(args, rank, local_rank, world):
     with_cpu = rank == 0 and world == 1 and not args.no_cpu_baseline
     extras = {}
 
-    def median_of(c, st, wu, e2e_steps, cpu):
+    def median_of(c, st, wu, e2e_steps, cpu, dump_name):
         if world == 1:
-            return median_single(E, c, st, wu, sampler, e2e_steps, cpu)
+            return median_single(E, c, st, wu, sampler, e2e_steps, cpu, dump_name)
         if c["scaling"] == "weak" and args.median_sharding == "rows":
-            return median_single(E, c, st, wu, sampler, e2e_steps, False, row_band=shard_plan(c["height"], rank, world))
+            return median_single(E, c, st, wu, sampler, e2e_steps, False, dump_name, row_band=shard_plan(c["height"], rank, world))
         if c["scaling"] == "weak":
-            return median_sharded(E, c, c["nframes"], c["nframes"] * rank, c["nframes"] * world, st, wu, sampler, e2e_steps)
+            return median_sharded(E, c, c["nframes"], c["nframes"] * rank, c["nframes"] * world, st, wu, sampler, e2e_steps,
+                                  dump_name)
         first, cnt = frame_chunk(c["nframes"], rank, world)
-        return median_sharded(E, c, cnt, first, c["nframes"], st, wu, sampler, e2e_steps)
+        return median_sharded(E, c, cnt, first, c["nframes"], st, wu, sampler, e2e_steps, dump_name)
 
-    def highlight_of(c, st, cpu, traffic=None):
+    def highlight_of(c, st, cpu, dump_name, traffic=None):
         first, cnt = frame_chunk(c["nframes"], rank, world)
         per = 1024 if c["width"] * c["height"] > 500_000 else 16384
-        return highlight_bench(E, c, cnt, 1000 + first, c["nframes"], st, sampler, cpu, traffic, frames_per_launch=per)
+        return highlight_bench(E, c, cnt, 1000 + first, c["nframes"], st, sampler, cpu, dump_name, traffic, frames_per_launch=per)
 
     if cfg["kind"] == "median":
-        main = median_of(cfg, steps, warmup, steps, with_cpu)
+        main = median_of(cfg, steps, warmup, steps, with_cpu, "background")
     else:
-        main = highlight_of(cfg, max(1, min(steps, 5)), with_cpu)
+        main = highlight_of(cfg, steps, with_cpu, "masks")
         main["steps_timed"] = main.pop("steps")
     clocks = sampler.summary()
     sampler.stop()
@@ -1057,7 +1129,7 @@ def run_gpu_arm(args, rank, local_rank, world):
         try:
             hl_cfg = dict(HL_STEP, nframes=HL_STEP["frames_per_gpu"] * world)
             h = highlight_bench(E, hl_cfg, HL_STEP["frames_per_gpu"], 1000 + rank * HL_STEP["frames_per_gpu"], hl_cfg["nframes"],
-                                max(3, min(steps, 10)), sampler, with_cpu,
+                                max(3, min(steps, 10)), sampler, with_cpu, "highlight_masks",
                                 "highlight_ncu_summary.json" if world == 1 else None)
             h["scaling"] = "weak"
             h["clocks"] = s2.summary()
@@ -1065,11 +1137,11 @@ def run_gpu_arm(args, rank, local_rank, world):
             if world == 1:
                 extras["frame_source"] = frame_source_bench(E, max(3, min(steps, 10)))
             if not args.no_extra_configs:
-                c5 = median_of(CONFIGS["C5"], 3, 3, 2, with_cpu)
+                c5 = median_of(CONFIGS["C5"], 3, 3, 2, with_cpu, "c5_median_background")
                 c5["metric"], c5["unit"], c5["scaling"] = metric_name(CONFIGS["C5"]), UNIT, "strong"
                 c5["config"] = job_config(CONFIGS["C5"], world, args)
                 extras["c5_median"] = c5
-                c4 = highlight_of(CONFIGS["C4"], 3, False)
+                c4 = highlight_of(CONFIGS["C4"], 3, False, "c4_highlight_masks")
                 c4["scaling"] = "strong"
                 extras["c4_highlight"] = c4
                 if world == 1 and not args.no_track:
@@ -1100,7 +1172,9 @@ def run_gpu_arm(args, rank, local_rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline workload; the extra objects of the C2 line time their own fixed "
+                         "counts (3 to 10 steps)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", choices=["cuda", "reference"], default="cuda")
     ap.add_argument("--config", choices=sorted(CONFIGS), default="C2", help="the workload of the line's headline (default: C2)")
@@ -1112,7 +1186,14 @@ def main():
     ap.add_argument("--median-sharding", choices=["frames", "rows"], default="frames",
                     help="N > 1, C2: frame chunks with the NVLink count exchange (default, weak scaling) or row bands of "
                          "the single stack with no data-path collective (strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32, at most 64 MB in "
+                         "all, shared among the arrays the run writes; larger results as a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path")
     if args.warmup < 3 and args.impl == "cuda":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))

@@ -132,3 +132,19 @@ def synthetic_case(cfg="C3", frame_index=7, scale=4):
     bg = np.sort(stack, axis=0)[31 // 2]
     frame = synth.synth_frame(frame_index, w, h, p["seed"], p["ndisks"])
     return frame, ho.canonical_params(bg)
+
+
+def reference_sha256(name):
+    """SHA-256 of the reference's own HighlightObjectsAlgo output on the case `name` (an adversarial case's name or
+    random_<t>), as tests/golden/make_highlight_golden.py stored it; None for a case it did not store."""
+    import json
+    from pathlib import Path
+
+    global _REF_SHA
+    if _REF_SHA is None:
+        golden = json.loads((Path(__file__).parent / "golden" / "highlight_golden.json").read_text())
+        _REF_SHA = {g["name"]: g["output_sha256"] for g in golden}
+    return _REF_SHA.get(name)
+
+
+_REF_SHA = None

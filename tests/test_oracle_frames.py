@@ -79,22 +79,24 @@ def test_oracle_matches_golden_and_closed_form(case):
 VIDEO_CASES = [c for c in CASES if c[1].ndim == 4 and c[1].shape[3] == 3 and c[1].shape[1] % 2 == 0]
 
 
-@needs_ref
 @pytest.mark.parametrize("case", VIDEO_CASES, ids=[c[0] for c in VIDEO_CASES])
 def test_restatement_matches_the_compiled_reference_generator(case, tmp_path):
     """CvVidFramesGeneratorAlgo::GetTokenSet (cv_vid_frames_generator_algo.h:119-189) on a lossless video of the case's
-    frames == oracle.prepare_frames on the decoded frames, and == the golden hash"""
+    frames == oracle.prepare_frames on the decoded frames, and == the golden hash, which is the generator's own output
+    (without oracle/_ref the restatement of the decoded frames is held to that hash alone)"""
     name, frames, crop, mode = case
     vid = video_util.write_lossless(tmp_path / "v.avi", frames)
-    assert np.array_equal(video_util.read_all(vid), frames)
-    toks = fref.tokens(vid, 0, len(frames), crop, mode, frames_in_batch=3)
-    want = fo.prepare_frames(frames, crop, mode)
-    assert len(toks) == len(want)
-    got = np.stack(toks)
-    assert got.dtype == np.uint8 and np.array_equal(got, want)
+    decoded = video_util.read_all(vid)
+    assert np.array_equal(decoded, frames)
+    want = fo.prepare_frames(decoded, crop, mode)
+    if fref.available():
+        toks = fref.tokens(vid, 0, len(frames), crop, mode, frames_in_batch=3)
+        assert len(toks) == len(want)
+        got = np.stack(toks)
+        assert got.dtype == np.uint8 and np.array_equal(got, want)
     g = next(e for e in GOLDEN if e["name"] == name)
     assert g["source"].startswith("reference")
-    assert hashlib.sha256(got.tobytes()).hexdigest() == g["output_sha256"]
+    assert hashlib.sha256(want.tobytes()).hexdigest() == g["output_sha256"]
 
 
 @needs_ref

@@ -48,21 +48,30 @@ def test_model_matches_cv2_adversarial(case):
     assert np.array_equal(a, b)
 
 
-@needs_ref
+def _against_reference(name, frame, p, out):
+    """out == the reference's output: the compiled reference where it was built, else its stored hash"""
+    if href.available():
+        got = href.highlight_objects(frame, p)
+        assert got.dtype == np.uint8 and got.shape == frame.shape
+        assert np.array_equal(got, out)
+        return
+    sha = hl_cases.reference_sha256(name)
+    if sha is None:
+        pytest.skip(f"oracle/_ref/cvvp_highlight_ref was not built and no output of the reference is stored for {name}")
+    assert hashlib.sha256(out.tobytes()).hexdigest() == sha
+
+
 @pytest.mark.parametrize("t", range(120))
 def test_restatement_matches_the_compiled_reference_random(t):
     """HighlightObjectsAlgo::Insert -> TryGetResult of the reference's own source == oracle.highlight_objects"""
     frame, p = hl_cases.random_case(t)
-    got = href.highlight_objects(frame, p)
-    assert got.dtype == np.uint8 and got.shape == frame.shape
-    assert np.array_equal(got, ho.highlight_objects(frame.copy(), p))
+    _against_reference(f"random_{t}", frame, p, ho.highlight_objects(frame.copy(), p))
 
 
-@needs_ref
 @pytest.mark.parametrize("case", ADV, ids=[c[0] for c in ADV])
 def test_restatement_matches_the_compiled_reference_adversarial(case):
-    _, frame, p = case
-    assert np.array_equal(href.highlight_objects(frame, p), ho.highlight_objects(frame.copy(), p))
+    name, frame, p = case
+    _against_reference(name, frame, p, ho.highlight_objects(frame.copy(), p))
 
 
 @needs_ref

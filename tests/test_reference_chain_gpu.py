@@ -5,6 +5,8 @@ oracle/_ref (built from /root/reference where it is mounted, shipped with the sn
     cvvp_frames_ref         CvVidFramesGeneratorAlgo      cv_vid_frames_generator_algo.h   (cv:: -> cv2 shim)
 -- chained the way the reference chains them (generator tokens -> median; generator tokens + background -> highlight
 -> callback), held against the C ABI and against the drop-in Python surface."""
+import hashlib
+
 import cv2
 import numpy as np
 import pytest
@@ -18,8 +20,8 @@ from oracle import frames_ref as fref
 from oracle import highlight_oracle as ho
 from oracle import highlight_ref as href
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not (href.available() and fref.available()), reason="oracle/_ref was not built")]
+pytestmark = pytest.mark.gpu
+needs_ref = pytest.mark.skipif(not (href.available() and fref.available()), reason="oracle/_ref was not built")
 
 ADV = hl_cases.adversarial_cases()
 
@@ -33,21 +35,38 @@ def _gpu_masks(ctx, frames, p):
         ctx.highlight_end()
 
 
+def _is_reference_output(name, frame, p, got):
+    """the compiled reference where it was built, else the stored hash of its output; None: neither is there"""
+    if href.available():
+        return np.array_equal(got, href.highlight_objects(frame, p))
+    sha = hl_cases.reference_sha256(name)
+    return None if sha is None else hashlib.sha256(np.ascontiguousarray(got).tobytes()).hexdigest() == sha
+
+
 @pytest.mark.parametrize("case", ADV, ids=[c[0] for c in ADV])
 def test_highlight_adversarial_cases_against_the_compiled_reference(gpu_ctx, case):
-    _, frame, p = case
+    name, frame, p = case
     got = _gpu_masks(gpu_ctx, frame[None], p)[0]
-    assert np.array_equal(got, href.highlight_objects(frame, p))
+    same = _is_reference_output(name, frame, p, got)
+    if same is None:
+        pytest.skip(f"oracle/_ref was not built and no output of the reference is stored for {name}")
+    assert same
 
 
 @pytest.mark.parametrize("t0", range(0, 120, 20))
 def test_highlight_random_cases_against_the_compiled_reference(gpu_ctx, t0):
+    checked = 0
     for t in range(t0, t0 + 20):
         frame, p = hl_cases.random_case(t)
         got = _gpu_masks(gpu_ctx, frame[None], p)[0]
-        assert np.array_equal(got, href.highlight_objects(frame, p)), f"random case {t}"
+        same = _is_reference_output(f"random_{t}", frame, p, got)
+        assert same is not False, f"random case {t}"
+        checked += same is not None
+    if not checked:
+        pytest.skip(f"oracle/_ref was not built and no output of the reference is stored for random cases {t0}..{t0 + 19}")
 
 
+@needs_ref
 @pytest.mark.parametrize("cfg,count", [("C3", 12), ("C4", 200)])
 def test_highlight_of_the_benchmark_streams_against_the_compiled_reference(gpu_ctx, cfg, count):
     """frames of the C3 (1080p) and C4 (512x256) streams at full size, canonical parameters, one batch on the device;
@@ -78,6 +97,7 @@ def colour_stream(tmp_path_factory):
     return path, frames
 
 
+@needs_ref
 @pytest.mark.parametrize("mode", ["grayscale", "vid_is_grayscale"])
 def test_the_whole_path_against_the_reference_chain(colour_stream, ref_median, mode):
     """GetVideoBackground and TrackObjects of the drop-in module on a cropped colour video against the chain of
@@ -125,6 +145,7 @@ def test_the_whole_path_against_the_reference_chain(colour_stream, ref_median, m
         assert white > (last - start) // 2
 
 
+@needs_ref
 def test_median_c_abi_against_the_reference_class_on_generator_tokens(gpu_ctx, colour_stream, ref_median):
     """the C ABI's frame source + median (cvvp_median_push_source) against generator tokens -> reference median"""
     if ref_median is None:
@@ -142,6 +163,7 @@ def test_median_c_abi_against_the_reference_class_on_generator_tokens(gpu_ctx, c
         assert np.array_equal(got, want), (crop, mode)
 
 
+@needs_ref
 def test_get_video_background_equals_the_reference_entry_point(colour_stream, tmp_path, capfd):
     """The drop-in claim at the public entry point: the reference's own GetVideoBackground -- cv_vid_bg_helpers.cpp with
     the whole AsyncTokens pipeline behind it, compiled unmodified (oracle/_ref/cvvp_background_ref; run in a child
