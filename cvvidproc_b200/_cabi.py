@@ -66,12 +66,21 @@ def load():
         "cvvp_median_abort": (i32, [vp]),
         "cvvp_median_device": (i32, [vp, vp, i64, sz, sz, vp, vp]),
         "cvvp_median_last_kernel_ms": (i32, [vp, C.POINTER(C.c_float)]),
+        "cvvp_median_rolling_device": (i32, [vp, vp, i64, sz, sz, i32, i64, i64, vp, sz, vp]),
         "cvvp_highlight_begin": (i32, [vp, vp, i32, i32, vp, i32, i32, i32, i32, i32, i32, i32, i32]),
         "cvvp_highlight_frames": (i32, [vp, vp, i64, sz, vp, sz]),
         "cvvp_highlight_device": (i32, [vp, vp, i64, sz, vp, sz, vp]),
         "cvvp_highlight_end": (i32, [vp]),
         "cvvp_highlight_device_cc": (i32, [vp, vp, i64, sz, vp, sz, vp, i32, vp, vp, sz, vp]),
         "cvvp_highlight_frames_cc": (i32, [vp, vp, i64, sz, vp, sz, vp, i32, vp, vp, sz]),
+        "cvvp_highlight_device_bg": (i32, [vp, vp, i64, sz, vp, sz, vp, sz, vp, i32, vp, vp, sz, vp]),
+        "cvvp_highlight_rolling_begin": (i32, [vp, i32, i64, vp, i32, i32]),
+        "cvvp_highlight_rolling_push": (i32, [vp, vp, i64, sz]),
+        "cvvp_highlight_rolling_close": (i32, [vp]),
+        "cvvp_highlight_rolling_pending": (i32, [vp]),
+        "cvvp_highlight_rolling_ready": (i32, [vp]),
+        "cvvp_highlight_rolling_next": (i32, [vp, vp, sz, i64, C.POINTER(i64), C.POINTER(i64), vp, vp, vp, sz]),
+        "cvvp_highlight_rolling_end": (i32, [vp]),
         "cvvp_highlight_set_path": (i32, [vp, i32]),
         "cvvp_highlight_frames_in_flight": (i32, [vp, C.POINTER(i32)]),
         "cvvp_synth_frames_device": (i32, [vp, vp, sz, i32, i32, i32, i32, i64, i64, u32, i32, vp]),
@@ -313,6 +322,12 @@ class Context:
     def median_device(self, d_frames: int, nframes: int, nelem: int, frame_stride: int, d_out: int, stream: int = 0):
         self._check(self._lib.cvvp_median_device(self._h, d_frames, nframes, nelem, frame_stride, d_out, stream or None))
 
+    def median_rolling_device(self, d_frames: int, nframes: int, nelem: int, frame_stride: int, window: int, t0: int,
+                              t1: int, d_out: int, out_stride: int, stream: int = 0):
+        """backgrounds of frames [t0, t1): the upper median of each frame's centred window of `window` frames"""
+        self._check(self._lib.cvvp_median_rolling_device(self._h, d_frames, nframes, nelem, frame_stride, window, t0, t1,
+                                                         d_out, out_stride, stream or None))
+
     def median_last_kernel_ms(self) -> float:
         v = C.c_float()
         self._check(self._lib.cvvp_median_last_kernel_ms(self._h, C.byref(v)))
@@ -484,6 +499,67 @@ class Context:
 
     def highlight_device(self, d_frames: int, n: int, frame_stride: int, d_out: int, out_stride: int, stream: int = 0):
         self._check(self._lib.cvvp_highlight_device(self._h, d_frames, n, frame_stride, d_out, out_stride, stream or None))
+
+    def highlight_device_bg(self, d_frames: int, n: int, frame_stride: int, d_backgrounds: int, bg_stride: int, d_out: int,
+                            out_stride: int, d_comps: int = 0, max_comps: int = 0, d_ncomps: int = 0, d_labels: int = 0,
+                            labels_stride: int = 0, stream: int = 0):
+        """frame f against its own background at d_backgrounds + f * bg_stride (0: one background for all)"""
+        self._check(self._lib.cvvp_highlight_device_bg(self._h, d_frames, n, frame_stride, d_backgrounds, bg_stride, d_out,
+                                                       out_stride, d_comps or None, max_comps, d_ncomps or None,
+                                                       d_labels or None, labels_stride, stream or None))
+
+    # rolling-median background stream (cvvp_highlight_rolling_*): masks come back later than their frames go in
+    def highlight_rolling_begin(self, window: int, max_batch: int, fmt: FrameFormat | None = None, max_comps: int = 0,
+                                labels: bool = False):
+        self._check(self._lib.cvvp_highlight_rolling_begin(self._h, window, max_batch,
+                                                           C.byref(fmt) if fmt is not None else None, max_comps,
+                                                           1 if labels else 0))
+        self._hr = (max_batch, max_comps, bool(labels))
+
+    def highlight_rolling_push(self, frames: np.ndarray):
+        """frames: uint8 (n, ...) -- prepared (n, H, W) frames, or decoded frames when the stream has a format"""
+        frames = np.ascontiguousarray(frames)
+        if frames.dtype != np.uint8:
+            raise TypeError("frames must be uint8")
+        self._check(self._lib.cvvp_highlight_rolling_push(self._h, frames.ctypes.data, frames.shape[0],
+                                                          int(np.prod(frames.shape[1:]))))
+
+    def highlight_rolling_close(self):
+        self._check(self._lib.cvvp_highlight_rolling_close(self._h))
+
+    def highlight_rolling_pending(self) -> int:
+        return int(self._lib.cvvp_highlight_rolling_pending(self._h))
+
+    def highlight_rolling_ready(self) -> bool:
+        rc = self._lib.cvvp_highlight_rolling_ready(self._h)
+        if rc < 0:
+            self._check(rc)
+        return rc == 1
+
+    def highlight_rolling_next(self):
+        """-> (first frame index, masks (n, H, W)[, comps (n, max_comps), ncomps (n,)[, labels (n, H, W)]]); n = 0 when
+        nothing is pending"""
+        max_batch, max_comps, labels = self._hr
+        h, w = self._hl_shape
+        out = np.empty((max_batch, h, w), np.uint8)
+        comps = np.zeros((max_batch, max_comps), self.COMPONENT_DTYPE) if max_comps else None
+        ncomps = np.zeros(max_batch, np.int32) if max_comps else None
+        lab = np.zeros((max_batch, h, w), np.int32) if labels else None
+        first, n = C.c_longlong(0), C.c_longlong(0)
+        self._check(self._lib.cvvp_highlight_rolling_next(self._h, out.ctypes.data, h * w, max_batch, C.byref(first),
+                                                          C.byref(n), comps.ctypes.data if max_comps else None,
+                                                          ncomps.ctypes.data if max_comps else None,
+                                                          lab.ctypes.data if labels else None, h * w))
+        k = int(n.value)
+        res = (int(first.value), out[:k])
+        if max_comps:
+            res += (comps[:k], ncomps[:k])
+        if labels:
+            res += (lab[:k],)
+        return res
+
+    def highlight_rolling_end(self):
+        self._check(self._lib.cvvp_highlight_rolling_end(self._h))
 
     def highlight_set_path(self, path: int):
         """0 = fused kernel (default), 1 = per-pixel kernels (on-device cross-check)"""

@@ -421,6 +421,7 @@ void cvvp_ctx_destroy(cvvp_ctx *ctx)
             cudaFreeHost(b.host);
     }
     highlight_queue_release(ctx);
+    highlight_rolling_release(ctx);
     highlight_release(ctx);
     raw_stage_release(ctx);
     median_shard_release(ctx);
@@ -742,6 +743,16 @@ int cvvp_median_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes
     return median_launch(ctx, d_frames, nframes, nelem, frame_stride, d_out, s);
 }
 
+int cvvp_median_rolling_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
+                               int window, long long t0, long long t1, uint8_t *d_out, size_t out_stride, void *stream)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->compute;
+    return median_roll_launch(ctx, d_frames, nframes, frame_stride, nframes, nelem, window, t0, t1, d_out, out_stride, s);
+}
+
 int cvvp_median_last_kernel_ms(cvvp_ctx *ctx, float *out_ms)
 {
     if (!ctx || !out_ms)
@@ -766,6 +777,7 @@ int cvvp_highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, in
     (void)width_border; // accepted and unused, exactly like the reference (FrameAndFill is dead code, :68-71)
     DeviceGuard guard(ctx->device);
     highlight_queue_release(ctx);
+    highlight_rolling_release(ctx);
     return highlight_begin(ctx, background, width, height, struct_element, kw, kh, threshold, threshold_lo, threshold_hi,
                            min_size_hyst, min_size_threshold);
 }
@@ -801,6 +813,19 @@ int cvvp_highlight_device_cc(cvvp_ctx *ctx, const uint8_t *d_frames, long long n
                                labels_stride, s);
 }
 
+int cvvp_highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride,
+                             const uint8_t *d_backgrounds, size_t bg_stride, uint8_t *d_out, size_t out_stride,
+                             cvvp_component *d_comps, int max_comps, int *d_ncomps, int32_t *d_labels, size_t labels_stride,
+                             void *stream)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->compute;
+    return highlight_device_bg(ctx, d_frames, n, frame_stride, d_backgrounds, bg_stride, d_out, out_stride, d_comps, max_comps,
+                               d_ncomps, d_labels, labels_stride, s);
+}
+
 int cvvp_highlight_frames_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, uint8_t *masks_out,
                              size_t out_stride, cvvp_component *comps_out, int max_comps, int *ncomps_out,
                              int32_t *labels_out, size_t labels_stride)
@@ -821,6 +846,7 @@ int cvvp_highlight_end(cvvp_ctx *ctx)
     cudaStreamSynchronize(ctx->compute);
     cudaStreamSynchronize(ctx->copy_out);
     highlight_queue_release(ctx);
+    highlight_rolling_release(ctx);
     highlight_release(ctx);
     return CVVP_OK;
 }
@@ -959,6 +985,64 @@ int cvvp_highlight_queue_end(cvvp_ctx *ctx)
         return fail(nullptr, CVVP_ERR_INVALID, "null context");
     DeviceGuard guard(ctx->device);
     highlight_queue_release(ctx);
+    return CVVP_OK;
+}
+
+int cvvp_highlight_rolling_begin(cvvp_ctx *ctx, int window, long long max_batch, const cvvp_frame_format *fmt, int max_comps,
+                                 int labels)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    return highlight_rolling_begin(ctx, window, max_batch, fmt, max_comps, labels);
+}
+
+int cvvp_highlight_rolling_push(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    return highlight_rolling_push(ctx, frames, n, frame_stride);
+}
+
+int cvvp_highlight_rolling_close(cvvp_ctx *ctx)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    return highlight_rolling_close(ctx);
+}
+
+int cvvp_highlight_rolling_pending(const cvvp_ctx *ctx)
+{
+    return ctx ? highlight_rolling_pending(ctx) : 0;
+}
+
+int cvvp_highlight_rolling_ready(cvvp_ctx *ctx)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    return highlight_rolling_ready(ctx);
+}
+
+int cvvp_highlight_rolling_next(cvvp_ctx *ctx, uint8_t *masks_out, size_t out_stride, long long max_n, long long *first_index,
+                                long long *n_out, cvvp_component *comps_out, int *ncomps_out, int32_t *labels_out,
+                                size_t labels_stride)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    return highlight_rolling_next(ctx, masks_out, out_stride, max_n, first_index, n_out, comps_out, ncomps_out, labels_out,
+                                  labels_stride);
+}
+
+int cvvp_highlight_rolling_end(cvvp_ctx *ctx)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    DeviceGuard guard(ctx->device);
+    highlight_rolling_release(ctx);
     return CVVP_OK;
 }
 

@@ -80,6 +80,7 @@ struct RawStage {
     size_t out_cap{0};
 };
 struct HighlightQueue; // frame_pipeline.cu
+struct RollingStream;  // highlight_rolling.cu
 } // namespace cvvp
 
 struct cvvp_ctx {
@@ -106,6 +107,7 @@ struct cvvp_ctx {
     size_t staging_next{0};
     cvvp::RawStage raw;
     cvvp::HighlightQueue *hq{nullptr};
+    cvvp::RollingStream *hr{nullptr};
 };
 
 namespace cvvp
@@ -171,6 +173,10 @@ int highlight_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t
 int highlight_device_cc(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, uint8_t *d_out,
                         size_t out_stride, cvvp_component *d_comps, int max_comps, int *d_ncomps, int32_t *d_labels,
                         size_t labels_stride, cudaStream_t stream);
+// per-frame backgrounds (frame f's at d_bgs + f * bg_stride, 0 = one for all); components when d_comps != nullptr
+int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, const uint8_t *d_bgs,
+                        size_t bg_stride, uint8_t *d_out, size_t out_stride, cvvp_component *d_comps, int max_comps,
+                        int *d_ncomps, int32_t *d_labels, size_t labels_stride, cudaStream_t stream);
 int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, uint8_t *masks_out,
                              size_t out_stride, cvvp_component *comps_out, int max_comps, int *ncomps_out,
                              int32_t *labels_out, size_t labels_stride);
@@ -202,6 +208,21 @@ int highlight_slot_commit(cvvp_ctx *ctx, long long n);
 int highlight_queue_next_view(cvvp_ctx *ctx, const uint8_t **h_masks, size_t *mask_pitch, long long *n_out,
                               const cvvp_component **comps, const int **ncomps);
 int highlight_queue_view_release(cvvp_ctx *ctx);
+// median_roll.cu: backgrounds of outputs [t0, t1) of a rolling-window median; frame i at d_frames + (i % ring) * stride
+int median_roll_launch(cvvp_ctx *ctx, const uint8_t *d_frames, long long ring, size_t frame_stride, long long nframes,
+                       size_t nelem, int window, long long t0, long long t1, uint8_t *d_out, size_t out_stride,
+                       cudaStream_t stream);
+// highlight_rolling.cu
+void highlight_rolling_release(cvvp_ctx *ctx);
+int highlight_rolling_begin(cvvp_ctx *ctx, int window, long long max_batch, const cvvp_frame_format *fmt, int max_comps,
+                            int labels);
+int highlight_rolling_push(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride);
+int highlight_rolling_close(cvvp_ctx *ctx);
+int highlight_rolling_pending(const cvvp_ctx *ctx);
+int highlight_rolling_ready(cvvp_ctx *ctx);
+int highlight_rolling_next(cvvp_ctx *ctx, uint8_t *masks_out, size_t out_stride, long long max_n, long long *first_index,
+                           long long *n_out, cvvp_component *comps_out, int *ncomps_out, int32_t *labels_out,
+                           size_t labels_stride);
 // highlight.cu: geometry of the running job (false: no job)
 bool highlight_geometry(const cvvp_ctx *ctx, int *width, int *height);
 // synth.cu

@@ -73,15 +73,15 @@ __device__ __forceinline__ void uf_union(uint32_t *lab, uint32_t a, uint32_t b)
 // K1: difference + the three thresholds
 // ------------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
-    diff_thresh_kernel(const uint8_t *__restrict__ frames, size_t frame_stride, const uint8_t *__restrict__ bg, HlGeom g,
-                       const int *__restrict__ th_a, int lo, int hi, uint8_t *__restrict__ diff,
+    diff_thresh_kernel(const uint8_t *__restrict__ frames, size_t frame_stride, const uint8_t *__restrict__ bg,
+                       size_t bg_stride, HlGeom g, const int *__restrict__ th_a, int lo, int hi, uint8_t *__restrict__ diff,
                        uint8_t *__restrict__ mask_a, uint8_t *__restrict__ mask_u, uint8_t *__restrict__ mask_l)
 {
     const uint32_t f = blockIdx.z;
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= g.npix)
         return;
-    const int d = max(int(bg[p]) - int(frames[size_t(f) * frame_stride + p]), 0);
+    const int d = max(int(bg[size_t(f) * bg_stride + p]) - int(frames[size_t(f) * frame_stride + p]), 0);
     const size_t o = size_t(f) * g.mstride + p;
     if (diff)
         diff[o] = uint8_t(d);
@@ -92,15 +92,15 @@ __global__ void __launch_bounds__(256)
 
 // 256-bin histogram of the difference image (only for threshold == -1, Otsu)
 __global__ void __launch_bounds__(256)
-    diff_hist_kernel(const uint8_t *__restrict__ frames, size_t frame_stride, const uint8_t *__restrict__ bg, HlGeom g,
-                     unsigned int *__restrict__ hist)
+    diff_hist_kernel(const uint8_t *__restrict__ frames, size_t frame_stride, const uint8_t *__restrict__ bg,
+                     size_t bg_stride, HlGeom g, unsigned int *__restrict__ hist)
 {
     __shared__ unsigned int sh[256];
     const uint32_t f = blockIdx.z;
     sh[threadIdx.x] = 0;
     __syncthreads();
     for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < g.npix; p += gridDim.x * blockDim.x) {
-        const int d = max(int(bg[p]) - int(frames[size_t(f) * frame_stride + p]), 0);
+        const int d = max(int(bg[size_t(f) * bg_stride + p]) - int(frames[size_t(f) * frame_stride + p]), 0);
         atomicAdd(&sh[d], 1u);
     }
     __syncthreads();
@@ -689,8 +689,8 @@ static int ensure_batch(cvvp_ctx *ctx, HighlightState *st, int nb)
 }
 
 // per-frame thresholds of branch A for nb frames -> st->d_th: the constant, or Otsu's per frame (threshold == -1, :89-95)
-int highlight_thresholds(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, unsigned nb,
-                         cudaStream_t stream)
+int highlight_thresholds(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
+                         size_t bg_stride, unsigned nb, cudaStream_t stream)
 {
     if (int(nb) > st->th_cap) {
         // the previous arrays may still be in use by work queued on `stream`
@@ -707,7 +707,7 @@ int highlight_thresholds(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, s
     }
     if (st->th == -1) {
         cudaMemsetAsync(st->d_hist, 0, size_t(nb) * 256 * sizeof(unsigned int), stream);
-        diff_hist_kernel<<<dim3(64, 1, nb), 256, 0, stream>>>(in, frame_stride, st->d_bg, st->g, st->d_hist);
+        diff_hist_kernel<<<dim3(64, 1, nb), 256, 0, stream>>>(in, frame_stride, bg, bg_stride, st->g, st->d_hist);
         otsu_kernel<<<(nb + 63) / 64, 64, 0, stream>>>(st->d_hist, st->g.npix, st->d_th, int(nb));
         ctx->launches += 2;
     } else {
@@ -730,7 +730,7 @@ static int pick_batch(const HighlightState *st, long long n)
 }
 
 static int highlight_pixels(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_frames, long long n, size_t frame_stride,
-                            uint8_t *d_out, size_t out_stride, cudaStream_t stream)
+                            const uint8_t *d_bg, size_t bg_stride, uint8_t *d_out, size_t out_stride, cudaStream_t stream)
 {
     const int bcap = pick_batch(st, n);
     int rc = ensure_batch(ctx, st, bcap);
@@ -739,11 +739,12 @@ static int highlight_pixels(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_
     for (long long done = 0; done < n; done += bcap) {
         const unsigned nb = unsigned(n - done < bcap ? n - done : bcap);
         const uint8_t *in = d_frames + size_t(done) * frame_stride;
+        const uint8_t *bg = d_bg + size_t(done) * bg_stride;
         Launcher L{ctx, stream, st->g, nb};
-        if ((rc = highlight_thresholds(ctx, st, in, frame_stride, nb, stream)) != CVVP_OK)
+        if ((rc = highlight_thresholds(ctx, st, in, frame_stride, bg, bg_stride, nb, stream)) != CVVP_OK)
             return rc;
-        diff_thresh_kernel<<<L.per_pixel(), 256, 0, stream>>>(in, frame_stride, st->d_bg, st->g, st->d_th, st->lo, st->hi,
-                                                              nullptr, st->m_a, st->m_u, st->m_l);
+        diff_thresh_kernel<<<L.per_pixel(), 256, 0, stream>>>(in, frame_stride, bg, bg_stride, st->g, st->d_th, st->lo,
+                                                              st->hi, nullptr, st->m_a, st->m_u, st->m_l);
         ctx->launches += 1;
         // ---- branch A: threshold -> open -> remove small -> fill holes
         run_open(L, *st, st->m_a, st->m_t);
@@ -793,6 +794,28 @@ int highlight_frames_in_flight(cvvp_ctx *ctx, int *out_frames)
     return CVVP_OK;
 }
 
+// n >= 1 validated frames; frame f against the background at d_bg + f * bg_stride (0: one background for all)
+static int highlight_run(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_frames, long long n, size_t frame_stride,
+                         const uint8_t *d_bg, size_t bg_stride, uint8_t *d_out, size_t out_stride, cudaStream_t stream)
+{
+    if (!use_fused(st))
+        return highlight_pixels(ctx, st, d_frames, n, frame_stride, d_bg, bg_stride, d_out, out_stride, stream);
+    // fused path: one launch per (up to) 2^20 frames; scratch is per resident CTA, not per frame
+    const long long bmax = 1ll << 20;
+    for (long long done = 0; done < n; done += bmax) {
+        const unsigned nb = unsigned(n - done < bmax ? n - done : bmax);
+        const uint8_t *in = d_frames + size_t(done) * frame_stride;
+        const uint8_t *bg = d_bg + size_t(done) * bg_stride;
+        int rc;
+        if (st->th == -1 && (rc = highlight_thresholds(ctx, st, in, frame_stride, bg, bg_stride, nb, stream)) != CVVP_OK)
+            return rc;
+        if ((rc = highlight_fused_batch(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out + size_t(done) * out_stride,
+                                        out_stride, stream)) != CVVP_OK)
+            return rc;
+    }
+    return CVVP_OK;
+}
+
 int highlight_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, uint8_t *d_out,
                      size_t out_stride, cudaStream_t stream)
 {
@@ -803,21 +826,37 @@ int highlight_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t
         return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments");
     if (n == 0)
         return CVVP_OK;
-    if (!use_fused(st))
-        return highlight_pixels(ctx, st, d_frames, n, frame_stride, d_out, out_stride, stream);
-    // fused path: one launch per (up to) 2^20 frames; scratch is per resident CTA, not per frame
-    const long long bmax = 1ll << 20;
-    for (long long done = 0; done < n; done += bmax) {
-        const unsigned nb = unsigned(n - done < bmax ? n - done : bmax);
-        const uint8_t *in = d_frames + size_t(done) * frame_stride;
-        int rc;
-        if (st->th == -1 && (rc = highlight_thresholds(ctx, st, in, frame_stride, nb, stream)) != CVVP_OK)
-            return rc;
-        if ((rc = highlight_fused_batch(ctx, st, in, frame_stride, nb, d_out + size_t(done) * out_stride, out_stride,
-                                        stream)) != CVVP_OK)
-            return rc;
+    return highlight_run(ctx, st, d_frames, n, frame_stride, st->d_bg, 0, d_out, out_stride, stream);
+}
+
+int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, const uint8_t *d_bgs,
+                        size_t bg_stride, uint8_t *d_out, size_t out_stride, cvvp_component *d_comps, int max_comps,
+                        int *d_ncomps, int32_t *d_labels, size_t labels_stride, cudaStream_t stream)
+{
+    HighlightState *st = ctx->hl;
+    if (!st)
+        return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
+    if (!d_frames || !d_bgs || !d_out || n < 0 || frame_stride < st->g.npix || out_stride < st->g.npix ||
+        (bg_stride != 0 && bg_stride < st->g.npix))
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments (bg_stride must be 0 or at least %u)", st->g.npix);
+    if (d_comps || d_ncomps || d_labels) {
+        if (!d_comps || !d_ncomps || max_comps < 1 || (d_labels && labels_stride < st->g.npix))
+            return fail(ctx, CVVP_ERR_INVALID, "highlight components: bad arguments");
+        if (!use_fused(st))
+            return fail(ctx, CVVP_ERR_UNSUPPORTED, "highlight components: only the fused path labels the final masks");
+        if (n > (1ll << 20))
+            return fail(ctx, CVVP_ERR_UNSUPPORTED, "highlight components: at most 2^20 frames per call");
     }
-    return CVVP_OK;
+    if (n == 0)
+        return CVVP_OK;
+    st->cc.comps = d_comps;
+    st->cc.max_comps = d_comps ? max_comps : 0;
+    st->cc.ncomps = d_comps ? d_ncomps : nullptr;
+    st->cc.labels = d_comps ? d_labels : nullptr;
+    st->cc.labels_stride = labels_stride;
+    const int rc = highlight_run(ctx, st, d_frames, n, frame_stride, d_bgs, bg_stride, d_out, out_stride, stream);
+    st->cc = CcOut();
+    return rc;
 }
 
 static_assert(sizeof(cvvp_component) == 48, "cvvp_component is part of the C ABI (include/cvvp.h, _cabi.COMPONENT_DTYPE)");

@@ -86,6 +86,7 @@ struct FusedArgs {
     const uint8_t *frames;
     size_t frame_stride;
     const uint8_t *bg;
+    size_t bg_stride; // frame f's background at bg + f * bg_stride (0: one background for every frame)
     uint8_t *out;
     size_t out_stride;
     const int *th_a; // per-frame threshold of branch A (Otsu), or nullptr -> th
@@ -345,6 +346,7 @@ __device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t
 {
     const int tid = threadIdx.x;
     const uint8_t *fr = P.frames + size_t(f) * P.frame_stride;
+    const uint8_t *bg = P.bg + size_t(f) * P.bg_stride;
     const int th_a = P.th_a ? __ldg(P.th_a + f) : P.th;
     if (P.fast_io) {
         const ThreshSpec ta = make_thresh(th_a), tu = make_thresh(P.hi), tl = make_thresh(P.lo);
@@ -363,15 +365,15 @@ __device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t
                 const size_t o = size_t(y0) * P.W + 32u * wx0;
                 fa0 = __ldcs(reinterpret_cast<const uint4 *>(fr + o)); // frames are read once: streaming
                 fa1 = __ldcs(reinterpret_cast<const uint4 *>(fr + o + 16));
-                ba0 = __ldg(reinterpret_cast<const uint4 *>(P.bg + o));
-                ba1 = __ldg(reinterpret_cast<const uint4 *>(P.bg + o + 16));
+                ba0 = __ldg(reinterpret_cast<const uint4 *>(bg + o));
+                ba1 = __ldg(reinterpret_cast<const uint4 *>(bg + o + 16));
             }
             if (v1) {
                 const size_t o = size_t(y1) * P.W + 32u * wx1;
                 fb0 = __ldcs(reinterpret_cast<const uint4 *>(fr + o));
                 fb1 = __ldcs(reinterpret_cast<const uint4 *>(fr + o + 16));
-                bb0 = __ldg(reinterpret_cast<const uint4 *>(P.bg + o));
-                bb1 = __ldg(reinterpret_cast<const uint4 *>(P.bg + o + 16));
+                bb0 = __ldg(reinterpret_cast<const uint4 *>(bg + o));
+                bb1 = __ldg(reinterpret_cast<const uint4 *>(bg + o + 16));
             }
             uint32_t wa = 0, wu = 0, wl = 0;
             if (v0)
@@ -397,7 +399,7 @@ __device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t
                 const size_t o = size_t(y) * P.W;
                 const int x1 = min(32 * wx + 32, P.W);
                 for (int x = 32 * wx; x < x1; ++x) {
-                    const int d = max(int(__ldg(P.bg + o + x)) - int(__ldg(fr + o + x)), 0);
+                    const int d = max(int(__ldg(bg + o + x)) - int(__ldg(fr + o + x)), 0);
                     const uint32_t b = 1u << (x & 31);
                     if (d > th_a)
                         wa |= b;
@@ -2093,13 +2095,13 @@ size_t slot_bytes(const FusedGeom &fg)
 } // namespace
 
 int HLF(fused_frames_in_flight)(cvvp_ctx *ctx, HighlightState *st);
-int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, unsigned nb,
-                               uint8_t *d_out, size_t out_stride, cudaStream_t stream);
+int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
+                               size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream);
 
 #ifndef CVVP_HLF_SMALL
 int fused_frames_in_flight_small(cvvp_ctx *ctx, HighlightState *st);
-int highlight_fused_batch_small(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, unsigned nb,
-                                uint8_t *d_out, size_t out_stride, cudaStream_t stream);
+int highlight_fused_batch_small(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
+                                size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream);
 
 bool fused_supports(const HighlightState *st)
 {
@@ -2138,11 +2140,11 @@ int fused_frames_in_flight(cvvp_ctx *ctx, HighlightState *st)
     return use_small(st) ? fused_frames_in_flight_small(ctx, st) : fused_frames_in_flight_large(ctx, st);
 }
 
-int highlight_fused_batch(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, unsigned nb,
-                          uint8_t *d_out, size_t out_stride, cudaStream_t stream)
+int highlight_fused_batch(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
+                          size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream)
 {
-    return use_small(st) ? highlight_fused_batch_small(ctx, st, in, frame_stride, nb, d_out, out_stride, stream)
-                         : highlight_fused_batch_large(ctx, st, in, frame_stride, nb, d_out, out_stride, stream);
+    return use_small(st) ? highlight_fused_batch_small(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out, out_stride, stream)
+                         : highlight_fused_batch_large(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out, out_stride, stream);
 }
 #endif
 
@@ -2212,8 +2214,8 @@ static int ensure_fused(cvvp_ctx *ctx, HighlightState *st)
 
 // One batch of nb frames (device pointers), one kernel launch.  Work in flight on a context's highlight scratch must
 // be on one stream at a time.
-int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, unsigned nb,
-                               uint8_t *d_out, size_t out_stride, cudaStream_t stream)
+int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
+                               size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream)
 {
     int rc = ensure_fused(ctx, st);
     if (rc != CVVP_OK)
@@ -2222,7 +2224,8 @@ int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t 
     FusedArgs P;
     P.frames = in;
     P.frame_stride = frame_stride;
-    P.bg = st->d_bg;
+    P.bg = bg;
+    P.bg_stride = bg_stride;
     P.out = d_out;
     P.out_stride = out_stride;
     P.th_a = st->th == -1 ? st->d_th : nullptr;
@@ -2258,8 +2261,8 @@ int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t 
     // the common structuring elements have compile-time instantiations of the opening (CVVP_HL_NO_CT=1: run-time plan)
     P.ct_elem = (P.plan.sep && P.band_rows > 0 && !getenv("CVVP_HL_NO_CT")) ? match_ct_elem(st->h_offs) : 0;
     auto aligned16 = [](const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
-    P.fast_io = (P.W % 32 == 0) && aligned16(in) && aligned16(d_out) && aligned16(st->d_bg) && frame_stride % 16 == 0 &&
-                out_stride % 16 == 0;
+    P.fast_io = (P.W % 32 == 0) && aligned16(in) && aligned16(d_out) && aligned16(bg) && frame_stride % 16 == 0 &&
+                out_stride % 16 == 0 && bg_stride % 16 == 0;
     const char *dbg = getenv("CVVP_HL_DEBUG_STAGE");
     P.debug_stage = dbg ? atoi(dbg) : 0;
     P.comps = st->cc.comps;

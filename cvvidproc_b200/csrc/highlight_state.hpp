@@ -71,12 +71,13 @@ struct HighlightState {
 };
 
 // highlight.cu
-int highlight_thresholds(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, unsigned nb,
-                         cudaStream_t stream);
+// bg: background of the batch's first frame, frame f's at bg + f * bg_stride (0 = one background for every frame)
+int highlight_thresholds(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
+                         size_t bg_stride, unsigned nb, cudaStream_t stream);
 // highlight_fused.cu
 bool fused_supports(const HighlightState *st);
 void fused_release(HighlightState *st);
 int fused_frames_in_flight(cvvp_ctx *ctx, HighlightState *st);
-int highlight_fused_batch(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, unsigned nb,
-                          uint8_t *d_out, size_t out_stride, cudaStream_t stream);
+int highlight_fused_batch(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
+                          size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream);
 } // namespace cvvp

@@ -458,4 +458,106 @@ private:
     std::deque<std::unique_ptr<FrameBatch>> m_ready{};
     bool m_no_more{false};
 };
+
+// ---------------------------------------------------------------------------------------------------------------------
+// highlight against a rolling temporal-median background (no counterpart in the reference, whose background is static):
+// frame t is compared with the median of a window of `window` frames centred on it (cvvp_highlight_rolling_*).  The
+// reference's four-method shape, but TryGetResult legitimately lags Insert: a frame's mask needs frames up to
+// ceil(window / 2) - 1 ahead of it (window - 1 at the start), and the last ones only come after NotifyNoMoreTokens.
+// The pack's background only sets the geometry.  Result batches are in frame order.
+// ---------------------------------------------------------------------------------------------------------------------
+class GpuRollingHighlightAlgo
+{
+public:
+    using token_type = FrameBatch;
+    using result_type = FrameBatch;
+    // pack.max_batch: frames per Insert (at most); pack.source: tokens are DECODED frames, prepared on the device
+    GpuRollingHighlightAlgo(GpuHighlightPack pack, int window) : m_pack{std::move(pack)}, m_ctx{m_pack.device}
+    {
+        CVVP_ASSERT(!m_pack.background.empty());
+        CVVP_ASSERT(!m_pack.struct_element.empty());
+        CVVP_ASSERT_MSG(m_pack.background.channels == 1, "the highlight stage works on single-channel frames");
+        CVVP_ASSERT(m_pack.max_batch > 0);
+        m_ctx.check(cvvp_highlight_begin(m_ctx.get(), m_pack.background.data.data(), m_pack.background.cols,
+                                         m_pack.background.rows, m_pack.struct_element.data.data(),
+                                         m_pack.struct_element.cols, m_pack.struct_element.rows, m_pack.threshold,
+                                         m_pack.threshold_lo, m_pack.threshold_hi, m_pack.min_size_hyst,
+                                         m_pack.min_size_threshold, m_pack.width_border));
+        m_ctx.check(cvvp_highlight_rolling_begin(m_ctx.get(), window, m_pack.max_batch,
+                                                 m_pack.source.enabled ? &m_pack.source.fmt : nullptr,
+                                                 m_pack.components ? m_pack.max_components : 0,
+                                                 m_pack.components && m_pack.labels ? 1 : 0));
+    }
+    void Insert(std::unique_ptr<FrameBatch> batch)
+    {
+        if (!batch || batch->empty())
+            return;
+        if (m_pack.source.enabled)
+            CVVP_ASSERT_MSG(batch->rows == m_pack.source.fmt.src_height && batch->cols == m_pack.source.fmt.src_width &&
+                                batch->channels == m_pack.source.fmt.src_channels,
+                            "decoded frame geometry must match the source format");
+        else
+            CVVP_ASSERT_MSG(batch->channels == 1 && batch->rows == m_pack.background.rows && batch->cols == m_pack.background.cols,
+                            "frame geometry must match the background");
+        for (int done = 0; done < batch->n;) {
+            const int k = int(std::min<long long>(batch->n - done, m_pack.max_batch));
+            m_ctx.check(cvvp_highlight_rolling_push(m_ctx.get(), batch->data.data() + std::size_t(done) * batch->frame_bytes(), k,
+                                                    batch->frame_bytes()));
+            done += k;
+        }
+    }
+    // null = none yet.  Before NotifyNoMoreTokens only a batch that is complete on the device is returned; after it,
+    // waits for what is pending, in order.
+    std::unique_ptr<FrameBatch> TryGetResult()
+    {
+        if (cvvp_highlight_rolling_pending(m_ctx.get()) == 0)
+            return nullptr;
+        const int ready = cvvp_highlight_rolling_ready(m_ctx.get());
+        if (ready < 0)
+            m_ctx.check(ready);
+        if (ready == 0 && !m_no_more)
+            return nullptr;
+        auto out = std::make_unique<FrameBatch>();
+        out->rows = m_pack.background.rows;
+        out->cols = m_pack.background.cols;
+        out->channels = 1;
+        out->data.resize(std::size_t(m_pack.max_batch) * out->frame_bytes());
+        const bool labels = m_pack.components && m_pack.labels;
+        if (m_pack.components) {
+            out->max_comps = m_pack.max_components;
+            out->comps.resize(std::size_t(m_pack.max_batch) * m_pack.max_components);
+            out->ncomps.resize(std::size_t(m_pack.max_batch));
+        }
+        if (labels)
+            out->labels.resize(std::size_t(m_pack.max_batch) * out->frame_bytes());
+        long long first = 0, n = 0;
+        m_ctx.check(cvvp_highlight_rolling_next(m_ctx.get(), out->data.data(), out->frame_bytes(), m_pack.max_batch, &first, &n,
+                                                m_pack.components ? out->comps.data() : nullptr,
+                                                m_pack.components ? out->ncomps.data() : nullptr,
+                                                labels ? out->labels.data() : nullptr, out->frame_bytes()));
+        CVVP_ASSERT_MSG(first == m_returned, "rolling highlight results out of order");
+        m_returned += n;
+        out->n = int(n);
+        out->data.resize(std::size_t(n) * out->frame_bytes());
+        if (labels)
+            out->labels.resize(std::size_t(n) * out->frame_bytes());
+        return out;
+    }
+    // end of the stream: the last frames' windows clamp to the frames inserted
+    void NotifyNoMoreTokens()
+    {
+        if (m_no_more)
+            return;
+        m_no_more = true;
+        m_ctx.check(cvvp_highlight_rolling_close(m_ctx.get()));
+    }
+    bool HasResults() const { return cvvp_highlight_rolling_pending(m_ctx.get()) > 0; }
+    int max_components() const { return m_pack.max_components; }
+
+private:
+    GpuHighlightPack m_pack;
+    Context m_ctx;
+    bool m_no_more{false};
+    long long m_returned{0};
+};
 } // namespace cvvp_host

@@ -571,8 +571,34 @@ FrameBatch to_u8_image(const py::array &src, const char *what)
     return b;
 }
 
+// kwargs["cvvp_background_window"]: 0 when absent, else an int in [1, 65535] (RuntimeError otherwise)
+int background_window(const py::dict &kwargs)
+{
+    if (!kwargs.contains("cvvp_background_window"))
+        return 0;
+    py::object w = kwargs["cvvp_background_window"];
+    bool ok = PyIndex_Check(w.ptr()) && !PyBool_Check(w.ptr());
+    long long v = 0;
+    if (ok) {
+        int overflow = 0;
+        py::int_ iw = py::reinterpret_steal<py::int_>(PyNumber_Index(w.ptr()));
+        v = PyLong_AsLongLongAndOverflow(iw.ptr(), &overflow);
+        ok = overflow == 0 && v >= 1 && v <= 65535;
+    }
+    CVVP_ASSERT_MSG(ok, "kwargs['cvvp_background_window'] must be an int in [1, 65535]");
+    return int(v);
+}
+
 py::dict TrackObjects(const VidObjectTrackPack &pack)
 {
+    // Opt-in extra of this implementation (the reference has no counterpart): kwargs["cvvp_background_window"] = W
+    // compares frame t with the rolling upper median of a window of W frames centred on it (shifted, not shortened,
+    // at both ends of the processed frames; cvvp_median_rolling_device) instead of the pack's background, which is
+    // then only validated (non-empty, the cropped frame's size) and not used for the masks.  Checked before any
+    // device work.  The masks reach the callback in frame order as always, but later than their frames are decoded
+    // (up to W - 1 frames).  With several devices in CVVP_DEVICES this mode runs on the first one.
+    const int roll_window = background_window(pack.assign_objects_pack.kwargs);
+    const bool rolling = roll_window > 0;
     FrameSource vid{pack.vid_path, pack.grayscale, pack.vid_is_grayscale};
     if (!vid.opened()) {
         std::cerr << "Video file not detected: " << pack.vid_path << '\n';
@@ -624,7 +650,12 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
         hp.max_components = std::max(1, user_kwargs["cvvp_max_components"].cast<int>());
     // label images only travel through the synchronous entry point; everything else is queued
     const bool on_device = !host_prep() && !want_labels;
+    // rolling mode takes the synchronous loop below (the rolling stream handles labels itself): frames are prepared on
+    // the device unless CVVP_HOST_PREP=1
+    const bool pipelined = on_device && !rolling;
+    const bool device_prep = rolling ? !host_prep() : on_device;
     std::unique_ptr<GpuHighlightAlgo> highlighter; // built once the first decoded frame tells the channel count
+    std::unique_ptr<GpuRollingHighlightAlgo> roller; // rolling mode's operator
 
     // frames per device batch: the reference's batch_size is a thread count; here it is sized for the GPU, and at most
     // token_storage_limit batches are in flight like the reference's queues (token_queue.h:209-214)
@@ -717,7 +748,9 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     };
 
     const std::vector<int> devices = device_list();
-    if (on_device) {
+    if (rolling)
+        hp.device = devices.front();
+    if (pipelined) {
         // ---- pipelined path: decode thread -> pinned queue slots -> device(s) -> ordered callbacks ----
         // the first frame is decoded here: it tells the channel count the device format needs
         h_gen.start();
@@ -837,13 +870,13 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
         }
     }
     long long consumed = 0;
-    bool eof = on_device; // the pipelined path above has consumed the stream
+    bool eof = pipelined; // the pipelined path above has consumed the stream
     while (!eof && consumed < num_frames) {
         h_batch.start();
         h_gen.start();
         auto batch = std::make_unique<FrameBatch>();
         while (batch->n < batch_frames && consumed < num_frames) {
-            py::object f = on_device ? vid.next_decoded() : vid.next();
+            py::object f = device_prep ? vid.next_decoded() : vid.next();
             if (f.is_none()) {
                 eof = true;
                 break;
@@ -851,17 +884,20 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
             py::array a = f.cast<py::array>();
             int r, c, ch;
             array_geometry(a, r, c, ch);
-            if (!highlighter) {
+            if (!highlighter && !roller) {
                 hp.queue_depth = depth;
                 hp.max_batch = batch_frames;
-                if (on_device) {
+                if (device_prep) {
                     CVVP_ASSERT(r == fh && c == fw);
                     hp.source = vid.format_for(r, c, ch);
                     CVVP_ASSERT_MSG(hp.source.out_channels() == 1,
                                     "TrackObjects needs single-channel frames: set grayscale or vid_is_grayscale "
                                     "(cv::findContours requires 8UC1)");
                 }
-                highlighter = std::make_unique<GpuHighlightAlgo>(std::move(hp));
+                if (rolling)
+                    roller = std::make_unique<GpuRollingHighlightAlgo>(std::move(hp), roll_window);
+                else
+                    highlighter = std::make_unique<GpuHighlightAlgo>(std::move(hp));
             }
             if (batch->n == 0) {
                 batch->rows = r;
@@ -870,7 +906,7 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
                 // one allocation per batch: a vector that grows frame by frame re-copies every decoded frame
                 batch->data.reserve(std::size_t(std::min(batch_frames, num_frames - consumed)) * r * c * ch);
             }
-            if (!on_device) {
+            if (!device_prep) {
                 CVVP_ASSERT_MSG(ch == 1, "TrackObjects needs single-channel frames: set grayscale or vid_is_grayscale "
                                          "(cv::findContours requires 8UC1)");
                 CVVP_ASSERT(r == crop.height && c == crop.width);
@@ -885,24 +921,30 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
         if (batch->n == 0)
             break;
         h_unit.start();
-        highlighter->Insert(std::move(batch)); // queued on the device; returns before the masks exist
+        if (roller)
+            roller->Insert(std::move(batch));
+        else
+            highlighter->Insert(std::move(batch)); // queued on the device; returns before the masks exist
         h_unit.stop();
         h_batch.stop();
         // masks that have come back meanwhile go to the tracker while the device works on the newer batches
         for (;;) {
             h_consume.start();
-            std::unique_ptr<FrameBatch> masks = highlighter->TryGetResult();
+            std::unique_ptr<FrameBatch> masks = roller ? roller->TryGetResult() : highlighter->TryGetResult();
             h_consume.stop();
             if (!masks)
                 break;
             deliver(*masks);
         }
     }
-    if (highlighter) { // end of stream: drain in order (token_processing_unit.h:334)
-        highlighter->NotifyNoMoreTokens();
+    if (highlighter || roller) { // end of stream: drain in order (token_processing_unit.h:334)
+        if (roller)
+            roller->NotifyNoMoreTokens(); // the last frames' windows clamp to the frames decoded
+        else
+            highlighter->NotifyNoMoreTokens();
         for (;;) {
             h_consume.start();
-            std::unique_ptr<FrameBatch> masks = highlighter->TryGetResult();
+            std::unique_ptr<FrameBatch> masks = roller ? roller->TryGetResult() : highlighter->TryGetResult();
             h_consume.stop();
             if (!masks)
                 break;

@@ -132,6 +132,23 @@ CVVP_API int cvvp_median_device(cvvp_ctx *ctx, const uint8_t *d_frames, long lon
                        size_t frame_stride, uint8_t *d_out, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * rolling temporal median -- a background that follows the video.  The reference has one static background per
+ *   TrackObjects call (Sources/cv_vid_objecttrack_helpers.cpp:167-175, the pack's background); here frame t of a
+ *   stream of N frames gets the upper median (histogram_median_algo.h:160-166, sorted[Weff/2], Weff = min(W, N)) of
+ *   a window of W frames centred on it and shifted, not shortened, at both ends:
+ *     N <= W : every window is all N frames
+ *     N >  W : window of frame t = frames s(t) .. s(t) + W - 1, s(t) = min(max(t - W/2, 0), N - W)
+ * Device-resident form, layout as cvvp_median_device (frame f at d_frames + f*frame_stride, nelem bytes each, any
+ * nelem: colour stacks work element by element): writes the backgrounds of frames t in [t0, t1) to
+ * d_out + (t - t0)*out_stride.  Exact for every window (16-bit counts per element and value, 1 <= window <= 65535).
+ * Runs on `stream` (NULL = the context's compute stream) and does not synchronize.  CVVP_ERR_INVALID for window < 1 or
+ * > 65535, nframes < 1, t0 / t1 outside 0 <= t0 <= t1 <= nframes, a stride shorter than nelem or a NULL pointer.
+ * ------------------------------------------------------------------------------------------- */
+CVVP_API int cvvp_median_rolling_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem,
+                                        size_t frame_stride, int window, long long t0, long long t1, uint8_t *d_out,
+                                        size_t out_stride, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * frame-sharded temporal median across GPUs (one process -- or at least one context -- per GPU).
  *   The reference splits the frame range of a video over its generator threads
  *   (Sources/cv_vid_bg_helpers.cpp:84-120) and merges them in ONE order-independent histogram
@@ -246,6 +263,14 @@ typedef struct cvvp_component {
 CVVP_API int cvvp_highlight_device_cc(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride,
                                       uint8_t *d_out, size_t out_stride, cvvp_component *d_comps, int max_comps,
                                       int *d_ncomps, int32_t *d_labels, size_t labels_stride, void *stream);
+/* Like cvvp_highlight_device_cc, but frame f is compared with its OWN background at d_backgrounds + f * bg_stride
+ * (DEVICE pointer; bg_stride = 0: the one image at d_backgrounds for every frame; else bg_stride >= width*height).
+ * The background given to cvvp_highlight_begin only sets the geometry here.  d_comps / d_ncomps / d_labels NULL =
+ * no components (then max_comps is ignored); with components, fused path only, like cvvp_highlight_device_cc. */
+CVVP_API int cvvp_highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride,
+                                      const uint8_t *d_backgrounds, size_t bg_stride, uint8_t *d_out, size_t out_stride,
+                                      cvvp_component *d_comps, int max_comps, int *d_ncomps, int32_t *d_labels,
+                                      size_t labels_stride, void *stream);
 /* HOST-buffer form (synchronous): masks, components, counts and (optionally, NULL = off) label images */
 CVVP_API int cvvp_highlight_frames_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride,
                                       uint8_t *masks_out, size_t out_stride, cvvp_component *comps_out, int max_comps,
@@ -347,6 +372,41 @@ CVVP_API int cvvp_highlight_next_view(cvvp_ctx *ctx, const uint8_t **h_masks, si
 CVVP_API int cvvp_highlight_view_release(cvvp_ctx *ctx);
 /* drains and frees the ring (pending results are dropped) */
 CVVP_API int cvvp_highlight_queue_end(cvvp_ctx *ctx);
+
+/* ---------------------------------------------------------------------------------------------
+ * highlight against a rolling median background, ordered stream -- TrackObjects with a background that follows the
+ *   video (see cvvp_median_rolling_device for the windows).  The mask of frame t is HighlightObjects(f_t) (highlight_
+ *   objects_algo.cpp:17-78) with B_t, the rolling median of its window, in place of the pack's background.  Masks come
+ *   back LATER than their frames go in: frame t needs W - 1 frames ahead at the start of the stream and
+ *   ceil(W/2) - 1 afterwards; the last ones are computed when the stream is closed (the frame count is only known
+ *   then), with windows clamped to the frames pushed.  The device keeps a ring of (W + max_batch) prepared frames of
+ *   round_up(width*height, 128) bytes.
+ *   cvvp_highlight_begin ... cvvp_highlight_rolling_begin, { push | next }*, close, next*, cvvp_highlight_rolling_end
+ * ------------------------------------------------------------------------------------------- */
+/* 1 <= window <= 65535, 1 <= max_batch <= 2^20 frames per push.  fmt != NULL: pushed frames are DECODED frames
+ * prepared on the device (prepared geometry = the background's, one channel); NULL: frames of width*height bytes.
+ * max_comps > 0 also returns the components of every mask; labels != 0 (needs max_comps > 0) also the label images.
+ * CVVP_ERR_NOMEM naming the window when the ring does not fit. */
+CVVP_API int cvvp_highlight_rolling_begin(cvvp_ctx *ctx, int window, long long max_batch, const cvvp_frame_format *fmt,
+                                          int max_comps, int labels);
+/* n frames from HOST memory (may be reused on return); queues the backgrounds, masks and downloads of every frame whose
+ * window is now complete, in chunks of at most max_batch frames */
+CVVP_API int cvvp_highlight_rolling_push(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride);
+/* end of the stream: queues the remaining frames; no push after it */
+CVVP_API int cvvp_highlight_rolling_close(cvvp_ctx *ctx);
+/* result chunks queued and not yet returned by cvvp_highlight_rolling_next */
+CVVP_API int cvvp_highlight_rolling_pending(const cvvp_ctx *ctx);
+/* 1 if the oldest pending chunk is complete, 0 if not (or nothing is pending); never blocks */
+CVVP_API int cvvp_highlight_rolling_ready(cvvp_ctx *ctx);
+/* Waits for the oldest pending chunk and copies its *n_out (<= max_n, at most max_batch) masks of frames
+ * *first_index, *first_index + 1, ... to masks_out (mask i at masks_out + i*out_stride) and, when begun with them and
+ * the pointers are not NULL, components (comps_out[i*max_comps + k]), counts and label images (labels_out +
+ * i*labels_stride elements).  *n_out = 0 when nothing is pending. */
+CVVP_API int cvvp_highlight_rolling_next(cvvp_ctx *ctx, uint8_t *masks_out, size_t out_stride, long long max_n,
+                                         long long *first_index, long long *n_out, cvvp_component *comps_out,
+                                         int *ncomps_out, int32_t *labels_out, size_t labels_stride);
+/* drains and frees the stream (pending results are dropped) */
+CVVP_API int cvvp_highlight_rolling_end(cvvp_ctx *ctx);
 
 /* ---------------------------------------------------------------------------------------------
  * synthetic input (SURVEY.md 8d): deterministic integer-hash frames generated directly in
