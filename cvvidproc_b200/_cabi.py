@@ -67,6 +67,8 @@ def load():
         "cvvp_median_device": (i32, [vp, vp, i64, sz, sz, vp, vp]),
         "cvvp_median_last_kernel_ms": (i32, [vp, C.POINTER(C.c_float)]),
         "cvvp_median_rolling_device": (i32, [vp, vp, i64, sz, sz, i32, i64, i64, vp, sz, vp]),
+        "cvvp_median_set_percentile": (i32, [vp, i32]),
+        "cvvp_median_percentile": (i32, [vp]),
         "cvvp_highlight_begin": (i32, [vp, vp, i32, i32, vp, i32, i32, i32, i32, i32, i32, i32, i32]),
         "cvvp_highlight_frames": (i32, [vp, vp, i64, sz, vp, sz]),
         "cvvp_highlight_device": (i32, [vp, vp, i64, sz, vp, sz, vp]),
@@ -324,9 +326,17 @@ class Context:
 
     def median_rolling_device(self, d_frames: int, nframes: int, nelem: int, frame_stride: int, window: int, t0: int,
                               t1: int, d_out: int, out_stride: int, stream: int = 0):
-        """backgrounds of frames [t0, t1): the upper median of each frame's centred window of `window` frames"""
+        """backgrounds of frames [t0, t1): the context's percentile (the upper median at the default) of each frame's
+        centred window of `window` frames"""
         self._check(self._lib.cvvp_median_rolling_device(self._h, d_frames, nframes, nelem, frame_stride, window, t0, t1,
                                                          d_out, out_stride, stream or None))
+
+    def median_set_percentile(self, percent: int):
+        """every background of this context becomes sorted[min(N - 1, N * percent // 100)]; jobs take it when they begin"""
+        self._check(self._lib.cvvp_median_set_percentile(self._h, percent))
+
+    def median_percentile(self) -> int:
+        return int(self._lib.cvvp_median_percentile(self._h))
 
     def median_last_kernel_ms(self) -> float:
         v = C.c_float()

@@ -563,6 +563,7 @@ int cvvp_median_begin(cvvp_ctx *ctx, size_t nelem, long long nframes_hint)
     m.split = false;
     m.half = 0;
     m.base = 0;
+    m.percent = ctx->percent; // the job keeps the percentile it began with
     if (m.d_out_bytes < stride) {
         if (m.d_out)
             cudaFree(m.d_out);
@@ -665,9 +666,9 @@ int cvvp_median_finish(cvvp_ctx *ctx, uint8_t *out)
             // constant-memory form: the rest of the stack joins the histograms, the median is read off them
             if ((rc = spill_resident(ctx)) != CVVP_OK)
                 break;
-            rc = median_hist_select(ctx, m.d_hist, m.stride, m.nelem, m.folded, m.d_out, ctx->compute);
+            rc = median_hist_select(ctx, m.d_hist, m.stride, m.nelem, m.folded, m.percent, m.d_out, ctx->compute);
         } else {
-            rc = median_launch(ctx, m.d_stack, m.count, m.nelem, m.stride, m.d_out, ctx->compute);
+            rc = median_launch(ctx, m.d_stack, m.count, m.nelem, m.stride, m.d_out, m.percent, ctx->compute);
         }
         if (rc != CVVP_OK)
             break;
@@ -740,7 +741,7 @@ int cvvp_median_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes
         return fail(nullptr, CVVP_ERR_INVALID, "null context");
     DeviceGuard guard(ctx->device);
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->compute;
-    return median_launch(ctx, d_frames, nframes, nelem, frame_stride, d_out, s);
+    return median_launch(ctx, d_frames, nframes, nelem, frame_stride, d_out, ctx->percent, s);
 }
 
 int cvvp_median_rolling_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
@@ -750,7 +751,28 @@ int cvvp_median_rolling_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long
         return fail(nullptr, CVVP_ERR_INVALID, "null context");
     DeviceGuard guard(ctx->device);
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->compute;
-    return median_roll_launch(ctx, d_frames, nframes, frame_stride, nframes, nelem, window, t0, t1, d_out, out_stride, s);
+    return median_roll_launch(ctx, d_frames, nframes, frame_stride, nframes, nelem, window, ctx->percent, t0, t1, d_out,
+                              out_stride, s);
+}
+
+int cvvp_median_set_percentile(cvvp_ctx *ctx, int percent)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    if (percent < 0 || percent > 100)
+        return fail(ctx, CVVP_ERR_INVALID, "median: percentile %d outside [0, 100]", percent);
+    // open jobs took the percentile when they began; changing it underneath them would mix two rank rules
+    if (ctx->med.active || ctx->shard || ctx->hr)
+        return fail(ctx, CVVP_ERR_STATE, "median: a median, sharded or rolling job is open on this context");
+    ctx->percent = percent;
+    return CVVP_OK;
+}
+
+int cvvp_median_percentile(const cvvp_ctx *ctx)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    return ctx->percent;
 }
 
 int cvvp_median_last_kernel_ms(cvvp_ctx *ctx, float *out_ms)

@@ -39,6 +39,7 @@ struct MedianJob {
     uint32_t *d_hist{nullptr}; // [256][stride] counts, or nullptr
     size_t d_hist_bytes{0};
     long long folded{0};       // frames that live in d_hist only (count = the frames resident in d_stack)
+    int percent{50};           // the context's percentile when the job began (cvvp_median_set_percentile)
     // after the first fold the stack is used as two halves: one is filled while the other is being folded
     bool split{false};
     int half{0};
@@ -108,6 +109,7 @@ struct cvvp_ctx {
     cvvp::RawStage raw;
     cvvp::HighlightQueue *hq{nullptr};
     cvvp::RollingStream *hr{nullptr};
+    int percent{50}; // percentile of every background (cvvp_median_set_percentile); jobs take it when they begin
 };
 
 namespace cvvp
@@ -145,24 +147,25 @@ struct DeviceGuard {
 };
 
 // median.cu
+// percent: the percentile every form selects, sorted[percentile_rank(N, percent)] (median_common.cuh)
 int median_launch(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
-                  uint8_t *d_out, cudaStream_t stream);
+                  uint8_t *d_out, int percent, cudaStream_t stream);
 int median_launch_mode(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
-                       uint8_t *d_out, int mode, const ShardPush &push, cudaStream_t stream);
+                       uint8_t *d_out, int mode, int percent, const ShardPush &push, cudaStream_t stream);
 // median_pipe.cu
 long long median_max_frames();
 int median_pipe_launch(cvvp_ctx *ctx, const CUtensorMap &tmap, int log2s, uint8_t *d_out, uint32_t nelem, uint32_t nframes,
-                       uint32_t nst, int mode, const ShardPush &push, cudaStream_t stream);
+                       uint32_t nst, int mode, uint32_t percent, const ShardPush &push, cudaStream_t stream);
 // median_hist.cu
 size_t median_hist_bytes(size_t frame_stride);
 int median_hist_fold(cvvp_ctx *ctx, const uint8_t *d_stack, long long nframes, size_t frame_stride, uint32_t *d_hist,
                      cudaStream_t stream);
-int median_hist_select(cvvp_ctx *ctx, const uint32_t *d_hist, size_t frame_stride, size_t nelem, long long total, uint8_t *d_out,
-                       cudaStream_t stream);
+int median_hist_select(cvvp_ctx *ctx, const uint32_t *d_hist, size_t frame_stride, size_t nelem, long long total, int percent,
+                       uint8_t *d_out, cudaStream_t stream);
 // median_shard.cu
 void median_shard_release(cvvp_ctx *ctx);
 int median_long_stack(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
-                      uint8_t *d_out, cudaStream_t stream, int window);
+                      uint8_t *d_out, int percent, cudaStream_t stream, int window);
 long long median_two_pass_max_frames();
 // highlight.cu
 void highlight_release(cvvp_ctx *ctx);
@@ -210,7 +213,7 @@ int highlight_queue_next_view(cvvp_ctx *ctx, const uint8_t **h_masks, size_t *ma
 int highlight_queue_view_release(cvvp_ctx *ctx);
 // median_roll.cu: backgrounds of outputs [t0, t1) of a rolling-window median; frame i at d_frames + (i % ring) * stride
 int median_roll_launch(cvvp_ctx *ctx, const uint8_t *d_frames, long long ring, size_t frame_stride, long long nframes,
-                       size_t nelem, int window, long long t0, long long t1, uint8_t *d_out, size_t out_stride,
+                       size_t nelem, int window, int percent, long long t0, long long t1, uint8_t *d_out, size_t out_stride,
                        cudaStream_t stream);
 // highlight_rolling.cu
 void highlight_rolling_release(cvvp_ctx *ctx);

@@ -44,6 +44,7 @@ struct RollSlot {
 
 struct RollingStream {
     int window{0};
+    int percent{50}; // the context's percentile when the stream began
     long long max_batch{0};
     bool has_fmt{false};
     cvvp_frame_format fmt{};
@@ -117,6 +118,7 @@ int highlight_rolling_begin(cvvp_ctx *ctx, int window, long long max_batch, cons
         return fail(ctx, CVVP_ERR_NOMEM, "out of host memory");
     ctx->hr = r;
     r->window = window;
+    r->percent = ctx->percent;
     r->max_batch = max_batch;
     r->has_fmt = fmt != nullptr;
     if (fmt)
@@ -213,8 +215,8 @@ static int launch_ready(cvvp_ctx *ctx, RollingStream *r)
         s->first = t0;
         s->n = n;
         r->pending.push_back(s);
-        rc = median_roll_launch(ctx, r->d_ring, r->ring, r->pitch, r->received, r->npix, r->window, t0, t0 + n, r->d_bgs,
-                                r->pitch, ctx->compute);
+        rc = median_roll_launch(ctx, r->d_ring, r->ring, r->pitch, r->received, r->npix, r->window, r->percent, t0, t0 + n,
+                                r->d_bgs, r->pitch, ctx->compute);
         if (rc != CVVP_OK)
             return rc;
         // the frames themselves, in at most two contiguous runs of ring slots

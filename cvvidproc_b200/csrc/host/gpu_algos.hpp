@@ -97,6 +97,7 @@ struct GpuMedianPack {
     int device{-1};
     long long frames_hint{-1}; // frames_to_analyze of GetVideoBackground (cv_vid_bg_helpers.cpp:226-229)
     SourceFormat source{};     // enabled: InsertDecoded takes decoded frames
+    int percent{50};           // the result is sorted[k(N, percent)] per element (cvvp_median_set_percentile)
 };
 
 class GpuMedianAlgo
@@ -104,7 +105,10 @@ class GpuMedianAlgo
 public:
     using token_type = FrameBatch;
     using result_type = FrameBatch;
-    explicit GpuMedianAlgo(GpuMedianPack pack) : m_pack{pack}, m_ctx{pack.device} {}
+    explicit GpuMedianAlgo(GpuMedianPack pack) : m_pack{pack}, m_ctx{pack.device}
+    {
+        m_ctx.check(cvvp_median_set_percentile(m_ctx.get(), m_pack.percent));
+    }
 
     // histogram_median_algo.h:66-87 -- null / empty tokens are skipped without counting
     void Insert(std::unique_ptr<FrameBatch> batch)
@@ -192,12 +196,16 @@ class GpuShardedMedianAlgo
 public:
     using token_type = FrameBatch;
     using result_type = FrameBatch;
-    GpuShardedMedianAlgo(const std::vector<int> &devices, long long frames_hint, SourceFormat source) : m_source{source}
+    // percent: every device's context selects sorted[k(N, percent)] -- the ranks of one job must agree on it
+    GpuShardedMedianAlgo(const std::vector<int> &devices, long long frames_hint, SourceFormat source, int percent = 50)
+        : m_source{source}
     {
         CVVP_ASSERT_MSG(!devices.empty() && devices.size() <= 16, "1..16 devices");
         CVVP_ASSERT_MSG(source.enabled, "the multi-device median takes decoded frames");
-        for (int d : devices)
+        for (int d : devices) {
             m_ctx.push_back(std::make_unique<Context>(d));
+            m_ctx.back()->check(cvvp_median_set_percentile(m_ctx.back()->get(), percent));
+        }
         m_hint = frames_hint > 0 ? (frames_hint + (long long)devices.size() - 1) / (long long)devices.size() : -1;
     }
     // `turn` tokens in a row go to one device, then the next device takes over
@@ -461,9 +469,10 @@ private:
 
 // ---------------------------------------------------------------------------------------------------------------------
 // highlight against a rolling temporal-median background (no counterpart in the reference, whose background is static):
-// frame t is compared with the median of a window of `window` frames centred on it (cvvp_highlight_rolling_*).  The
-// reference's four-method shape, but TryGetResult legitimately lags Insert: a frame's mask needs frames up to
-// ceil(window / 2) - 1 ahead of it (window - 1 at the start), and the last ones only come after NotifyNoMoreTokens.
+// frame t is compared with the percentile `percent` (the upper median at 50) of a window of `window` frames centred on
+// it (cvvp_highlight_rolling_*).  The reference's four-method shape, but TryGetResult legitimately lags Insert: a
+// frame's mask needs frames up to ceil(window / 2) - 1 ahead of it (window - 1 at the start), and the last ones only
+// come after NotifyNoMoreTokens.
 // The pack's background only sets the geometry.  Result batches are in frame order.
 // ---------------------------------------------------------------------------------------------------------------------
 class GpuRollingHighlightAlgo
@@ -472,7 +481,7 @@ public:
     using token_type = FrameBatch;
     using result_type = FrameBatch;
     // pack.max_batch: frames per Insert (at most); pack.source: tokens are DECODED frames, prepared on the device
-    GpuRollingHighlightAlgo(GpuHighlightPack pack, int window) : m_pack{std::move(pack)}, m_ctx{m_pack.device}
+    GpuRollingHighlightAlgo(GpuHighlightPack pack, int window, int percent = 50) : m_pack{std::move(pack)}, m_ctx{m_pack.device}
     {
         CVVP_ASSERT(!m_pack.background.empty());
         CVVP_ASSERT(!m_pack.struct_element.empty());
@@ -483,6 +492,7 @@ public:
                                          m_pack.struct_element.cols, m_pack.struct_element.rows, m_pack.threshold,
                                          m_pack.threshold_lo, m_pack.threshold_hi, m_pack.min_size_hyst,
                                          m_pack.min_size_threshold, m_pack.width_border));
+        m_ctx.check(cvvp_median_set_percentile(m_ctx.get(), percent));
         m_ctx.check(cvvp_highlight_rolling_begin(m_ctx.get(), window, m_pack.max_batch,
                                                  m_pack.source.enabled ? &m_pack.source.fmt : nullptr,
                                                  m_pack.components ? m_pack.max_components : 0,

@@ -425,6 +425,33 @@ private:
 // ---------------------------------------------------------------------------------------------------------------------
 // GetVideoBackground  (cv_vid_bg_helpers.cpp:197-264)
 // ---------------------------------------------------------------------------------------------------------------------
+// The background algorithm names GetVideoBackground accepts (GetBGAlgo, cv_vid_bg_helpers.cpp:27-37): the reference's
+// "hist" (the upper median), and "cvvp_percentile:P" -- P an integer percent written without leading zeros, 0..100 --,
+// the same histogram path selecting sorted[k(N, P)] (cvvp_median_set_percentile).  false: an unknown algorithm.
+bool background_percent(const std::string &algo, int *percent)
+{
+    if (algo == "hist") {
+        *percent = 50;
+        return true;
+    }
+    static const std::string prefix = "cvvp_percentile:";
+    if (algo.compare(0, prefix.size(), prefix) != 0)
+        return false;
+    const std::string digits = algo.substr(prefix.size());
+    if (digits.empty() || digits.size() > 3 || (digits.size() > 1 && digits[0] == '0'))
+        return false;
+    int v = 0;
+    for (char c : digits) {
+        if (c < '0' || c > '9')
+            return false;
+        v = v * 10 + (c - '0');
+    }
+    if (v > 100)
+        return false;
+    *percent = v;
+    return true;
+}
+
 py::object GetVideoBackground(const VidBgPack &pack)
 {
     FrameSource vid{pack.vid_path, pack.grayscale, pack.vid_is_grayscale};
@@ -446,7 +473,8 @@ py::object GetVideoBackground(const VidBgPack &pack)
     if (frames_to_analyze <= 0 || frames_to_analyze > total_frames)
         frames_to_analyze = total_frames;
 
-    if (pack.bg_algo != "hist") { // GetBGAlgo :27-37 + the switch default :255-260
+    int percent = 50;
+    if (!background_percent(pack.bg_algo, &percent)) { // GetBGAlgo :27-37 + the switch default :255-260
         std::cerr << "Unknown background algorithm detected: " << pack.bg_algo << '\n';
         std::cerr << "tried to get vid background with unknown algorithm: " << pack.bg_algo << '\n';
         return py::none();
@@ -498,9 +526,10 @@ py::object GetVideoBackground(const VidBgPack &pack)
         t_gen.stop();
         if (!algo_p && !sharded_p) {
             if (on_device && devices.size() > 1) {
-                sharded_p = std::make_unique<GpuShardedMedianAlgo>(devices, frames_to_analyze, vid.format_for(rows, cols, channels));
+                sharded_p = std::make_unique<GpuShardedMedianAlgo>(devices, frames_to_analyze, vid.format_for(rows, cols, channels),
+                                                                   percent);
             } else {
-                GpuMedianPack mp{devices[0], frames_to_analyze, {}};
+                GpuMedianPack mp{devices[0], frames_to_analyze, {}, percent};
                 if (on_device)
                     mp.source = vid.format_for(rows, cols, channels);
                 algo_p = std::make_unique<GpuMedianAlgo>(mp);
@@ -589,6 +618,28 @@ int background_window(const py::dict &kwargs)
     return int(v);
 }
 
+// kwargs["cvvp_background_percentile"]: 50 when absent, else an int (not a bool) in [0, 100] -- and only together with a
+// window: the static path computes no background (RuntimeError otherwise)
+int background_percentile(const py::dict &kwargs)
+{
+    if (!kwargs.contains("cvvp_background_percentile"))
+        return 50;
+    CVVP_ASSERT_MSG(kwargs.contains("cvvp_background_window"),
+                    "kwargs['cvvp_background_percentile'] needs kwargs['cvvp_background_window']: only the rolling "
+                    "background has a percentile");
+    py::object p = kwargs["cvvp_background_percentile"];
+    bool ok = PyIndex_Check(p.ptr()) && !PyBool_Check(p.ptr());
+    long long v = 0;
+    if (ok) {
+        int overflow = 0;
+        py::int_ ip = py::reinterpret_steal<py::int_>(PyNumber_Index(p.ptr()));
+        v = PyLong_AsLongLongAndOverflow(ip.ptr(), &overflow);
+        ok = overflow == 0 && v >= 0 && v <= 100;
+    }
+    CVVP_ASSERT_MSG(ok, "kwargs['cvvp_background_percentile'] must be an int in [0, 100]");
+    return int(v);
+}
+
 py::dict TrackObjects(const VidObjectTrackPack &pack)
 {
     // Opt-in extra of this implementation (the reference has no counterpart): kwargs["cvvp_background_window"] = W
@@ -597,7 +648,10 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     // then only validated (non-empty, the cropped frame's size) and not used for the masks.  Checked before any
     // device work.  The masks reach the callback in frame order as always, but later than their frames are decoded
     // (up to W - 1 frames).  With several devices in CVVP_DEVICES this mode runs on the first one.
+    // kwargs["cvvp_background_percentile"] = P (with a window) makes that background the window's percentile P instead
+    // of its upper median (P = 50).
     const int roll_window = background_window(pack.assign_objects_pack.kwargs);
+    const int roll_percent = background_percentile(pack.assign_objects_pack.kwargs);
     const bool rolling = roll_window > 0;
     FrameSource vid{pack.vid_path, pack.grayscale, pack.vid_is_grayscale};
     if (!vid.opened()) {
@@ -895,7 +949,7 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
                                     "(cv::findContours requires 8UC1)");
                 }
                 if (rolling)
-                    roller = std::make_unique<GpuRollingHighlightAlgo>(std::move(hp), roll_window);
+                    roller = std::make_unique<GpuRollingHighlightAlgo>(std::move(hp), roll_window, roll_percent);
                 else
                     highlighter = std::make_unique<GpuHighlightAlgo>(std::move(hp));
             }

@@ -2,7 +2,8 @@
 // (/root/reference/Sources/ProcessorAlgos/histogram_median_algo.h:116-193).
 //
 // The reference builds a 256-bin histogram per element and returns the first bin whose
-// cumulative count exceeds N/2, i.e. sorted[N/2].  On B200 a shared-memory histogram costs one
+// cumulative count exceeds N/2, i.e. sorted[N/2].  Every form here selects sorted[k(N, p)] instead
+// (percentile_rank, median_common.cuh), which is sorted[N/2] at the default p = 50.  On B200 a shared-memory histogram costs one
 // (atomic) read-modify-write per input byte and cannot keep up with HBM, so this kernel computes
 // the same order statistic with an on-chip BIT-SLICED RADIX SELECT:
 //
@@ -31,7 +32,7 @@
 namespace cvvp
 {
 int median_launch(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
-                  uint8_t *d_out, cudaStream_t stream)
+                  uint8_t *d_out, int percent, cudaStream_t stream)
 {
     if (!d_out)
         return fail(ctx, CVVP_ERR_INVALID, "median: null output pointer");
@@ -54,14 +55,15 @@ int median_launch(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, siz
             return fail(ctx, CVVP_ERR_UNSUPPORTED, "median: %lld frames exceed the supported maximum (%lld)", nframes,
                         median_two_pass_max_frames());
         const char *win = getenv("CVVP_MEDIAN_WINDOW");
-        return median_long_stack(ctx, d_frames, nframes, nelem, frame_stride, d_out, stream, win ? win[0] != '0' : 1);
+        return median_long_stack(ctx, d_frames, nframes, nelem, frame_stride, d_out, percent, stream, win ? win[0] != '0' : 1);
     }
-    return median_launch_mode(ctx, d_frames, nframes, nelem, frame_stride, d_out, 0, ShardPush{}, stream);
+    return median_launch_mode(ctx, d_frames, nframes, nelem, frame_stride, d_out, 0, percent, ShardPush{}, stream);
 }
 
-// mode 0: on-chip select into d_out; modes 1 / 2: the two counting rounds of a frame-sharded job (median_shard.cu)
+// mode 0: on-chip select into d_out; modes 1 / 2 / 3: the counting rounds of a frame-sharded job (median_shard.cu).
+// percent: the order statistic modes 0 and 3 select (percentile_rank, median_common.cuh)
 int median_launch_mode(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
-                       uint8_t *d_out, int mode, const ShardPush &push, cudaStream_t stream)
+                       uint8_t *d_out, int mode, int percent, const ShardPush &push, cudaStream_t stream)
 {
     if (!d_frames || nframes <= 0 || nelem == 0)
         return fail(ctx, CVVP_ERR_INVALID, "median: null pointer or empty stack");
@@ -70,6 +72,8 @@ int median_launch_mode(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes
                     "median: device stack must be 16-byte aligned with a frame stride that is a multiple of 16 and >= nelem");
     if (nelem >= (1ull << 31))
         return fail(ctx, CVVP_ERR_UNSUPPORTED, "median: more than 2^31 elements per frame");
+    if (percent < 0 || percent > 100)
+        return fail(ctx, CVVP_ERR_INVALID, "median: percentile %d outside [0, 100]", percent);
     if (nframes > median_max_frames())
         return fail(ctx, CVVP_ERR_UNSUPPORTED, "median: %lld frames exceed the on-chip select capacity (%lld)", nframes,
                     median_max_frames());
@@ -101,6 +105,6 @@ int median_launch_mode(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes
                                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (cr != CUDA_SUCCESS)
         return fail(ctx, CVVP_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", int(cr));
-    return median_pipe_launch(ctx, tmap, log2s, d_out, uint32_t(nelem), uint32_t(nframes), nst, mode, push, stream);
+    return median_pipe_launch(ctx, tmap, log2s, d_out, uint32_t(nelem), uint32_t(nframes), nst, mode, uint32_t(percent), push, stream);
 }
 } // namespace cvvp

@@ -1,9 +1,24 @@
-// Shared device helpers of the median kernels: single-LOP3 bit select and the in-register 32x32 bit transpose.
+// Shared helpers of the median kernels: the rank rule of every background, single-LOP3 bit select and the in-register
+// 32x32 bit transpose.
 #pragma once
 #include <cstdint>
 
 namespace cvvp
 {
+// Rank of percentile `percent` (integer, 0..100) among n values: the result is sorted[k] with
+// k = min(n - 1, floor(n * percent / 100)).  percent = 50 gives n / 2, the reference's upper median
+// (histogram_median_algo.h:160-166); 0 the minimum, 100 the maximum.  Every kernel and the host code take the rank
+// from here.  n = 0 gives 0 (no value to select).  U is the unsigned type of the arithmetic: the host uses 64 bits;
+// the kernels use 32, which is exact while n * 100 < 2^32 (their n is at most 16 x 65535 frames) and keeps the
+// per-element cost of the owner kernels at that of the n / 2 it replaced (a multiply-high, not a 64-bit division).
+template <typename U>
+__host__ __device__ __forceinline__ U percentile_rank(U n, uint32_t percent)
+{
+    static_assert(U(-1) > U(0), "unsigned arithmetic");
+    const U k = n * U(percent) / U(100);
+    return k < n ? k : (n ? n - U(1) : U(0));
+}
+
 // bitwise select: (a & m) | (b & ~m) as ONE LOP3 (ptxas does not fuse the two-mask C expression)
 __device__ __forceinline__ uint32_t bitsel(uint32_t a, uint32_t b, uint32_t m)
 {

@@ -15,8 +15,10 @@
 //            values costs one update.  Neighbouring elements of a video background have neighbouring values, so the
 //            updates of a warp land in few planes.  HBM/L2-bound integer work at about three times the rate of the
 //            PCIe link that feeds the job; abi.cu overlaps it with the uploads (two stack halves).
-//   select : one thread per element accumulates the 256 planes (coalesced) until the count exceeds N/2.
+//   select : one thread per element accumulates the 256 planes (coalesced) until the count exceeds k(N, p)
+//            (percentile_rank; N/2 at the default p = 50).
 #include "context.hpp"
+#include "median_common.cuh"
 
 namespace cvvp
 {
@@ -57,18 +59,18 @@ __global__ void __launch_bounds__(kHistThreads) median_hist_fold_kernel(const ui
 }
 
 __global__ void __launch_bounds__(kHistThreads) median_hist_select_kernel(const uint32_t *__restrict__ hist, const size_t plane,
-                                                                           const uint32_t nelem, const unsigned long long total,
+                                                                           const uint32_t nelem, const unsigned long long rank,
                                                                            uint8_t *__restrict__ out)
 {
     const uint32_t e = blockIdx.x * kHistThreads + threadIdx.x;
     if (e >= nelem)
         return;
-    const unsigned long long half = total / 2ull; // first bin whose cumulative count exceeds N/2 (:160-166)
+    // first bin whose cumulative count exceeds the rank (N/2 at p = 50: the reference's rule, :160-166)
     unsigned long long cum = 0;
     uint32_t v = 0;
     for (; v < 255u; ++v) {
         cum += __ldcs(hist + size_t(v) * plane + e);
-        if (cum > half)
+        if (cum > rank)
             break;
     }
     out[e] = uint8_t(v);
@@ -97,11 +99,12 @@ int median_hist_fold(cvvp_ctx *ctx, const uint8_t *d_stack, long long nframes, s
     return CVVP_OK;
 }
 
-int median_hist_select(cvvp_ctx *ctx, const uint32_t *d_hist, size_t frame_stride, size_t nelem, long long total, uint8_t *d_out,
-                       cudaStream_t stream)
+int median_hist_select(cvvp_ctx *ctx, const uint32_t *d_hist, size_t frame_stride, size_t nelem, long long total, int percent,
+                       uint8_t *d_out, cudaStream_t stream)
 {
     const uint32_t grid = uint32_t((nelem + kHistThreads - 1) / kHistThreads);
-    median_hist_select_kernel<<<grid, kHistThreads, 0, stream>>>(d_hist, frame_stride, uint32_t(nelem), (unsigned long long)total, d_out);
+    median_hist_select_kernel<<<grid, kHistThreads, 0, stream>>>(d_hist, frame_stride, uint32_t(nelem),
+                                                                  percentile_rank<uint64_t>(uint64_t(total), uint32_t(percent)), d_out);
     CVVP_CUDA_OK(ctx, cudaGetLastError());
     ctx->launches++;
     return CVVP_OK;

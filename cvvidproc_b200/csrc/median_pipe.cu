@@ -178,14 +178,15 @@ __device__ __forceinline__ void window_row(uint32_t (&acc)[4], uint32_t &below, 
 // LOG2S : log2(32-frame sub-blocks per stage per element); P = 128 >> LOG2S elements per tile
 // JT    : stages per select thread (compile time)
 // NSELW : select warps, 8 (two stage classes, two plane buffers) or 16 (four stage classes, one plane buffer)
-// MODE  : 0 = select the median on chip (single-GPU job)
+// MODE  : 0 = select the percentile on chip (single-GPU job): rank percentile_rank(nframes, percent), the upper
+//             median at percent = 50
 //         1 = frame-sharded job, round 1: 16-bin counts of the HIGH nibble of this rank's frames, pushed to the
 //             element's owner rank through peer memory
 //         2 = round 2: 16-bin counts of the LOW nibble among the frames whose high nibble equals the globally selected
 //             one (push.sel[e] & 15), pushed the same way
 //         3 = frame-sharded job / long stack in ONE pass over the frames: every element's select threads first pick a
-//             PILOT median of two of their plane rows (256 of the launch's <= 1024 frames) on chip, then count all
-//             frames in the 8-value window [pilot - 4, pilot + 3] (8 bins) and below it, and push
+//             PILOT (the same percentile of two of their plane rows: 256 of the launch's <= 1024 frames) on chip, then
+//             count all frames in the 8-value window [pilot - 4, pilot + 3] (8 bins) and below it, and push
 //             {8 x u16 bins, below | window base << 16} (20 B) to the element's owner (the launch's frame count goes to
 //             a header word per owner).  The owner can name the median of
 //             ALL sources exactly whenever it lies inside every source's window (shard_window_final_kernel); elements
@@ -194,7 +195,7 @@ template <int LOG2S, int JT, int NSELW, int MODE>
 __global__ void __launch_bounds__((NSELW + kTrWarps) * 32, 1)
     median_pipe_kernel(const __grid_constant__ CUtensorMap tmap, uint8_t *__restrict__ out, const uint32_t nelem,
                        const uint32_t nframes, const uint32_t nst, const uint32_t ntiles, const uint64_t l2_policy,
-                       const __grid_constant__ ShardPush push)
+                       const uint32_t percent, const __grid_constant__ ShardPush push)
 {
     constexpr int S = 1 << LOG2S;
     constexpr int P = 128 >> LOG2S;
@@ -416,7 +417,8 @@ __global__ void __launch_bounds__((NSELW + kTrWarps) * 32, 1)
     // element of (transposer lane c, register block p): byte p of word c, or what the matrix loads deliver
     const uint32_t s_elem = kLdsm ? 64u * (s_p >> 1) + 16u * (s_c & 3u) + 8u * (s_p & 1u) + (s_c >> 2) : 4u * s_c + s_p;
     const bool s_writer = (s_g == 0u) && ((lane >> kColBits) == 0u);
-    const uint32_t k0 = nframes / 2u + (nst * kSlotsPerStage - nframes); // wanted rank incl. zero pad slots
+    // wanted rank incl. zero pad slots
+    const uint32_t k0 = percentile_rank(nframes, percent) + (nst * kSlotsPerStage - nframes);
     const uint32_t zero = nst >> 8; // 0 (nst <= 32), but not to the compiler: see landed()
 
     for (uint32_t it = 0; it < my_tiles; ++it) {
@@ -470,7 +472,7 @@ __global__ void __launch_bounds__((NSELW + kTrWarps) * 32, 1)
 #pragma unroll
                 for (int i = 0; i < JP; ++i)
                     alive[i] = (G * pilot_row(i) + s_g) < nst ? 0xFFFFFFFFu : 0u;
-                uint32_t k = p_real / 2u + (p_slots - p_real);
+                uint32_t k = percentile_rank(p_real, percent) + (p_slots - p_real);
 #pragma unroll
                 for (int bit = 7; bit >= 0; --bit) {
                     uint32_t cnt = 0;
@@ -812,7 +814,7 @@ __global__ void __launch_bounds__((NSELW + kTrWarps) * 32, 1)
 
 template <int LOG2S, int JT, int NSELW, int MODE>
 int launch_pipe_variant(cvvp_ctx *ctx, const CUtensorMap &tmap, uint8_t *d_out, uint32_t nelem, uint32_t nframes,
-                        uint32_t nst, const ShardPush &push, cudaStream_t stream)
+                        uint32_t nst, uint32_t percent, const ShardPush &push, cudaStream_t stream)
 {
     constexpr int P = 128 >> LOG2S;
     constexpr uint32_t G = NSELW / 4;
@@ -827,7 +829,7 @@ int launch_pipe_variant(cvvp_ctx *ctx, const CUtensorMap &tmap, uint8_t *d_out, 
     // P == 128: every line is read exactly once -> evict-first.  P < 128: the neighbouring CTA reads the other part
     // of the line at about the same time and should hit L2.
     const uint64_t policy = (LOG2S == 0) ? kL2EvictFirst : kL2EvictNormal;
-    kern<<<grid, (NSELW + kTrWarps) * 32, smem_bytes, stream>>>(tmap, d_out, nelem, nframes, nst, ntiles, policy, push);
+    kern<<<grid, (NSELW + kTrWarps) * 32, smem_bytes, stream>>>(tmap, d_out, nelem, nframes, nst, ntiles, policy, percent, push);
     CVVP_CUDA_OK(ctx, cudaGetLastError());
     ctx->launches++;
     return CVVP_OK;
@@ -835,12 +837,12 @@ int launch_pipe_variant(cvvp_ctx *ctx, const CUtensorMap &tmap, uint8_t *d_out, 
 
 template <int LOG2S, int NSELW, int MODE>
 int dispatch_jt(cvvp_ctx *ctx, const CUtensorMap &tmap, uint8_t *d_out, uint32_t nelem, uint32_t nframes, uint32_t nst,
-                const ShardPush &push, cudaStream_t stream)
+                uint32_t percent, const ShardPush &push, cudaStream_t stream)
 {
     constexpr uint32_t G = NSELW / 4;
     switch ((nst + G - 1u) / G) {
 #define CVVP_JT_CASE(J) \
-    case J: return launch_pipe_variant<LOG2S, J, NSELW, MODE>(ctx, tmap, d_out, nelem, nframes, nst, push, stream);
+    case J: return launch_pipe_variant<LOG2S, J, NSELW, MODE>(ctx, tmap, d_out, nelem, nframes, nst, percent, push, stream);
         CVVP_JT_CASE(1)
         CVVP_JT_CASE(2)
         CVVP_JT_CASE(3)
@@ -856,26 +858,26 @@ int dispatch_jt(cvvp_ctx *ctx, const CUtensorMap &tmap, uint8_t *d_out, uint32_t
 
 template <int LOG2S, int MODE>
 int dispatch_bufs(cvvp_ctx *ctx, const CUtensorMap &tmap, uint8_t *d_out, uint32_t nelem, uint32_t nframes, uint32_t nst,
-                  const ShardPush &push, cudaStream_t stream)
+                  uint32_t percent, const ShardPush &push, cudaStream_t stream)
 {
     const char *e = getenv("CVVP_MEDIAN_BUFFERS"); // development switch: "1" forces the single-buffer mode
     const bool force_single = e && e[0] == '1';
     if (nst <= 16 && !force_single)
-        return dispatch_jt<LOG2S, 8, MODE>(ctx, tmap, d_out, nelem, nframes, nst, push, stream);
-    return dispatch_jt<LOG2S, 16, MODE>(ctx, tmap, d_out, nelem, nframes, nst, push, stream);
+        return dispatch_jt<LOG2S, 8, MODE>(ctx, tmap, d_out, nelem, nframes, nst, percent, push, stream);
+    return dispatch_jt<LOG2S, 16, MODE>(ctx, tmap, d_out, nelem, nframes, nst, percent, push, stream);
 }
 
 template <int LOG2S>
 int dispatch_mode(cvvp_ctx *ctx, const CUtensorMap &tmap, uint8_t *d_out, uint32_t nelem, uint32_t nframes, uint32_t nst,
-                  int mode, const ShardPush &push, cudaStream_t stream)
+                  int mode, uint32_t percent, const ShardPush &push, cudaStream_t stream)
 {
     switch (mode) {
-    case 0: return dispatch_bufs<LOG2S, 0>(ctx, tmap, d_out, nelem, nframes, nst, push, stream);
-    case 1: return dispatch_bufs<LOG2S, 1>(ctx, tmap, d_out, nelem, nframes, nst, push, stream);
-    case 2: return dispatch_bufs<LOG2S, 2>(ctx, tmap, d_out, nelem, nframes, nst, push, stream);
+    case 0: return dispatch_bufs<LOG2S, 0>(ctx, tmap, d_out, nelem, nframes, nst, percent, push, stream);
+    case 1: return dispatch_bufs<LOG2S, 1>(ctx, tmap, d_out, nelem, nframes, nst, percent, push, stream);
+    case 2: return dispatch_bufs<LOG2S, 2>(ctx, tmap, d_out, nelem, nframes, nst, percent, push, stream);
     case 3:
         if constexpr (LOG2S == 0)
-            return dispatch_jt<0, 16, 3>(ctx, tmap, d_out, nelem, nframes, nst, push, stream);
+            return dispatch_jt<0, 16, 3>(ctx, tmap, d_out, nelem, nframes, nst, percent, push, stream);
         else
             return fail(ctx, CVVP_ERR_UNSUPPORTED, "median: window counting takes at most 1024 frames per launch");
     default: return fail(ctx, CVVP_ERR_INVALID, "median: bad kernel mode %d", mode);
@@ -890,15 +892,16 @@ long long median_max_frames()
 }
 
 int median_pipe_launch(cvvp_ctx *ctx, const CUtensorMap &tmap, int log2s, uint8_t *d_out, uint32_t nelem,
-                       uint32_t nframes, uint32_t nst, int mode, const ShardPush &push, cudaStream_t stream)
+                       uint32_t nframes, uint32_t nst, int mode, uint32_t percent, const ShardPush &push,
+                       cudaStream_t stream)
 {
     if (nst == 0 || nst > 32)
         return fail(ctx, CVVP_ERR_UNSUPPORTED, "median: %u stages exceed the plane buffer", nst);
     switch (log2s) {
-    case 0: return dispatch_mode<0>(ctx, tmap, d_out, nelem, nframes, nst, mode, push, stream);
-    case 1: return dispatch_mode<1>(ctx, tmap, d_out, nelem, nframes, nst, mode, push, stream);
-    case 2: return dispatch_mode<2>(ctx, tmap, d_out, nelem, nframes, nst, mode, push, stream);
-    case 3: return dispatch_mode<3>(ctx, tmap, d_out, nelem, nframes, nst, mode, push, stream);
+    case 0: return dispatch_mode<0>(ctx, tmap, d_out, nelem, nframes, nst, mode, percent, push, stream);
+    case 1: return dispatch_mode<1>(ctx, tmap, d_out, nelem, nframes, nst, mode, percent, push, stream);
+    case 2: return dispatch_mode<2>(ctx, tmap, d_out, nelem, nframes, nst, mode, percent, push, stream);
+    case 3: return dispatch_mode<3>(ctx, tmap, d_out, nelem, nframes, nst, mode, percent, push, stream);
     default: return fail(ctx, CVVP_ERR_INVALID, "median: bad tile variant");
     }
 }

@@ -1,16 +1,16 @@
-// Rolling temporal median on sm_100a: the background of frame t is the per-element upper median of a window of W
-// frames centred on t, shifted (not shortened) at both ends of the stream:
+// Rolling temporal median on sm_100a: the background of frame t is the per-element percentile p (the upper median at the
+// default p = 50) of a window of W frames centred on t, shifted (not shortened) at both ends of the stream:
 //
 //   N <= W : every frame's window is all N frames
 //   N >  W : s(t) = min(max(t - W/2, 0), N - W), window = frames s(t) .. s(t) + W - 1
-//   B_t[e] = min{v : #{window values <= v} > Weff/2}  (Weff = min(W, N); the reference's rule,
-//            /root/reference/Sources/ProcessorAlgos/histogram_median_algo.h:160-166)
+//   B_t[e] = min{v : #{window values <= v} > k}  (Weff = min(W, N), k = k(Weff, p) of percentile_rank; k = Weff/2 at
+//            p = 50 is the reference's rule, /root/reference/Sources/ProcessorAlgos/histogram_median_algo.h:160-166)
 //
 // Incremental form.  One CTA owns a tile of kRollE consecutive elements (one thread each) and a chunk of consecutive
 // outputs.  Every element keeps a 256-bin histogram of its window on chip with 16-bit counts (W <= 65535, so counts
 // never saturate and the result is exact), plus the current median m and lt = #{window values < m}.  The CTA builds
 // the histograms once from the W rows of its first window; every later output whose window moves adds the entering
-// row and removes the leaving one, updates lt against m and walks m until lt <= Weff/2 < lt + h[m] holds again (a
+// row and removes the leaving one, updates lt against m and walks m until lt <= k < lt + h[m] holds again (a
 // level or two on sensor noise, at most 255 steps on a scene cut).  Outputs whose window does not move (the clamped
 // ends) repeat m.
 //
@@ -22,6 +22,7 @@
 // the output count allows, so reads stay below 3 bytes per output element.  Frames may live in a ring (frame i at
 // frames + (i % ring) * stride): the streaming operator of highlight_rolling.cu keeps only W + max_batch frames.
 #include "context.hpp"
+#include "median_common.cuh"
 
 namespace cvvp
 {
@@ -38,6 +39,7 @@ struct RollArgs {
     long long nframes;  // N: the windows clamp to it
     long long half_w;   // W / 2
     long long weff;     // min(W, N)
+    uint32_t rank;      // k(Weff, p): the window's order statistic
     long long t0, t1;   // outputs [t0, t1)
     long long chunk;    // outputs per CTA
     uint8_t *out;       // B_t at out + (t - t0) * out_stride
@@ -95,9 +97,9 @@ __global__ void __launch_bounds__(kRollE) median_roll_kernel(const RollArgs a)
             if (v[j] < 256u)
                 bin_add(h, v[j]);
     }
-    const uint32_t half = uint32_t(a.weff / 2);
+    const uint32_t rank = a.rank;
     uint32_t m = 0, lt = 0;
-    for (uint32_t c = bin_count(h, 0); lt + c <= half; c = bin_count(h, m)) {
+    for (uint32_t c = bin_count(h, 0); lt + c <= rank; c = bin_count(h, m)) {
         lt += c;
         ++m;
     }
@@ -128,11 +130,11 @@ __global__ void __launch_bounds__(kRollE) median_roll_kernel(const RollArgs a)
                 bin_add(h, vin[j]);
                 bin_sub(h, vout[j]);
                 lt = lt + (vin[j] < m) - (vout[j] < m);
-                while (lt > half) {
+                while (lt > rank) {
                     --m;
                     lt -= bin_count(h, m);
                 }
-                for (uint32_t c = bin_count(h, m); lt + c <= half; c = bin_count(h, m)) {
+                for (uint32_t c = bin_count(h, m); lt + c <= rank; c = bin_count(h, m)) {
                     lt += c;
                     ++m;
                 }
@@ -145,11 +147,13 @@ __global__ void __launch_bounds__(kRollE) median_roll_kernel(const RollArgs a)
 } // namespace
 
 int median_roll_launch(cvvp_ctx *ctx, const uint8_t *d_frames, long long ring, size_t frame_stride, long long nframes,
-                       size_t nelem, int window, long long t0, long long t1, uint8_t *d_out, size_t out_stride,
-                       cudaStream_t stream)
+                       size_t nelem, int window, int percent, long long t0, long long t1, uint8_t *d_out,
+                       size_t out_stride, cudaStream_t stream)
 {
     if (window < 1 || window > 65535)
         return fail(ctx, CVVP_ERR_INVALID, "rolling median: window %d outside [1, 65535]", window);
+    if (percent < 0 || percent > 100)
+        return fail(ctx, CVVP_ERR_INVALID, "rolling median: percentile %d outside [0, 100]", percent);
     if (!d_frames || !d_out || nframes < 1 || nelem == 0 || t0 < 0 || t1 > nframes || t0 > t1)
         return fail(ctx, CVVP_ERR_INVALID, "rolling median: bad arguments (need 0 <= t0 <= t1 <= nframes, nframes >= 1, nelem >= 1)");
     if (frame_stride < nelem || out_stride < nelem)
@@ -182,6 +186,7 @@ int median_roll_launch(cvvp_ctx *ctx, const uint8_t *d_frames, long long ring, s
     a.nframes = nframes;
     a.half_w = window / 2;
     a.weff = weff;
+    a.rank = uint32_t(percentile_rank<uint64_t>(uint64_t(weff), uint32_t(percent)));
     a.t0 = t0;
     a.t1 = t1;
     a.chunk = chunk;

@@ -3,7 +3,9 @@
 //
 // The reference's analogue is its temporal sharding of the frame range over generator threads
 // (/root/reference/Sources/cv_vid_bg_helpers.cpp:84-120) feeding one order-independent histogram
-// (histogram_median_algo.h:116-141); the result is the same sorted[N/2] of ALL frames (:160-166).
+// (histogram_median_algo.h:116-141); the result is the same sorted[N/2] of ALL frames (:160-166) -- in general
+// sorted[k(N, p)] for the job's percentile p (percentile_rank, median_common.cuh; the owner kernels below take the rank
+// from there, and the window test and the nibble rounds are exact for any rank).
 //
 // Every rank holds a chunk of the frames (all elements).  Element e is OWNED by rank e / slice.  Instead of
 // all-reducing 256-bin histograms (512 B per element), the select is a two-round radix select on nibbles, and
@@ -12,7 +14,7 @@
 //   phase 0  every rank : 16-bin counts of the HIGH nibble of its frames (median_pipe_kernel MODE 1, the same
 //                         TMA -> bit-transpose pipeline as the single-GPU kernel), 32 B per element stored into
 //                         owner's  counts1[src rank][e - owner * slice]
-//   phase 1  owner      : sums the `world` count vectors, N = their total, k = N / 2, picks the high nibble h with
+//   phase 1  owner      : sums the `world` count vectors, N = their total, k = k(N, p), picks the high nibble h with
 //                         cum(h) > k and the residual rank k' = k - cum(< h); stores  sel[e] = h | k' << 8  into
 //                         EVERY rank's sel array (4 B per element)
 //   phase 2  every rank : 16-bin counts of the LOW nibble among its frames with high nibble == h (MODE 2), pushed
@@ -25,8 +27,8 @@
 // median of 256 of its own frames on chip and counts ALL its frames in the 8-value window [pilot - 4, pilot + 3]
 // and below it; the 20-byte record {8 x u16 bins, below | window base << 16} goes to the element's owner like the
 // nibble counts do (the launch's frame count goes to one header word per owner).  Phase 5 (shard_window_final_kernel, owner): the cumulative count of all sources is exact on the
-// intersection [lo - 1, hi] of their windows, so whenever G(lo - 1) <= N/2 < G(hi) the median is the first value
-// there with G(v) > N/2 -- the reference's rule (:160-166) -- and it is stored into every rank's result image.
+// intersection [lo - 1, hi] of their windows, so whenever G(lo - 1) <= k < G(hi) the result is the first value
+// there with G(v) > k -- the reference's rule (:160-166) at k = N/2 -- and it is stored into every rank's result image.
 // Elements whose median lies outside some source's window (sources with very different content) are counted into
 // every rank's `unresolved` word and their 128-element tile is flagged on every rank; the job then runs phases
 // 10..13 = phases 0..3 restricted to the flagged tiles (the counting kernels walk a compacted tile list, the owner
@@ -40,6 +42,7 @@
 // 2 x 32 B x (world-1)/world in, + 5 B broadcast -- 8x less than all-reducing 256 x u16 histograms, and the two
 // passes over the frames stay at HBM speed.
 #include "context.hpp"
+#include "median_common.cuh"
 
 #include <algorithm>
 #include <cstdlib>
@@ -70,6 +73,7 @@ struct MedianShard {
     size_t off_bar{0};   // [kMaxShardRanks] words: bar[r] = the last barrier epoch rank r has arrived at (cvvp_median_shard_barrier)
     uint32_t ntiles{0};
     uint32_t epoch{0};   // barriers this rank has issued
+    int percent{50};     // the percentile this rank selects (every rank of a job must use the same)
 };
 
 // frames one launch of the counting kernel takes at full tile width (128-byte TMA boxes): 32 stages x 32 frames
@@ -91,6 +95,7 @@ struct OwnerArgs {
     const uint32_t *tile_list;        // restricted rounds: the flagged tiles and how many there are
     const uint32_t *tile_count;
     const uint32_t *src_frames;       // window pass: frames behind every source slot's records (0: skip the slot)
+    uint32_t percent;                 // the job's percentile: rank k(N, percent) of the N frames of all sources
 };
 
 // the s-th vector / record of the round lives in slot (s % used) of rank (s / used)
@@ -124,7 +129,8 @@ __device__ __forceinline__ void pick_element(const OwnerArgs &A, uint32_t i)
 #pragma unroll
     for (int b = 0; b < 16; ++b)
         total += cnt[b];
-    const uint32_t k = total / 2u; // halfway rank: first bin with cumulative count > N / 2  (:160-166)
+    // first bin with cumulative count > k(N, p)  (N / 2 at p = 50: the reference's rule, :160-166)
+    const uint32_t k = percentile_rank(total, A.percent);
     uint32_t h = 15u, below = 0u, cum = 0u;
     bool found = false;
 #pragma unroll
@@ -310,7 +316,8 @@ __global__ void __launch_bounds__(256) shard_window_final_kernel(const __grid_co
         bool ok = true;
         if (mine) {
             ok = false;
-            const uint32_t k = total / 2u; // halfway rank: first value with cumulative count > N / 2  (:160-166)
+            // first value with cumulative count > k(N, p)  (N / 2 at p = 50: the reference's rule, :160-166)
+            const uint32_t k = percentile_rank(total, A.percent);
             if (total != 0u && !far && lo <= hi) {
                 // G(lo - 1) = frames below every window + the counted values <= lo - 1; G is exact up to hi
                 const uint32_t p0 = lo - base0 + 7u; // position of value lo
@@ -474,6 +481,7 @@ static int shard_create(cvvp_ctx *ctx, size_t nelem, int rank, int world, int sp
     MedianShard *sh = new (std::nothrow) MedianShard();
     if (!sh)
         return fail(ctx, CVVP_ERR_NOMEM, "out of host memory");
+    sh->percent = ctx->percent; // a sharded job takes the context's percentile when it begins
     sh->rank = rank;
     sh->world = world;
     sh->spr = spr;
@@ -524,7 +532,8 @@ static int shard_count_slot(cvvp_ctx *ctx, MedianShard *sh, int phase, const uin
         return CVVP_OK;
     }
     if (nframes <= kChunkFrames)
-        return median_launch_mode(ctx, d_frames, nframes, sh->nelem, frame_stride, nullptr, phase == 0 ? 1 : 2, push, s);
+        return median_launch_mode(ctx, d_frames, nframes, sh->nelem, frame_stride, nullptr, phase == 0 ? 1 : 2, sh->percent,
+                                  push, s);
     // long chunk of frames: several launches at full tile width; the counts of launch c are added to those of
     // launches < c in a local array, the last launch pushes the totals to the owners
     if (!sh->accum && cudaMalloc(reinterpret_cast<void **>(&sh->accum), sh->nelem * 32u) != cudaSuccess) {
@@ -547,7 +556,7 @@ static int shard_count_slot(cvvp_ctx *ctx, MedianShard *sh, int phase, const uin
             cp.slice = 0x80000000u;
         }
         const int rc = median_launch_mode(ctx, d_frames + size_t(first) * frame_stride, n, sh->nelem, frame_stride, nullptr,
-                                          phase == 0 ? 1 : 2, cp, s);
+                                          phase == 0 ? 1 : 2, sh->percent, cp, s);
         if (rc != CVVP_OK)
             return rc;
     }
@@ -595,7 +604,7 @@ static int shard_window_count(cvvp_ctx *ctx, MedianShard *sh, const uint8_t *d_f
             continue;
         }
         const int rc = median_launch_mode(ctx, d_frames + size_t(first) * frame_stride, n, sh->nelem, frame_stride, nullptr, 3,
-                                          push, s);
+                                          sh->percent, push, s);
         if (rc != CVVP_OK)
             return rc;
     }
@@ -666,6 +675,7 @@ static int shard_phase(cvvp_ctx *ctx, MedianShard *sh, int phase, const uint8_t 
         A.tile_list = tlist;
         A.tile_count = tcount;
         A.src_frames = reinterpret_cast<const uint32_t *>(sh->buf + sh->off_hdr);
+        A.percent = uint32_t(sh->percent);
         for (int r = 0; r < sh->world; ++r) {
             A.flag[r] = reinterpret_cast<uint32_t *>(sh->peer[r] + sh->off_flag);
             A.tflag[r] = reinterpret_cast<uint32_t *>(sh->peer[r] + sh->off_tflag);
@@ -717,7 +727,7 @@ long long median_two_pass_max_frames()
 // over the frames in chunks of <= 1024 at 128-byte tiles beat one pass at the 32- or 16-byte tiles the on-chip
 // select would need beyond 2048 frames (DESIGN.md section 3).
 int median_long_stack(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes, size_t nelem, size_t frame_stride,
-                      uint8_t *d_out, cudaStream_t stream, int window)
+                      uint8_t *d_out, int percent, cudaStream_t stream, int window)
 {
     const int spr = int((nframes + kSlotFrames - 1) / kSlotFrames);
     const int wsubs = window ? int((nframes + kChunkFrames - 1) / kChunkFrames) : 1;
@@ -728,6 +738,7 @@ int median_long_stack(cvvp_ctx *ctx, const uint8_t *d_frames, long long nframes,
         if (rc != CVVP_OK)
             return rc;
     }
+    ctx->big->percent = percent; // the internal job is reused across calls: it takes each call's percentile
     if ((reinterpret_cast<uintptr_t>(d_out) & 3u) != 0) // the owner kernels store four result bytes at a time
         return fail(ctx, CVVP_ERR_INVALID, "median: the result pointer of a stack that takes the counting path (more than 1024 frames) must be 4-byte aligned");
     if (window) {

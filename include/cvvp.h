@@ -85,9 +85,25 @@ CVVP_API int cvvp_ctx_copy_to_host(cvvp_ctx *ctx, void *host_dst, const void *de
  *   saturate, which GetVideoBackground's choice guarantees (SURVEY.md 8a a5).
  *
  * An "element" is one byte of a frame (rows*cols*channels of them, cv_util.cpp:251-254); the
- * median is taken per element over all pushed frames and is the UPPER median sorted[N/2]
- * (histogram_median_algo.h:160-166).
+ * median is taken per element over all pushed frames and is sorted[k(N, p)], the upper median
+ * sorted[N/2] (histogram_median_algo.h:160-166) at the default (see cvvp_median_set_percentile).
  * ------------------------------------------------------------------------------------------- */
+
+/* Percentile backgrounds.  Every background of a context -- the streaming job, the device-resident form, the
+ * frame-sharded job and the rolling median -- is the per-element order statistic sorted[k(N, p)] of its N values
+ * (N = Weff for a rolling window), with
+ *     k(N, p) = min(N - 1, floor(N * p / 100))      (integer arithmetic, p an integer percent in [0, 100])
+ * p = 50 (the default) gives N / 2, the reference's upper median; p = 0 the minimum, p = 100 the maximum.  A higher
+ * percentile keeps dark objects that cover a pixel in a fraction c < p / 100 of the frames out of the background.
+ * The percentile is a setting of the context: jobs take it when they begin (cvvp_median_begin -- and so push,
+ * push_source and finish --, cvvp_median_shard_begin*, cvvp_highlight_rolling_begin); the device-resident forms
+ * (cvvp_median_device, cvvp_median_rolling_device) read it at the call.  CVVP_ERR_INVALID for p outside [0, 100];
+ * CVVP_ERR_STATE while a median, sharded or rolling job is open on the context.  Every rank of a sharded job must
+ * use the same percentile: the host operators of this library set it on all their contexts, but ranks in other
+ * processes are not checked for agreement. */
+CVVP_API int cvvp_median_set_percentile(cvvp_ctx *ctx, int percent);
+/* the context's percentile (50 unless set), or CVVP_ERR_INVALID for a NULL context */
+CVVP_API int cvvp_median_percentile(const cvvp_ctx *ctx);
 
 /* Start a median job on frames of `nelem` bytes.  nframes_hint > 0 sizes the device stack for exactly that many
  * frames (rounded up to 16; it grows by half if more are pushed, and the old and new stacks coexist while it does).
@@ -95,7 +111,7 @@ CVVP_API int cvvp_ctx_copy_to_host(cvvp_ctx *ctx, void *host_dst, const void *de
  * selects the median on chip.  When the stack cannot be allocated or grown any further, the resident frames are folded
  * into per-element value histograms (256 x round_up(nelem, 128) x 4 bytes, 32-bit counts) and the stack is reused for
  * the frames that follow: from there on the job's memory is independent of the frame count, like the reference's
- * histograms (histogram_median_algo.h:123-126), and the result is the same upper median of ALL frames.
+ * histograms (histogram_median_algo.h:123-126), and the result is the same sorted[k(N, p)] of ALL frames.
  * CVVP_ERR_NOMEM only when neither a stack of 16 frames nor the histograms fit. */
 CVVP_API int cvvp_median_begin(cvvp_ctx *ctx, size_t nelem, long long nframes_hint);
 /* Append n frames from HOST memory; frame i starts at frames + i*frame_stride and holds nelem
@@ -134,8 +150,9 @@ CVVP_API int cvvp_median_device(cvvp_ctx *ctx, const uint8_t *d_frames, long lon
 /* ---------------------------------------------------------------------------------------------
  * rolling temporal median -- a background that follows the video.  The reference has one static background per
  *   TrackObjects call (Sources/cv_vid_objecttrack_helpers.cpp:167-175, the pack's background); here frame t of a
- *   stream of N frames gets the upper median (histogram_median_algo.h:160-166, sorted[Weff/2], Weff = min(W, N)) of
- *   a window of W frames centred on it and shifted, not shortened, at both ends:
+ *   stream of N frames gets sorted[k(Weff, p)] (Weff = min(W, N)), the upper median sorted[Weff/2]
+ *   (histogram_median_algo.h:160-166) at the default, of a window of W frames centred on it and shifted, not
+ *   shortened, at both ends:
  *     N <= W : every window is all N frames
  *     N >  W : window of frame t = frames s(t) .. s(t) + W - 1, s(t) = min(max(t - W/2, 0), N - W)
  * Device-resident form, layout as cvvp_median_device (frame f at d_frames + f*frame_stride, nelem bytes each, any
@@ -154,8 +171,8 @@ CVVP_API int cvvp_median_rolling_device(cvvp_ctx *ctx, const uint8_t *d_frames, 
  *   (Sources/cv_vid_bg_helpers.cpp:84-120) and merges them in ONE order-independent histogram
  *   (histogram_median_algo.h:116-141); here every rank keeps a chunk of the frames in its own HBM
  *   and the merge is a two-round exchange of 16-bin nibble counts written directly into the
- *   owner rank's memory over NVLink (csrc/median_shard.cu).  The result is the same upper median
- *   sorted[N/2] of ALL ranks' frames (:160-166), delivered to every rank.
+ *   owner rank's memory over NVLink (csrc/median_shard.cu).  The result is the same sorted[k(N, p)]
+ *   of ALL ranks' frames, the upper median sorted[N/2] (:160-166) at the default, delivered to every rank.
  *
  *   call order on every rank:
  *     cvvp_median_shard_begin
@@ -376,7 +393,7 @@ CVVP_API int cvvp_highlight_queue_end(cvvp_ctx *ctx);
 /* ---------------------------------------------------------------------------------------------
  * highlight against a rolling median background, ordered stream -- TrackObjects with a background that follows the
  *   video (see cvvp_median_rolling_device for the windows).  The mask of frame t is HighlightObjects(f_t) (highlight_
- *   objects_algo.cpp:17-78) with B_t, the rolling median of its window, in place of the pack's background.  Masks come
+ *   objects_algo.cpp:17-78) with B_t, the rolling percentile of its window, in place of the pack's background.  Masks come
  *   back LATER than their frames go in: frame t needs W - 1 frames ahead at the start of the stream and
  *   ceil(W/2) - 1 afterwards; the last ones are computed when the stream is closed (the frame count is only known
  *   then), with windows clamped to the frames pushed.  The device keeps a ring of (W + max_batch) prepared frames of
