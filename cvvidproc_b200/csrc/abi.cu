@@ -16,11 +16,6 @@ namespace
 thread_local std::string g_err;
 constexpr size_t kStagingBytes = size_t(32) << 20; // per pinned staging buffer
 constexpr int kStagingBufs = 3;
-
-size_t round_up(size_t v, size_t a)
-{
-    return (v + a - 1) / a * a;
-}
 } // namespace
 
 void set_global_error(const char *fmt, ...)
@@ -820,7 +815,7 @@ int cvvp_highlight_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, s
         return fail(nullptr, CVVP_ERR_INVALID, "null context");
     DeviceGuard guard(ctx->device);
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->compute;
-    return highlight_device(ctx, d_frames, n, frame_stride, d_out, out_stride, s);
+    return highlight_device_bg(ctx, d_frames, n, frame_stride, nullptr, 0, d_out, out_stride, CcOut(), s);
 }
 
 int cvvp_highlight_device_cc(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, uint8_t *d_out,
@@ -831,8 +826,10 @@ int cvvp_highlight_device_cc(cvvp_ctx *ctx, const uint8_t *d_frames, long long n
         return fail(nullptr, CVVP_ERR_INVALID, "null context");
     DeviceGuard guard(ctx->device);
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->compute;
-    return highlight_device_cc(ctx, d_frames, n, frame_stride, d_out, out_stride, d_comps, max_comps, d_ncomps, d_labels,
-                               labels_stride, s);
+    // components are required here, and their arguments and the path are checked before the frame arguments
+    const CcOut cc{d_comps, max_comps, d_ncomps, d_labels, labels_stride};
+    const int rc = highlight_check_cc(ctx, n, cc);
+    return rc != CVVP_OK ? rc : highlight_device_bg(ctx, d_frames, n, frame_stride, nullptr, 0, d_out, out_stride, cc, s);
 }
 
 int cvvp_highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride,
@@ -844,8 +841,11 @@ int cvvp_highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n
         return fail(nullptr, CVVP_ERR_INVALID, "null context");
     DeviceGuard guard(ctx->device);
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->compute;
-    return highlight_device_bg(ctx, d_frames, n, frame_stride, d_backgrounds, bg_stride, d_out, out_stride, d_comps, max_comps,
-                               d_ncomps, d_labels, labels_stride, s);
+    // this entry point requires backgrounds: to the internal call a null one means the job's own
+    if (!d_backgrounds && ctx->hl)
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments (null backgrounds)");
+    return highlight_device_bg(ctx, d_frames, n, frame_stride, d_backgrounds, bg_stride, d_out, out_stride,
+                               CcOut{d_comps, max_comps, d_ncomps, d_labels, labels_stride}, s);
 }
 
 int cvvp_highlight_frames_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, uint8_t *masks_out,
@@ -864,9 +864,7 @@ int cvvp_highlight_end(cvvp_ctx *ctx)
     if (!ctx)
         return fail(nullptr, CVVP_ERR_INVALID, "null context");
     DeviceGuard guard(ctx->device);
-    cudaStreamSynchronize(ctx->copy);
-    cudaStreamSynchronize(ctx->compute);
-    cudaStreamSynchronize(ctx->copy_out);
+    sync_streams(ctx);
     highlight_queue_release(ctx);
     highlight_rolling_release(ctx);
     highlight_release(ctx);

@@ -119,6 +119,11 @@ const char *global_error();
 
 int fail(cvvp_ctx *ctx, int code, const char *fmt, ...);
 
+inline size_t round_up(size_t v, size_t a)
+{
+    return (v + a - 1) / a * a;
+}
+
 #define CVVP_CUDA_OK(ctx, expr)                                                                                       \
     do {                                                                                                               \
         cudaError_t _e = (expr);                                                                                       \
@@ -171,15 +176,19 @@ long long median_two_pass_max_frames();
 void highlight_release(cvvp_ctx *ctx);
 int highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, int height, const uint8_t *selem, int kw, int kh,
                     int threshold, int threshold_lo, int threshold_hi, int min_size_hyst, int min_size_threshold);
-int highlight_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, uint8_t *d_out,
-                     size_t out_stride, cudaStream_t stream);
-int highlight_device_cc(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, uint8_t *d_out,
-                        size_t out_stride, cvvp_component *d_comps, int max_comps, int *d_ncomps, int32_t *d_labels,
-                        size_t labels_stride, cudaStream_t stream);
-// per-frame backgrounds (frame f's at d_bgs + f * bg_stride, 0 = one for all); components when d_comps != nullptr
+// optional component output of a highlight call: all pointers null = off
+struct CcOut {
+    cvvp_component *comps{nullptr}; // [frame][max_comps]
+    int max_comps{0};
+    int *ncomps{nullptr};
+    int32_t *labels{nullptr}; // [frame][labels_stride] or nullptr
+    size_t labels_stride{0};
+};
+// the component arguments are complete and the job's path can label (a highlight job must exist)
+int highlight_check_cc(cvvp_ctx *ctx, long long n, const CcOut &cc);
+// frame f against the background at d_bgs + f * bg_stride (0 = one for all; d_bgs == nullptr: the job's own)
 int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, const uint8_t *d_bgs,
-                        size_t bg_stride, uint8_t *d_out, size_t out_stride, cvvp_component *d_comps, int max_comps,
-                        int *d_ncomps, int32_t *d_labels, size_t labels_stride, cudaStream_t stream);
+                        size_t bg_stride, uint8_t *d_out, size_t out_stride, const CcOut &cc, cudaStream_t stream);
 int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, uint8_t *masks_out,
                              size_t out_stride, cvvp_component *comps_out, int max_comps, int *ncomps_out,
                              int32_t *labels_out, size_t labels_stride);
@@ -199,6 +208,42 @@ int frames_prepare_host(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_
                         uint8_t *out, size_t out_stride);
 int frames_upload_prepare(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, const cvvp_frame_format &f,
                           uint8_t *d_dst, size_t dst_stride);
+// Shared by the highlight queue and the rolling stream: the results of one batch of up to max_batch frames on their way
+// to the host, and the event that marks the end of their download.
+struct HlResults {
+    size_t npix{0}, pitch{0}; // mask bytes / pitch of the masks on both sides
+    int max_comps{0};         // 0: no components
+    bool labels{false};
+    size_t mask_bytes{0};     // of each pooled mask buffer (pool.hpp)
+    uint8_t *h_out{nullptr}, *d_out{nullptr}; // h_*: pinned
+    cvvp_component *h_comps{nullptr}, *d_comps{nullptr};
+    int *h_ncomps{nullptr}, *d_ncomps{nullptr};
+    int32_t *h_labels{nullptr}, *d_labels{nullptr};
+    cudaEvent_t down{nullptr};
+    long long n{0}; // frames of the batch
+};
+// false: out of memory (what was allocated stays for hl_results_free)
+bool hl_results_alloc(HlResults &r, long long max_batch, size_t npix, size_t pitch, int max_comps, bool labels);
+void hl_results_free(HlResults &r);
+// the n frames' component outputs, starting at frame `first` of the batch
+CcOut hl_results_cc(const HlResults &r, long long first);
+// queues the download of r.n frames after the work on the compute stream: copy_out waits, copies and records `down`
+int hl_results_download(cvvp_ctx *ctx, HlResults &r);
+// 1: downloaded, 0: not yet, < 0: the batch failed (the message starts with `who`)
+int hl_results_ready(cvvp_ctx *ctx, const HlResults &r, const char *who);
+// waits for the download; CVVP_OK or the batch's failure
+int hl_results_wait(cvvp_ctx *ctx, const HlResults &r, const char *who);
+// copies the downloaded batch into the caller's buffers (null comps / ncomps / labels: not wanted)
+void hl_results_copy(const HlResults &r, uint8_t *masks, size_t mask_stride, cvvp_component *comps, int *ncomps,
+                     int32_t *labels, size_t labels_stride);
+void sync_streams(cvvp_ctx *ctx); // copy, compute and copy_out
+// A call that failed half-way may leave work of unknown extent queued: drain the streams, keep the error, set the
+// stream's `failed` (it refuses further work until it is ended) and return rc.
+int drain_after_failure(cvvp_ctx *ctx, bool &failed, int rc);
+// Begin-time checks of a stream, in this order: a highlight job exists (*W x *H), the stream has not begun, its own
+// arguments (args_rc: the caller's checks, whose message is the last one set), and frames of the format fmt (null:
+// prepared frames) prepare to single-channel frames of the job's size.
+int highlight_stream_check(cvvp_ctx *ctx, const char *who, bool begun, int args_rc, const cvvp_frame_format *fmt, int *W, int *H);
 void highlight_queue_release(cvvp_ctx *ctx);
 int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const cvvp_frame_format *fmt, int max_comps);
 int highlight_queue_pending(const cvvp_ctx *ctx);

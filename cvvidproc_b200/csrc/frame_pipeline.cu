@@ -19,11 +19,6 @@ namespace cvvp
 {
 namespace
 {
-size_t round_up(size_t v, size_t a)
-{
-    return (v + a - 1) / a * a;
-}
-
 constexpr size_t kRawChunkBytes = size_t(64) << 20; // decoded bytes per upload chunk
 
 // the rows of a decoded frame that the crop needs: [crop_y, crop_y + crop_height), a contiguous band
@@ -188,21 +183,169 @@ int frames_prepare_host(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_
 }
 
 /* ------------------------------------------------------------------------------------------------------------------- */
+/* shared by the highlight queue and the rolling stream (highlight_rolling.cu)                                         */
+/* ------------------------------------------------------------------------------------------------------------------- */
+bool hl_results_alloc(HlResults &r, long long max_batch, size_t npix, size_t pitch, int max_comps, bool labels)
+{
+    const size_t nb = size_t(max_batch);
+    r.npix = npix;
+    r.pitch = pitch;
+    r.max_comps = max_comps;
+    r.labels = labels;
+    r.mask_bytes = nb * pitch;
+    // the masks come from the process-wide pool: a job on the next video of the same geometry reuses them
+    void *p = nullptr;
+    bool ok = pool_host_alloc(&p, r.mask_bytes) == cudaSuccess;
+    if (ok) {
+        r.h_out = static_cast<uint8_t *>(p);
+        ok = pool_dev_alloc(&p, r.mask_bytes) == cudaSuccess;
+    }
+    if (ok)
+        r.d_out = static_cast<uint8_t *>(p);
+    if (max_comps > 0) {
+        ok = ok && cudaMallocHost(&r.h_comps, nb * size_t(max_comps) * sizeof(cvvp_component)) == cudaSuccess;
+        ok = ok && cudaMallocHost(&r.h_ncomps, nb * sizeof(int)) == cudaSuccess;
+        ok = ok && cudaMalloc(&r.d_comps, nb * size_t(max_comps) * sizeof(cvvp_component)) == cudaSuccess;
+        ok = ok && cudaMalloc(&r.d_ncomps, nb * sizeof(int)) == cudaSuccess;
+    }
+    if (labels) {
+        ok = ok && cudaMallocHost(&r.h_labels, nb * npix * sizeof(int32_t)) == cudaSuccess;
+        ok = ok && cudaMalloc(&r.d_labels, nb * npix * sizeof(int32_t)) == cudaSuccess;
+    }
+    ok = ok && cudaEventCreateWithFlags(&r.down, cudaEventDisableTiming) == cudaSuccess;
+    if (!ok)
+        cudaGetLastError();
+    return ok;
+}
+
+void hl_results_free(HlResults &r)
+{
+    pool_host_free(r.h_out, r.mask_bytes);
+    pool_dev_free(r.d_out, r.mask_bytes);
+    free_host(r.h_comps);
+    free_host(r.h_ncomps);
+    free_host(r.h_labels);
+    free_dev(r.d_comps);
+    free_dev(r.d_ncomps);
+    free_dev(r.d_labels);
+    if (r.down)
+        cudaEventDestroy(r.down);
+    r = HlResults();
+}
+
+CcOut hl_results_cc(const HlResults &r, long long first)
+{
+    CcOut cc;
+    if (r.max_comps > 0) {
+        cc.comps = r.d_comps + size_t(first) * size_t(r.max_comps);
+        cc.max_comps = r.max_comps;
+        cc.ncomps = r.d_ncomps + first;
+        cc.labels = r.labels ? r.d_labels + size_t(first) * r.npix : nullptr;
+        cc.labels_stride = r.npix;
+    }
+    return cc;
+}
+
+int hl_results_download(cvvp_ctx *ctx, HlResults &r)
+{
+    const size_t n = size_t(r.n);
+    CVVP_CUDA_OK(ctx, cudaEventRecord(ctx->ev_copy, ctx->compute));
+    CVVP_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->copy_out, ctx->ev_copy, 0));
+    CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_out, r.d_out, n * r.pitch, cudaMemcpyDeviceToHost, ctx->copy_out));
+    if (r.max_comps > 0) {
+        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_comps, r.d_comps, n * size_t(r.max_comps) * sizeof(cvvp_component),
+                                          cudaMemcpyDeviceToHost, ctx->copy_out));
+        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_ncomps, r.d_ncomps, n * sizeof(int), cudaMemcpyDeviceToHost, ctx->copy_out));
+    }
+    if (r.labels)
+        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_labels, r.d_labels, n * r.npix * sizeof(int32_t), cudaMemcpyDeviceToHost,
+                                          ctx->copy_out));
+    CVVP_CUDA_OK(ctx, cudaEventRecord(r.down, ctx->copy_out));
+    return CVVP_OK;
+}
+
+int hl_results_ready(cvvp_ctx *ctx, const HlResults &r, const char *who)
+{
+    const cudaError_t e = cudaEventQuery(r.down);
+    if (e == cudaSuccess)
+        return 1;
+    if (e != cudaErrorNotReady)
+        return fail(ctx, CVVP_ERR_CUDA, "%s: %s", who, cudaGetErrorString(e));
+    return 0;
+}
+
+int hl_results_wait(cvvp_ctx *ctx, const HlResults &r, const char *who)
+{
+    const cudaError_t e = cudaEventSynchronize(r.down);
+    if (e != cudaSuccess)
+        return fail(ctx, CVVP_ERR_CUDA, "%s: batch failed: %s", who, cudaGetErrorString(e));
+    return CVVP_OK;
+}
+
+void hl_results_copy(const HlResults &r, uint8_t *masks, size_t mask_stride, cvvp_component *comps, int *ncomps,
+                     int32_t *labels, size_t labels_stride)
+{
+    const size_t n = size_t(r.n);
+    for (size_t i = 0; i < n; ++i)
+        std::memcpy(masks + i * mask_stride, r.h_out + i * r.pitch, r.npix);
+    if (r.max_comps > 0 && comps)
+        std::memcpy(comps, r.h_comps, n * size_t(r.max_comps) * sizeof(cvvp_component));
+    if (r.max_comps > 0 && ncomps)
+        std::memcpy(ncomps, r.h_ncomps, n * sizeof(int));
+    if (r.labels && labels)
+        for (size_t i = 0; i < n; ++i)
+            std::memcpy(labels + i * labels_stride, r.h_labels + i * r.npix, r.npix * sizeof(int32_t));
+}
+
+void sync_streams(cvvp_ctx *ctx)
+{
+    cudaStreamSynchronize(ctx->copy);
+    cudaStreamSynchronize(ctx->compute);
+    cudaStreamSynchronize(ctx->copy_out);
+}
+
+int drain_after_failure(cvvp_ctx *ctx, bool &failed, int rc)
+{
+    failed = true;
+    const std::string why = ctx->err;
+    sync_streams(ctx);
+    cudaGetLastError();
+    ctx->err = why;
+    return rc;
+}
+
+int highlight_stream_check(cvvp_ctx *ctx, const char *who, bool begun, int args_rc, const cvvp_frame_format *fmt, int *W, int *H)
+{
+    if (!highlight_geometry(ctx, W, H))
+        return fail(ctx, CVVP_ERR_STATE, "%s: no parameters set (call cvvp_highlight_begin first)", who);
+    if (begun)
+        return fail(ctx, CVVP_ERR_STATE, "%s: already begun", who);
+    if (args_rc != CVVP_OK)
+        return args_rc;
+    if (!fmt)
+        return CVVP_OK;
+    const int rc = frames_check_format(ctx, fmt);
+    if (rc != CVVP_OK)
+        return rc;
+    if (fmt->crop_width != *W || fmt->crop_height != *H || frames_out_bytes(*fmt) != size_t(*W) * size_t(*H))
+        return fail(ctx, CVVP_ERR_INVALID,
+                    "%s: prepared frames must be single-channel %dx%d like the background (cv::findContours requires 8UC1)",
+                    who, *W, *H);
+    return CVVP_OK;
+}
+
+/* ------------------------------------------------------------------------------------------------------------------- */
 /* asynchronous ordered highlight queue                                                                                */
 /* ------------------------------------------------------------------------------------------------------------------- */
 // A slot's pinned input holds WHOLE frames as the caller has them (decoded frames when the queue has a frame format,
 // prepared frames otherwise), one every host_pitch bytes, so that a decoder can write straight into it
 // (cvvp_highlight_slot_acquire); only the crop band of every frame crosses the link.
 struct HqSlot {
-    size_t b_h_in{0}, b_h_out{0}, b_raw{0}, b_in{0}, b_out{0}; // bytes of the pooled buffers below (pool.hpp)
-    uint8_t *h_in{nullptr}, *h_out{nullptr}; // pinned
-    cvvp_component *h_comps{nullptr};
-    int *h_ncomps{nullptr};
-    uint8_t *d_raw{nullptr}, *d_in{nullptr}, *d_out{nullptr};
-    cvvp_component *d_comps{nullptr};
-    int *d_ncomps{nullptr};
-    cudaEvent_t up{nullptr}, kdone{nullptr}, down{nullptr};
-    long long n{0};
+    size_t b_h_in{0}, b_raw{0}, b_in{0}; // bytes of the pooled buffers below (pool.hpp)
+    uint8_t *h_in{nullptr};              // pinned
+    uint8_t *d_raw{nullptr}, *d_in{nullptr};
+    cudaEvent_t up{nullptr};
+    HlResults res;
 };
 
 struct HighlightQueue {
@@ -210,7 +353,6 @@ struct HighlightQueue {
     long long max_batch{0};
     bool has_fmt{false};
     cvvp_frame_format fmt{};
-    int max_comps{0};
     size_t npix{0}, pitch{0}; // prepared frame bytes / device pitch
     size_t in_bytes{0}, in_pitch{0}, in_offset{0}; // what one frame uploads (crop band or the frame) and where it starts
     size_t host_pitch{0};                          // bytes between the caller's frames in a slot's pinned input
@@ -227,26 +369,14 @@ void highlight_queue_release(cvvp_ctx *ctx)
     HighlightQueue *q = ctx->hq;
     if (!q)
         return;
-    cudaStreamSynchronize(ctx->copy);
-    cudaStreamSynchronize(ctx->compute);
-    cudaStreamSynchronize(ctx->copy_out);
+    sync_streams(ctx);
     for (HqSlot &s : q->slots) {
         pool_host_free(s.h_in, s.b_h_in);
-        pool_host_free(s.h_out, s.b_h_out);
-        free_host(s.h_comps);
-        free_host(s.h_ncomps);
         pool_dev_free(s.d_raw, s.b_raw);
         pool_dev_free(s.d_in, s.b_in);
-        pool_dev_free(s.d_out, s.b_out);
-        s.h_in = s.h_out = s.d_raw = s.d_in = s.d_out = nullptr;
-        free_dev(s.d_comps);
-        free_dev(s.d_ncomps);
         if (s.up)
             cudaEventDestroy(s.up);
-        if (s.kdone)
-            cudaEventDestroy(s.kdone);
-        if (s.down)
-            cudaEventDestroy(s.down);
+        hl_results_free(s.res);
     }
     cudaGetLastError();
     delete q;
@@ -255,22 +385,14 @@ void highlight_queue_release(cvvp_ctx *ctx)
 
 int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const cvvp_frame_format *fmt, int max_comps)
 {
+    const int args = depth < 1 || depth > 64 || max_batch < 1 || max_batch > (1ll << 20) || max_comps < 0
+                         ? fail(ctx, CVVP_ERR_INVALID,
+                                "highlight queue: depth must be in [1, 64], max_batch in [1, 2^20], max_comps >= 0")
+                         : CVVP_OK;
     int W = 0, H = 0;
-    if (!highlight_geometry(ctx, &W, &H))
-        return fail(ctx, CVVP_ERR_STATE, "highlight queue: no parameters set (call cvvp_highlight_begin first)");
-    if (ctx->hq)
-        return fail(ctx, CVVP_ERR_STATE, "highlight queue: already begun");
-    if (depth < 1 || depth > 64 || max_batch < 1 || max_batch > (1ll << 20) || max_comps < 0)
-        return fail(ctx, CVVP_ERR_INVALID, "highlight queue: depth must be in [1, 64], max_batch in [1, 2^20], max_comps >= 0");
-    if (fmt) {
-        int rc = frames_check_format(ctx, fmt);
-        if (rc != CVVP_OK)
-            return rc;
-        if (fmt->crop_width != W || fmt->crop_height != H || frames_out_bytes(*fmt) != size_t(W) * size_t(H))
-            return fail(ctx, CVVP_ERR_INVALID,
-                        "highlight queue: prepared frames must be single-channel %dx%d like the background (cv::findContours "
-                        "requires 8UC1)", W, H);
-    }
+    const int rc = highlight_stream_check(ctx, "highlight queue", ctx->hq != nullptr, args, fmt, &W, &H);
+    if (rc != CVVP_OK)
+        return rc;
     HighlightQueue *q = new (std::nothrow) HighlightQueue();
     if (!q)
         return fail(ctx, CVVP_ERR_NOMEM, "out of host memory");
@@ -280,7 +402,6 @@ int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const c
     q->has_fmt = fmt != nullptr;
     if (fmt)
         q->fmt = *fmt;
-    q->max_comps = max_comps;
     q->npix = size_t(W) * size_t(H);
     q->pitch = round_up(q->npix, 128);
     if (fmt) {
@@ -300,14 +421,6 @@ int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const c
     bool ok = true;
     for (HqSlot &s : q->slots) {
         // the big buffers come from the process-wide pool: a job on the next video of the same geometry reuses them
-        auto host = [&](uint8_t *&p, size_t &b, size_t bytes) {
-            void *v = nullptr;
-            if (pool_host_alloc(&v, bytes) != cudaSuccess)
-                return false;
-            p = static_cast<uint8_t *>(v);
-            b = bytes;
-            return true;
-        };
         auto dev = [&](uint8_t *&p, size_t &b, size_t bytes) {
             void *v = nullptr;
             if (pool_dev_alloc(&v, bytes) != cudaSuccess)
@@ -316,21 +429,17 @@ int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const c
             b = bytes;
             return true;
         };
-        ok = ok && host(s.h_in, s.b_h_in, nb * q->host_pitch);
-        ok = ok && host(s.h_out, s.b_h_out, nb * q->pitch);
+        void *h = nullptr;
+        ok = ok && pool_host_alloc(&h, nb * q->host_pitch) == cudaSuccess;
+        if (ok) {
+            s.h_in = static_cast<uint8_t *>(h);
+            s.b_h_in = nb * q->host_pitch;
+        }
         if (fmt)
             ok = ok && dev(s.d_raw, s.b_raw, nb * q->in_pitch);
         ok = ok && dev(s.d_in, s.b_in, nb * q->pitch);
-        ok = ok && dev(s.d_out, s.b_out, nb * q->pitch);
-        if (max_comps > 0) {
-            ok = ok && cudaMallocHost(&s.h_comps, nb * size_t(max_comps) * sizeof(cvvp_component)) == cudaSuccess;
-            ok = ok && cudaMallocHost(&s.h_ncomps, nb * sizeof(int)) == cudaSuccess;
-            ok = ok && cudaMalloc(&s.d_comps, nb * size_t(max_comps) * sizeof(cvvp_component)) == cudaSuccess;
-            ok = ok && cudaMalloc(&s.d_ncomps, nb * sizeof(int)) == cudaSuccess;
-        }
         ok = ok && cudaEventCreateWithFlags(&s.up, cudaEventDisableTiming) == cudaSuccess;
-        ok = ok && cudaEventCreateWithFlags(&s.kdone, cudaEventDisableTiming) == cudaSuccess;
-        ok = ok && cudaEventCreateWithFlags(&s.down, cudaEventDisableTiming) == cudaSuccess;
+        ok = ok && hl_results_alloc(s.res, max_batch, q->npix, q->pitch, max_comps, false);
         if (!ok)
             break;
     }
@@ -350,7 +459,7 @@ int highlight_queue_pending(const cvvp_ctx *ctx)
 // queues H2D (crop bands only) -> [frame preparation] -> highlight kernel -> D2H for the n frames in the slot's pinned input
 static int launch_slot(cvvp_ctx *ctx, HighlightQueue *q, HqSlot &s, long long n)
 {
-    s.n = n;
+    s.res.n = n;
     uint8_t *up_to = q->has_fmt ? s.d_raw : s.d_in;
     CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(up_to, q->in_pitch, s.h_in + q->in_offset, q->host_pitch, q->in_bytes, size_t(n),
                                         cudaMemcpyHostToDevice, ctx->copy));
@@ -363,38 +472,11 @@ static int launch_slot(cvvp_ctx *ctx, HighlightQueue *q, HqSlot &s, long long n)
         if (rc != CVVP_OK)
             return rc;
     }
-    if (q->max_comps > 0)
-        rc = highlight_device_cc(ctx, s.d_in, n, q->pitch, s.d_out, q->pitch, s.d_comps, q->max_comps, s.d_ncomps, nullptr, 0,
-                                 ctx->compute);
-    else
-        rc = highlight_device(ctx, s.d_in, n, q->pitch, s.d_out, q->pitch, ctx->compute);
+    rc = highlight_device_bg(ctx, s.d_in, n, q->pitch, nullptr, 0, s.res.d_out, q->pitch, hl_results_cc(s.res, 0),
+                             ctx->compute);
     if (rc != CVVP_OK)
         return rc;
-    CVVP_CUDA_OK(ctx, cudaEventRecord(s.kdone, ctx->compute));
-    CVVP_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->copy_out, s.kdone, 0));
-    CVVP_CUDA_OK(ctx, cudaMemcpyAsync(s.h_out, s.d_out, size_t(n) * q->pitch, cudaMemcpyDeviceToHost, ctx->copy_out));
-    if (q->max_comps > 0) {
-        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(s.h_comps, s.d_comps, size_t(n) * size_t(q->max_comps) * sizeof(cvvp_component),
-                                          cudaMemcpyDeviceToHost, ctx->copy_out));
-        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(s.h_ncomps, s.d_ncomps, size_t(n) * sizeof(int), cudaMemcpyDeviceToHost, ctx->copy_out));
-    }
-    CVVP_CUDA_OK(ctx, cudaEventRecord(s.down, ctx->copy_out));
-    return CVVP_OK;
-}
-
-// A launch that failed half-way leaves copies / kernels of unknown extent queued on the slot while the slot is not
-// counted as pending: the next submit would overwrite pinned memory an earlier H2D may still be reading.  Drain the
-// streams and refuse further submits; cvvp_highlight_queue_end (or cvvp_highlight_end) clears the state.
-static int slot_failed(cvvp_ctx *ctx, HighlightQueue *q, int rc)
-{
-    const std::string why = ctx->err;
-    cudaStreamSynchronize(ctx->copy);
-    cudaStreamSynchronize(ctx->compute);
-    cudaStreamSynchronize(ctx->copy_out);
-    cudaGetLastError();
-    q->failed = true;
-    ctx->err = why;
-    return rc;
+    return hl_results_download(ctx, s.res);
 }
 
 static int check_can_fill(cvvp_ctx *ctx, HighlightQueue *q)
@@ -406,6 +488,18 @@ static int check_can_fill(cvvp_ctx *ctx, HighlightQueue *q)
     if (q->count + q->acquired >= q->depth)
         return fail(ctx, CVVP_ERR_STATE, "highlight queue: %d batches pending or being filled; call cvvp_highlight_next first",
                     q->depth);
+    return CVVP_OK;
+}
+
+// A launch that failed half-way leaves copies / kernels of unknown extent queued on the slot while the slot is not
+// counted as pending: the next submit would overwrite pinned memory an earlier H2D may still be reading.  Further
+// submits are refused; cvvp_highlight_queue_end (or cvvp_highlight_end) clears the state.
+static int queue_slot(cvvp_ctx *ctx, HighlightQueue *q, HqSlot &s, long long n)
+{
+    const int rc = launch_slot(ctx, q, s, n);
+    if (rc != CVVP_OK)
+        return drain_after_failure(ctx, q->failed, rc);
+    q->count++;
     return CVVP_OK;
 }
 
@@ -424,11 +518,7 @@ int highlight_queue_submit(cvvp_ctx *ctx, const uint8_t *frames, long long n, si
     // a slot is handed out again only after cvvp_highlight_next waited for its `down` event: nothing of it is in flight
     for (long long i = 0; i < n; ++i)
         std::memcpy(s.h_in + size_t(i) * q->host_pitch + q->in_offset, frames + size_t(i) * frame_stride + q->in_offset, q->in_bytes);
-    rc = launch_slot(ctx, q, s, n);
-    if (rc != CVVP_OK)
-        return slot_failed(ctx, q, rc);
-    q->count++;
-    return CVVP_OK;
+    return queue_slot(ctx, q, s, n);
 }
 
 int highlight_slot_acquire(cvvp_ctx *ctx, uint8_t **h_frames, size_t *frame_pitch, long long *max_frames)
@@ -461,12 +551,7 @@ int highlight_slot_commit(cvvp_ctx *ctx, long long n)
         q->gap = q->acquired > 0;
         return CVVP_OK;
     }
-    HqSlot &s = q->slots[size_t((q->head + q->count) % q->depth)];
-    const int rc = launch_slot(ctx, q, s, n);
-    if (rc != CVVP_OK)
-        return slot_failed(ctx, q, rc);
-    q->count++;
-    return CVVP_OK;
+    return queue_slot(ctx, q, q->slots[size_t((q->head + q->count) % q->depth)], n);
 }
 
 int highlight_queue_ready(cvvp_ctx *ctx)
@@ -476,12 +561,7 @@ int highlight_queue_ready(cvvp_ctx *ctx)
         return 0;
     if (q->lent)
         return 1;
-    const cudaError_t e = cudaEventQuery(q->slots[size_t(q->head)].down);
-    if (e == cudaSuccess)
-        return 1;
-    if (e != cudaErrorNotReady)
-        return fail(ctx, CVVP_ERR_CUDA, "highlight queue: %s", cudaGetErrorString(e));
-    return 0;
+    return hl_results_ready(ctx, q->slots[size_t(q->head)].res, "highlight queue");
 }
 
 int highlight_queue_next(cvvp_ctx *ctx, uint8_t *masks_out, size_t out_stride, long long *n_out, cvvp_component *comps_out,
@@ -496,19 +576,14 @@ int highlight_queue_next(cvvp_ctx *ctx, uint8_t *masks_out, size_t out_stride, l
         return fail(ctx, CVVP_ERR_STATE, "highlight queue: nothing pending");
     if (q->lent)
         return fail(ctx, CVVP_ERR_STATE, "highlight queue: the oldest batch is lent out; release the view first");
-    HqSlot &s = q->slots[size_t(q->head)];
-    const cudaError_t e = cudaEventSynchronize(s.down);
+    const HlResults &r = q->slots[size_t(q->head)].res;
+    const int rc = hl_results_wait(ctx, r, "highlight queue");
     q->head = (q->head + 1) % q->depth;
     q->count--;
-    if (e != cudaSuccess)
-        return fail(ctx, CVVP_ERR_CUDA, "highlight queue: batch failed: %s", cudaGetErrorString(e));
-    for (long long i = 0; i < s.n; ++i)
-        std::memcpy(masks_out + size_t(i) * out_stride, s.h_out + size_t(i) * q->pitch, q->npix);
-    if (q->max_comps > 0 && comps_out)
-        std::memcpy(comps_out, s.h_comps, size_t(s.n) * size_t(q->max_comps) * sizeof(cvvp_component));
-    if (q->max_comps > 0 && ncomps_out)
-        std::memcpy(ncomps_out, s.h_ncomps, size_t(s.n) * sizeof(int));
-    *n_out = s.n;
+    if (rc != CVVP_OK)
+        return rc;
+    hl_results_copy(r, masks_out, out_stride, comps_out, ncomps_out, nullptr, 0);
+    *n_out = r.n;
     return CVVP_OK;
 }
 
@@ -524,21 +599,21 @@ int highlight_queue_next_view(cvvp_ctx *ctx, const uint8_t **h_masks, size_t *ma
         return fail(ctx, CVVP_ERR_STATE, "highlight queue: nothing pending");
     if (q->lent)
         return fail(ctx, CVVP_ERR_STATE, "highlight queue: the oldest batch is already lent out");
-    HqSlot &s = q->slots[size_t(q->head)];
-    const cudaError_t e = cudaEventSynchronize(s.down);
-    if (e != cudaSuccess) {
+    const HlResults &r = q->slots[size_t(q->head)].res;
+    const int rc = hl_results_wait(ctx, r, "highlight queue");
+    if (rc != CVVP_OK) {
         q->head = (q->head + 1) % q->depth;
         q->count--;
-        return fail(ctx, CVVP_ERR_CUDA, "highlight queue: batch failed: %s", cudaGetErrorString(e));
+        return rc;
     }
     q->lent = true;
-    *h_masks = s.h_out;
+    *h_masks = r.h_out;
     *mask_pitch = q->pitch;
-    *n_out = s.n;
+    *n_out = r.n;
     if (comps)
-        *comps = q->max_comps > 0 ? s.h_comps : nullptr;
+        *comps = r.h_comps; // null without components
     if (ncomps)
-        *ncomps = q->max_comps > 0 ? s.h_ncomps : nullptr;
+        *ncomps = r.h_ncomps;
     return CVVP_OK;
 }
 

@@ -796,7 +796,8 @@ int highlight_frames_in_flight(cvvp_ctx *ctx, int *out_frames)
 
 // n >= 1 validated frames; frame f against the background at d_bg + f * bg_stride (0: one background for all)
 static int highlight_run(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_frames, long long n, size_t frame_stride,
-                         const uint8_t *d_bg, size_t bg_stride, uint8_t *d_out, size_t out_stride, cudaStream_t stream)
+                         const uint8_t *d_bg, size_t bg_stride, uint8_t *d_out, size_t out_stride, const CcOut &cc,
+                         cudaStream_t stream)
 {
     if (!use_fused(st))
         return highlight_pixels(ctx, st, d_frames, n, frame_stride, d_bg, bg_stride, d_out, out_stride, stream);
@@ -810,78 +811,51 @@ static int highlight_run(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_fra
         if (st->th == -1 && (rc = highlight_thresholds(ctx, st, in, frame_stride, bg, bg_stride, nb, stream)) != CVVP_OK)
             return rc;
         if ((rc = highlight_fused_batch(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out + size_t(done) * out_stride,
-                                        out_stride, stream)) != CVVP_OK)
+                                        out_stride, cc, stream)) != CVVP_OK)
             return rc;
     }
     return CVVP_OK;
 }
 
-int highlight_device(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, uint8_t *d_out,
-                     size_t out_stride, cudaStream_t stream)
-{
-    HighlightState *st = ctx->hl;
-    if (!st)
-        return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
-    if (!d_frames || !d_out || n < 0 || frame_stride < st->g.npix || out_stride < st->g.npix)
-        return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments");
-    if (n == 0)
-        return CVVP_OK;
-    return highlight_run(ctx, st, d_frames, n, frame_stride, st->d_bg, 0, d_out, out_stride, stream);
-}
-
-int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, const uint8_t *d_bgs,
-                        size_t bg_stride, uint8_t *d_out, size_t out_stride, cvvp_component *d_comps, int max_comps,
-                        int *d_ncomps, int32_t *d_labels, size_t labels_stride, cudaStream_t stream)
-{
-    HighlightState *st = ctx->hl;
-    if (!st)
-        return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
-    if (!d_frames || !d_bgs || !d_out || n < 0 || frame_stride < st->g.npix || out_stride < st->g.npix ||
-        (bg_stride != 0 && bg_stride < st->g.npix))
-        return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments (bg_stride must be 0 or at least %u)", st->g.npix);
-    if (d_comps || d_ncomps || d_labels) {
-        if (!d_comps || !d_ncomps || max_comps < 1 || (d_labels && labels_stride < st->g.npix))
-            return fail(ctx, CVVP_ERR_INVALID, "highlight components: bad arguments");
-        if (!use_fused(st))
-            return fail(ctx, CVVP_ERR_UNSUPPORTED, "highlight components: only the fused path labels the final masks");
-        if (n > (1ll << 20))
-            return fail(ctx, CVVP_ERR_UNSUPPORTED, "highlight components: at most 2^20 frames per call");
-    }
-    if (n == 0)
-        return CVVP_OK;
-    st->cc.comps = d_comps;
-    st->cc.max_comps = d_comps ? max_comps : 0;
-    st->cc.ncomps = d_comps ? d_ncomps : nullptr;
-    st->cc.labels = d_comps ? d_labels : nullptr;
-    st->cc.labels_stride = labels_stride;
-    const int rc = highlight_run(ctx, st, d_frames, n, frame_stride, d_bgs, bg_stride, d_out, out_stride, stream);
-    st->cc = CcOut();
-    return rc;
-}
-
 static_assert(sizeof(cvvp_component) == 48, "cvvp_component is part of the C ABI (include/cvvp.h, _cabi.COMPONENT_DTYPE)");
 
-int highlight_device_cc(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, uint8_t *d_out,
-                        size_t out_stride, cvvp_component *d_comps, int max_comps, int *d_ncomps, int32_t *d_labels,
-                        size_t labels_stride, cudaStream_t stream)
+int highlight_check_cc(cvvp_ctx *ctx, long long n, const CcOut &cc)
 {
     HighlightState *st = ctx->hl;
     if (!st)
         return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
-    if (!d_comps || !d_ncomps || max_comps < 1 || (d_labels && labels_stride < st->g.npix))
+    if (!cc.comps || !cc.ncomps || cc.max_comps < 1 || (cc.labels && cc.labels_stride < st->g.npix))
         return fail(ctx, CVVP_ERR_INVALID, "highlight components: bad arguments");
     if (!use_fused(st))
         return fail(ctx, CVVP_ERR_UNSUPPORTED, "highlight components: only the fused path labels the final masks");
     if (n > (1ll << 20))
         return fail(ctx, CVVP_ERR_UNSUPPORTED, "highlight components: at most 2^20 frames per call");
-    st->cc.comps = d_comps;
-    st->cc.max_comps = max_comps;
-    st->cc.ncomps = d_ncomps;
-    st->cc.labels = d_labels;
-    st->cc.labels_stride = labels_stride;
-    const int rc = highlight_device(ctx, d_frames, n, frame_stride, d_out, out_stride, stream);
-    st->cc = CcOut();
-    return rc;
+    return CVVP_OK;
+}
+
+int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, const uint8_t *d_bgs,
+                        size_t bg_stride, uint8_t *d_out, size_t out_stride, const CcOut &cc, cudaStream_t stream)
+{
+    HighlightState *st = ctx->hl;
+    if (!st)
+        return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
+    if (!d_frames || !d_out || n < 0 || frame_stride < st->g.npix || out_stride < st->g.npix ||
+        (bg_stride != 0 && bg_stride < st->g.npix))
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments (bg_stride must be 0 or at least %u)", st->g.npix);
+    const bool want_cc = cc.comps || cc.ncomps || cc.labels;
+    if (want_cc) {
+        const int rc = highlight_check_cc(ctx, n, cc);
+        if (rc != CVVP_OK)
+            return rc;
+    }
+    if (n == 0)
+        return CVVP_OK;
+    if (!d_bgs) {
+        d_bgs = st->d_bg;
+        bg_stride = 0;
+    }
+    return highlight_run(ctx, st, d_frames, n, frame_stride, d_bgs, bg_stride, d_out, out_stride, want_cc ? cc : CcOut(),
+                         stream);
 }
 
 template <typename T>
@@ -939,8 +913,8 @@ int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, 
         const long long nb = n - done < chunk ? n - done : chunk;
         CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(st->d_in, pitch, frames + size_t(done) * frame_stride, frame_stride, np, size_t(nb),
                                             cudaMemcpyHostToDevice, s));
-        rc = highlight_device_cc(ctx, st->d_in, nb, pitch, st->d_res, pitch, st->d_comps, max_comps, st->d_ncomps,
-                                 labels_out ? st->d_labels : nullptr, np, s);
+        rc = highlight_device_bg(ctx, st->d_in, nb, pitch, nullptr, 0, st->d_res, pitch,
+                                 CcOut{st->d_comps, max_comps, st->d_ncomps, labels_out ? st->d_labels : nullptr, np}, s);
         if (rc != CVVP_OK)
             return rc;
         CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(masks_out + size_t(done) * out_stride, out_stride, st->d_res, pitch, np, size_t(nb),
@@ -1020,7 +994,7 @@ int highlight_frames_host(cvvp_ctx *ctx, const uint8_t *frames, long long n, siz
         cudaStreamWaitEvent(ctx->compute, up[b], 0);
         if (idx >= 2)
             cudaStreamWaitEvent(ctx->compute, down[b], 0); // this result half's previous masks have left the device
-        rc = highlight_device(ctx, din, nb, pitch, dres, pitch, ctx->compute);
+        rc = highlight_device_bg(ctx, din, nb, pitch, nullptr, 0, dres, pitch, CcOut(), ctx->compute);
         if (rc != CVVP_OK)
             break;
         cudaEventRecord(kdone[b], ctx->compute);

@@ -1961,11 +1961,6 @@ __global__ void __launch_bounds__(NT, kCtasPerSm) highlight_fused_kernel(const F
     }
 }
 
-size_t round_up_sz(size_t v, size_t a)
-{
-    return (v + a - 1) / a * a;
-}
-
 struct FusedGeom {
     int WW, WWp, wwp_shift;
     uint32_t nwords, cap, rstride;
@@ -2078,14 +2073,14 @@ FusedGeom fused_geom(const HlGeom &g)
     }
     fg.WWp = wwp;
     fg.nwords = uint32_t(g.H) * uint32_t(wwp);
-    fg.cap = uint32_t(round_up_sz(size_t(g.npix) + 2, 4));
-    fg.rstride = uint32_t(round_up_sz(size_t(g.H) + 2, 4));
+    fg.cap = uint32_t(round_up(size_t(g.npix) + 2, 4));
+    fg.rstride = uint32_t(round_up(size_t(g.H) + 2, 4));
     return fg;
 }
 
 size_t run_words(const FusedGeom &fg)
 {
-    return size_t(kRunArrays) * fg.cap + round_up_sz(fg.cap / 32 + 4, 4);
+    return size_t(kRunArrays) * fg.cap + round_up(fg.cap / 32 + 4, 4);
 }
 
 size_t slot_bytes(const FusedGeom &fg)
@@ -2096,12 +2091,14 @@ size_t slot_bytes(const FusedGeom &fg)
 
 int HLF(fused_frames_in_flight)(cvvp_ctx *ctx, HighlightState *st);
 int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
-                               size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream);
+                               size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, const CcOut &cc,
+                               cudaStream_t stream);
 
 #ifndef CVVP_HLF_SMALL
 int fused_frames_in_flight_small(cvvp_ctx *ctx, HighlightState *st);
 int highlight_fused_batch_small(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
-                                size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream);
+                                size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, const CcOut &cc,
+                                cudaStream_t stream);
 
 bool fused_supports(const HighlightState *st)
 {
@@ -2141,10 +2138,11 @@ int fused_frames_in_flight(cvvp_ctx *ctx, HighlightState *st)
 }
 
 int highlight_fused_batch(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
-                          size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream)
+                          size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, const CcOut &cc,
+                          cudaStream_t stream)
 {
-    return use_small(st) ? highlight_fused_batch_small(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out, out_stride, stream)
-                         : highlight_fused_batch_large(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out, out_stride, stream);
+    return use_small(st) ? highlight_fused_batch_small(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out, out_stride, cc, stream)
+                         : highlight_fused_batch_large(ctx, st, in, frame_stride, bg, bg_stride, nb, d_out, out_stride, cc, stream);
 }
 #endif
 
@@ -2215,7 +2213,8 @@ static int ensure_fused(cvvp_ctx *ctx, HighlightState *st)
 // One batch of nb frames (device pointers), one kernel launch.  Work in flight on a context's highlight scratch must
 // be on one stream at a time.
 int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
-                               size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream)
+                               size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, const CcOut &cc,
+                               cudaStream_t stream)
 {
     int rc = ensure_fused(ctx, st);
     if (rc != CVVP_OK)
@@ -2265,11 +2264,11 @@ int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t 
                 out_stride % 16 == 0 && bg_stride % 16 == 0;
     const char *dbg = getenv("CVVP_HL_DEBUG_STAGE");
     P.debug_stage = dbg ? atoi(dbg) : 0;
-    P.comps = st->cc.comps;
-    P.ncomps = st->cc.ncomps;
-    P.max_comps = st->cc.max_comps;
-    P.labels = st->cc.labels;
-    P.labels_stride = st->cc.labels_stride;
+    P.comps = cc.comps;
+    P.ncomps = cc.ncomps;
+    P.max_comps = cc.max_comps;
+    P.labels = cc.labels;
+    P.labels_stride = cc.labels_stride;
     P.prof = nullptr;
     const bool want_prof = getenv("CVVP_HL_PROF") != nullptr;
     if (want_prof && cudaMalloc(reinterpret_cast<void **>(&P.prof), kPCount * sizeof(unsigned long long)) == cudaSuccess)

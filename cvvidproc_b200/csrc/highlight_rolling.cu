@@ -16,7 +16,6 @@
 #include "context.hpp"
 #include "pool.hpp"
 
-#include <cstring>
 #include <deque>
 #include <memory>
 #include <new>
@@ -26,19 +25,9 @@ namespace cvvp
 {
 namespace
 {
-size_t round_up(size_t v, size_t a)
-{
-    return (v + a - 1) / a * a;
-}
-
 struct RollSlot {
-    long long first{0}, n{0}; // frames [first, first + n)
-    size_t b_h_out{0}, b_d_out{0};
-    uint8_t *h_out{nullptr}, *d_out{nullptr}; // h_out: pinned (pool), d_out: device (pool)
-    cvvp_component *h_comps{nullptr}, *d_comps{nullptr};
-    int *h_ncomps{nullptr}, *d_ncomps{nullptr};
-    int32_t *h_labels{nullptr}, *d_labels{nullptr};
-    cudaEvent_t down{nullptr};
+    long long first{0}; // frames [first, first + res.n)
+    HlResults res;
 };
 } // namespace
 
@@ -61,30 +50,14 @@ struct RollingStream {
     std::deque<RollSlot *> pending;
 };
 
-static void free_slot(RollSlot &s)
-{
-    pool_host_free(s.h_out, s.b_h_out);
-    pool_dev_free(s.d_out, s.b_d_out);
-    if (s.h_comps) cudaFreeHost(s.h_comps);
-    if (s.h_ncomps) cudaFreeHost(s.h_ncomps);
-    if (s.h_labels) cudaFreeHost(s.h_labels);
-    if (s.d_comps) cudaFree(s.d_comps);
-    if (s.d_ncomps) cudaFree(s.d_ncomps);
-    if (s.d_labels) cudaFree(s.d_labels);
-    if (s.down) cudaEventDestroy(s.down);
-    s = RollSlot();
-}
-
 void highlight_rolling_release(cvvp_ctx *ctx)
 {
     RollingStream *r = ctx->hr;
     if (!r)
         return;
-    cudaStreamSynchronize(ctx->copy);
-    cudaStreamSynchronize(ctx->compute);
-    cudaStreamSynchronize(ctx->copy_out);
+    sync_streams(ctx);
     for (auto &s : r->slots)
-        free_slot(*s);
+        hl_results_free(s->res);
     pool_dev_free(r->d_ring, r->b_ring);
     pool_dev_free(r->d_bgs, r->b_bgs);
     cudaGetLastError();
@@ -95,24 +68,15 @@ void highlight_rolling_release(cvvp_ctx *ctx)
 int highlight_rolling_begin(cvvp_ctx *ctx, int window, long long max_batch, const cvvp_frame_format *fmt, int max_comps,
                             int labels)
 {
-    int W = 0, H = 0;
-    if (!highlight_geometry(ctx, &W, &H))
-        return fail(ctx, CVVP_ERR_STATE, "rolling highlight: no parameters set (call cvvp_highlight_begin first)");
-    if (ctx->hr)
-        return fail(ctx, CVVP_ERR_STATE, "rolling highlight: already begun");
+    int args = CVVP_OK;
     if (window < 1 || window > 65535)
-        return fail(ctx, CVVP_ERR_INVALID, "rolling highlight: window %d outside [1, 65535]", window);
-    if (max_batch < 1 || max_batch > (1ll << 20) || max_comps < 0 || (labels && max_comps < 1))
-        return fail(ctx, CVVP_ERR_INVALID, "rolling highlight: max_batch must be in [1, 2^20], max_comps >= 0 (>= 1 with labels)");
-    if (fmt) {
-        int rc = frames_check_format(ctx, fmt);
-        if (rc != CVVP_OK)
-            return rc;
-        if (fmt->crop_width != W || fmt->crop_height != H || frames_out_bytes(*fmt) != size_t(W) * size_t(H))
-            return fail(ctx, CVVP_ERR_INVALID,
-                        "rolling highlight: prepared frames must be single-channel %dx%d like the background (cv::findContours "
-                        "requires 8UC1)", W, H);
-    }
+        args = fail(ctx, CVVP_ERR_INVALID, "rolling highlight: window %d outside [1, 65535]", window);
+    else if (max_batch < 1 || max_batch > (1ll << 20) || max_comps < 0 || (labels && max_comps < 1))
+        args = fail(ctx, CVVP_ERR_INVALID, "rolling highlight: max_batch must be in [1, 2^20], max_comps >= 0 (>= 1 with labels)");
+    int W = 0, H = 0;
+    const int rc = highlight_stream_check(ctx, "rolling highlight", ctx->hr != nullptr, args, fmt, &W, &H);
+    if (rc != CVVP_OK)
+        return rc;
     RollingStream *r = new (std::nothrow) RollingStream();
     if (!r)
         return fail(ctx, CVVP_ERR_NOMEM, "out of host memory");
@@ -158,32 +122,8 @@ static int get_slot(cvvp_ctx *ctx, RollingStream *r, RollSlot **out)
         return CVVP_OK;
     }
     auto s = std::make_unique<RollSlot>();
-    const size_t nb = size_t(r->max_batch);
-    void *p = nullptr;
-    bool ok = pool_host_alloc(&p, nb * r->pitch) == cudaSuccess;
-    if (ok) {
-        s->h_out = static_cast<uint8_t *>(p);
-        s->b_h_out = nb * r->pitch;
-        ok = pool_dev_alloc(&p, nb * r->pitch) == cudaSuccess;
-    }
-    if (ok) {
-        s->d_out = static_cast<uint8_t *>(p);
-        s->b_d_out = nb * r->pitch;
-    }
-    if (ok && r->max_comps > 0) {
-        ok = ok && cudaMallocHost(&s->h_comps, nb * size_t(r->max_comps) * sizeof(cvvp_component)) == cudaSuccess;
-        ok = ok && cudaMallocHost(&s->h_ncomps, nb * sizeof(int)) == cudaSuccess;
-        ok = ok && cudaMalloc(&s->d_comps, nb * size_t(r->max_comps) * sizeof(cvvp_component)) == cudaSuccess;
-        ok = ok && cudaMalloc(&s->d_ncomps, nb * sizeof(int)) == cudaSuccess;
-    }
-    if (ok && r->labels) {
-        ok = ok && cudaMallocHost(&s->h_labels, nb * r->npix * sizeof(int32_t)) == cudaSuccess;
-        ok = ok && cudaMalloc(&s->d_labels, nb * r->npix * sizeof(int32_t)) == cudaSuccess;
-    }
-    ok = ok && cudaEventCreateWithFlags(&s->down, cudaEventDisableTiming) == cudaSuccess;
-    if (!ok) {
-        cudaGetLastError();
-        free_slot(*s);
+    if (!hl_results_alloc(s->res, r->max_batch, r->npix, r->pitch, r->max_comps, r->labels)) {
+        hl_results_free(s->res);
         return fail(ctx, CVVP_ERR_NOMEM, "rolling highlight: allocation of a result slot of %lld frames failed", r->max_batch);
     }
     *out = s.get();
@@ -213,7 +153,7 @@ static int launch_ready(cvvp_ctx *ctx, RollingStream *r)
         if (rc != CVVP_OK)
             return rc;
         s->first = t0;
-        s->n = n;
+        s->res.n = n;
         r->pending.push_back(s);
         rc = median_roll_launch(ctx, r->d_ring, r->ring, r->pitch, r->received, r->npix, r->window, r->percent, t0, t0 + n,
                                 r->d_bgs, r->pitch, ctx->compute);
@@ -223,43 +163,18 @@ static int launch_ready(cvvp_ctx *ctx, RollingStream *r)
         for (long long done = 0; done < n;) {
             const long long slot = (t0 + done) % r->ring;
             const long long k = n - done < r->ring - slot ? n - done : r->ring - slot;
-            rc = highlight_device_bg(ctx, r->d_ring + size_t(slot) * r->pitch, k, r->pitch, r->d_bgs + size_t(done) * r->pitch,
-                                     r->pitch, s->d_out + size_t(done) * r->pitch, r->pitch,
-                                     s->d_comps ? s->d_comps + size_t(done) * size_t(r->max_comps) : nullptr, r->max_comps,
-                                     s->d_ncomps ? s->d_ncomps + done : nullptr,
-                                     s->d_labels ? s->d_labels + size_t(done) * r->npix : nullptr, r->npix, ctx->compute);
+            rc = highlight_device_bg(ctx, r->d_ring + size_t(slot) * r->pitch, k, r->pitch,
+                                     r->d_bgs + size_t(done) * r->pitch, r->pitch, s->res.d_out + size_t(done) * r->pitch,
+                                     r->pitch, hl_results_cc(s->res, done), ctx->compute);
             if (rc != CVVP_OK)
                 return rc;
             done += k;
         }
-        CVVP_CUDA_OK(ctx, cudaEventRecord(ctx->ev_copy, ctx->compute));
-        CVVP_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->copy_out, ctx->ev_copy, 0));
-        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(s->h_out, s->d_out, size_t(n) * r->pitch, cudaMemcpyDeviceToHost, ctx->copy_out));
-        if (s->d_comps) {
-            CVVP_CUDA_OK(ctx, cudaMemcpyAsync(s->h_comps, s->d_comps, size_t(n) * size_t(r->max_comps) * sizeof(cvvp_component),
-                                              cudaMemcpyDeviceToHost, ctx->copy_out));
-            CVVP_CUDA_OK(ctx, cudaMemcpyAsync(s->h_ncomps, s->d_ncomps, size_t(n) * sizeof(int), cudaMemcpyDeviceToHost, ctx->copy_out));
-        }
-        if (s->d_labels)
-            CVVP_CUDA_OK(ctx, cudaMemcpyAsync(s->h_labels, s->d_labels, size_t(n) * r->npix * sizeof(int32_t),
-                                              cudaMemcpyDeviceToHost, ctx->copy_out));
-        CVVP_CUDA_OK(ctx, cudaEventRecord(s->down, ctx->copy_out));
+        if ((rc = hl_results_download(ctx, s->res)) != CVVP_OK)
+            return rc;
         r->launched = t0 + n;
     }
     return CVVP_OK;
-}
-
-// work of unknown extent may be queued after a failure half-way: drain, and refuse further pushes
-static int stream_failed(cvvp_ctx *ctx, RollingStream *r, int rc)
-{
-    const std::string why = ctx->err;
-    cudaStreamSynchronize(ctx->copy);
-    cudaStreamSynchronize(ctx->compute);
-    cudaStreamSynchronize(ctx->copy_out);
-    cudaGetLastError();
-    r->failed = true;
-    ctx->err = why;
-    return rc;
 }
 
 static int check_open(cvvp_ctx *ctx, RollingStream *r)
@@ -292,18 +207,19 @@ int highlight_rolling_push(cvvp_ctx *ctx, const uint8_t *frames, long long n, si
         if (r->has_fmt) {
             rc = frames_upload_prepare(ctx, frames + size_t(done) * frame_stride, k, frame_stride, r->fmt, dst, r->pitch);
             if (rc != CVVP_OK)
-                return stream_failed(ctx, r, rc);
+                return drain_after_failure(ctx, r->failed, rc);
         } else {
             const cudaError_t e = cudaMemcpy2DAsync(dst, r->pitch, frames + size_t(done) * frame_stride, frame_stride, r->npix,
                                                     size_t(k), cudaMemcpyHostToDevice, ctx->compute);
             if (e != cudaSuccess)
-                return stream_failed(ctx, r, fail(ctx, CVVP_ERR_CUDA, "rolling highlight: H2D failed: %s", cudaGetErrorString(e)));
+                return drain_after_failure(ctx, r->failed,
+                                           fail(ctx, CVVP_ERR_CUDA, "rolling highlight: H2D failed: %s", cudaGetErrorString(e)));
         }
         done += k;
     }
     r->received += n;
     rc = launch_ready(ctx, r);
-    return rc == CVVP_OK ? rc : stream_failed(ctx, r, rc);
+    return rc == CVVP_OK ? rc : drain_after_failure(ctx, r->failed, rc);
 }
 
 int highlight_rolling_close(cvvp_ctx *ctx)
@@ -314,7 +230,7 @@ int highlight_rolling_close(cvvp_ctx *ctx)
         return rc;
     r->closed = true;
     rc = launch_ready(ctx, r);
-    return rc == CVVP_OK ? rc : stream_failed(ctx, r, rc);
+    return rc == CVVP_OK ? rc : drain_after_failure(ctx, r->failed, rc);
 }
 
 int highlight_rolling_pending(const cvvp_ctx *ctx)
@@ -327,12 +243,7 @@ int highlight_rolling_ready(cvvp_ctx *ctx)
     RollingStream *r = ctx->hr;
     if (!r || r->pending.empty())
         return 0;
-    const cudaError_t e = cudaEventQuery(r->pending.front()->down);
-    if (e == cudaSuccess)
-        return 1;
-    if (e != cudaErrorNotReady)
-        return fail(ctx, CVVP_ERR_CUDA, "rolling highlight: %s", cudaGetErrorString(e));
-    return 0;
+    return hl_results_ready(ctx, r->pending.front()->res, "rolling highlight");
 }
 
 int highlight_rolling_next(cvvp_ctx *ctx, uint8_t *masks_out, size_t out_stride, long long max_n, long long *first_index,
@@ -350,24 +261,17 @@ int highlight_rolling_next(cvvp_ctx *ctx, uint8_t *masks_out, size_t out_stride,
         return CVVP_OK;
     }
     RollSlot *s = r->pending.front();
-    if (max_n < s->n)
-        return fail(ctx, CVVP_ERR_INVALID, "rolling highlight: the next batch holds %lld frames, the buffers %lld", s->n, max_n);
-    const cudaError_t e = cudaEventSynchronize(s->down);
+    if (max_n < s->res.n)
+        return fail(ctx, CVVP_ERR_INVALID, "rolling highlight: the next batch holds %lld frames, the buffers %lld", s->res.n,
+                    max_n);
+    const int rc = hl_results_wait(ctx, s->res, "rolling highlight");
     r->pending.pop_front();
     r->idle.push_back(s);
-    if (e != cudaSuccess)
-        return fail(ctx, CVVP_ERR_CUDA, "rolling highlight: batch failed: %s", cudaGetErrorString(e));
-    for (long long i = 0; i < s->n; ++i)
-        std::memcpy(masks_out + size_t(i) * out_stride, s->h_out + size_t(i) * r->pitch, r->npix);
-    if (r->max_comps > 0 && comps_out)
-        std::memcpy(comps_out, s->h_comps, size_t(s->n) * size_t(r->max_comps) * sizeof(cvvp_component));
-    if (r->max_comps > 0 && ncomps_out)
-        std::memcpy(ncomps_out, s->h_ncomps, size_t(s->n) * sizeof(int));
-    if (r->labels && labels_out)
-        for (long long i = 0; i < s->n; ++i)
-            std::memcpy(labels_out + size_t(i) * labels_stride, s->h_labels + size_t(i) * r->npix, r->npix * sizeof(int32_t));
+    if (rc != CVVP_OK)
+        return rc;
+    hl_results_copy(s->res, masks_out, out_stride, comps_out, ncomps_out, labels_out, labels_stride);
     *first_index = s->first;
-    *n_out = s->n;
+    *n_out = s->res.n;
     return CVVP_OK;
 }
 } // namespace cvvp

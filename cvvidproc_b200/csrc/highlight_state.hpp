@@ -29,15 +29,6 @@ struct FusedScratch {
     size_t bits_bytes{0}, runs_bytes{0}, rowoff_bytes{0}; // sizes of the pooled allocations above (pool.hpp)
 };
 
-// optional component output of the call in progress (cvvp_highlight_device_cc); comps == nullptr: off
-struct CcOut {
-    cvvp_component *comps{nullptr};
-    int max_comps{0};
-    int *ncomps{nullptr};
-    int32_t *labels{nullptr};
-    size_t labels_stride{0};
-};
-
 struct HighlightState {
     HlGeom g{};
     int th{}, lo{}, hi{}, min_hyst{}, min_th{};
@@ -59,7 +50,6 @@ struct HighlightState {
     // fused path
     int fused_variant{-1}; // which build of the fused kernel the job uses: 0 = 1024-thread CTAs, 1 = 256-thread CTAs, -1 = not chosen yet
     FusedScratch fs;
-    CcOut cc;
     // staging of the host-buffer component entry point
     cvvp_component *d_comps{nullptr};
     int *d_ncomps{nullptr};
@@ -78,6 +68,8 @@ int highlight_thresholds(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, s
 bool fused_supports(const HighlightState *st);
 void fused_release(HighlightState *st);
 int fused_frames_in_flight(cvvp_ctx *ctx, HighlightState *st);
+// cc: component output of the final masks (comps == nullptr: off)
 int highlight_fused_batch(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, size_t frame_stride, const uint8_t *bg,
-                          size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, cudaStream_t stream);
+                          size_t bg_stride, unsigned nb, uint8_t *d_out, size_t out_stride, const CcOut &cc,
+                          cudaStream_t stream);
 } // namespace cvvp

@@ -311,6 +311,57 @@ struct GpuHighlightPack { // TokenProcessorPack<HighlightObjectsAlgo> :21-32
     SourceFormat source{}; // enabled (queue mode only): tokens are DECODED frames, prepared on the device
 };
 
+// What the two highlight operators below share: the job's parameters, the check of a token's geometry, and the
+// batch their results are read into.
+inline void begin_highlight(const Context &ctx, const GpuHighlightPack &p)
+{
+    CVVP_ASSERT(!p.background.empty());
+    CVVP_ASSERT(!p.struct_element.empty());
+    CVVP_ASSERT_MSG(p.background.channels == 1, "the highlight stage works on single-channel frames");
+    ctx.check(cvvp_highlight_begin(ctx.get(), p.background.data.data(), p.background.cols, p.background.rows,
+                                   p.struct_element.data.data(), p.struct_element.cols, p.struct_element.rows, p.threshold,
+                                   p.threshold_lo, p.threshold_hi, p.min_size_hyst, p.min_size_threshold, p.width_border));
+}
+
+// tokens are decoded frames of the pack's source format, or prepared frames of the background's geometry
+inline void check_token_geometry(const GpuHighlightPack &p, const FrameBatch &b)
+{
+    if (p.source.enabled)
+        CVVP_ASSERT_MSG(b.rows == p.source.fmt.src_height && b.cols == p.source.fmt.src_width &&
+                            b.channels == p.source.fmt.src_channels,
+                        "decoded frame geometry must match the source format");
+    else
+        CVVP_ASSERT_MSG(b.channels == 1 && b.rows == p.background.rows && b.cols == p.background.cols,
+                        "frame geometry must match the background");
+}
+
+// room for max_batch frames of masks, with components and label images when the pack asks for them; the caller reads
+// n frames into it and calls trim_result_batch
+inline std::unique_ptr<FrameBatch> result_batch(const GpuHighlightPack &p)
+{
+    auto out = std::make_unique<FrameBatch>();
+    out->rows = p.background.rows;
+    out->cols = p.background.cols;
+    out->channels = 1;
+    out->data.resize(std::size_t(p.max_batch) * out->frame_bytes());
+    if (p.components) {
+        out->max_comps = p.max_components;
+        out->comps.resize(std::size_t(p.max_batch) * p.max_components);
+        out->ncomps.resize(std::size_t(p.max_batch));
+        if (p.labels)
+            out->labels.resize(std::size_t(p.max_batch) * out->frame_bytes());
+    }
+    return out;
+}
+
+inline void trim_result_batch(FrameBatch &out, long long n)
+{
+    out.n = int(n);
+    out.data.resize(std::size_t(n) * out.frame_bytes());
+    if (!out.labels.empty())
+        out.labels.resize(std::size_t(n) * out.frame_bytes());
+}
+
 class GpuHighlightAlgo
 {
 public:
@@ -318,14 +369,7 @@ public:
     using result_type = FrameBatch;
     explicit GpuHighlightAlgo(GpuHighlightPack pack) : m_pack{std::move(pack)}, m_ctx{m_pack.device}
     {
-        CVVP_ASSERT(!m_pack.background.empty());
-        CVVP_ASSERT(!m_pack.struct_element.empty());
-        CVVP_ASSERT_MSG(m_pack.background.channels == 1, "the highlight stage works on single-channel frames");
-        m_ctx.check(cvvp_highlight_begin(m_ctx.get(), m_pack.background.data.data(), m_pack.background.cols,
-                                         m_pack.background.rows, m_pack.struct_element.data.data(),
-                                         m_pack.struct_element.cols, m_pack.struct_element.rows, m_pack.threshold,
-                                         m_pack.threshold_lo, m_pack.threshold_hi, m_pack.min_size_hyst,
-                                         m_pack.min_size_threshold, m_pack.width_border));
+        begin_highlight(m_ctx, m_pack);
         if (m_pack.labels) // label images only travel through the synchronous entry point
             m_pack.queue_depth = 0;
         CVVP_ASSERT_MSG(m_pack.queue_depth > 0 || !m_pack.source.enabled, "decoded-frame tokens need the queue");
@@ -341,14 +385,8 @@ public:
     {
         if (!batch || batch->empty())
             return;
+        check_token_geometry(m_pack, *batch);
         if (m_pack.queue_depth > 0) {
-            if (m_pack.source.enabled)
-                CVVP_ASSERT_MSG(batch->rows == m_pack.source.fmt.src_height && batch->cols == m_pack.source.fmt.src_width &&
-                                    batch->channels == m_pack.source.fmt.src_channels,
-                                "decoded frame geometry must match the source format");
-            else
-                CVVP_ASSERT_MSG(batch->channels == 1 && batch->rows == m_pack.background.rows && batch->cols == m_pack.background.cols,
-                                "frame geometry must match the background");
             // back-pressure: a full ring first gives up its oldest batch (the reference's TryInsert fails until a
             // result was taken, token_processing_unit.h:117-135)
             if (cvvp_highlight_queue_pending(m_ctx.get()) == m_pack.queue_depth)
@@ -356,8 +394,6 @@ public:
             m_ctx.check(cvvp_highlight_submit(m_ctx.get(), batch->data.data(), batch->n, batch->frame_bytes()));
             return; // the token's bytes were copied into the slot: it is dropped here like a consumed token
         }
-        CVVP_ASSERT_MSG(batch->channels == 1 && batch->rows == m_pack.background.rows && batch->cols == m_pack.background.cols,
-                        "frame geometry must match the background");
         if (m_pack.components) {
             batch->max_comps = m_pack.max_components;
             batch->comps.assign(std::size_t(batch->n) * m_pack.max_components, cvvp_component{});
@@ -442,22 +478,12 @@ public:
 private:
     std::unique_ptr<FrameBatch> take_next()
     {
-        auto out = std::make_unique<FrameBatch>();
-        out->rows = m_pack.background.rows;
-        out->cols = m_pack.background.cols;
-        out->channels = 1;
-        out->data.resize(std::size_t(m_pack.max_batch) * out->frame_bytes());
-        if (m_pack.components) {
-            out->max_comps = m_pack.max_components;
-            out->comps.resize(std::size_t(m_pack.max_batch) * m_pack.max_components);
-            out->ncomps.resize(std::size_t(m_pack.max_batch));
-        }
+        auto out = result_batch(m_pack); // (queue mode has no label images)
         long long n = 0;
         m_ctx.check(cvvp_highlight_next(m_ctx.get(), out->data.data(), out->frame_bytes(), &n,
                                         m_pack.components ? out->comps.data() : nullptr,
                                         m_pack.components ? out->ncomps.data() : nullptr));
-        out->n = int(n);
-        out->data.resize(std::size_t(n) * out->frame_bytes());
+        trim_result_batch(*out, n);
         return out;
     }
 
@@ -483,15 +509,8 @@ public:
     // pack.max_batch: frames per Insert (at most); pack.source: tokens are DECODED frames, prepared on the device
     GpuRollingHighlightAlgo(GpuHighlightPack pack, int window, int percent = 50) : m_pack{std::move(pack)}, m_ctx{m_pack.device}
     {
-        CVVP_ASSERT(!m_pack.background.empty());
-        CVVP_ASSERT(!m_pack.struct_element.empty());
-        CVVP_ASSERT_MSG(m_pack.background.channels == 1, "the highlight stage works on single-channel frames");
         CVVP_ASSERT(m_pack.max_batch > 0);
-        m_ctx.check(cvvp_highlight_begin(m_ctx.get(), m_pack.background.data.data(), m_pack.background.cols,
-                                         m_pack.background.rows, m_pack.struct_element.data.data(),
-                                         m_pack.struct_element.cols, m_pack.struct_element.rows, m_pack.threshold,
-                                         m_pack.threshold_lo, m_pack.threshold_hi, m_pack.min_size_hyst,
-                                         m_pack.min_size_threshold, m_pack.width_border));
+        begin_highlight(m_ctx, m_pack);
         m_ctx.check(cvvp_median_set_percentile(m_ctx.get(), percent));
         m_ctx.check(cvvp_highlight_rolling_begin(m_ctx.get(), window, m_pack.max_batch,
                                                  m_pack.source.enabled ? &m_pack.source.fmt : nullptr,
@@ -502,13 +521,7 @@ public:
     {
         if (!batch || batch->empty())
             return;
-        if (m_pack.source.enabled)
-            CVVP_ASSERT_MSG(batch->rows == m_pack.source.fmt.src_height && batch->cols == m_pack.source.fmt.src_width &&
-                                batch->channels == m_pack.source.fmt.src_channels,
-                            "decoded frame geometry must match the source format");
-        else
-            CVVP_ASSERT_MSG(batch->channels == 1 && batch->rows == m_pack.background.rows && batch->cols == m_pack.background.cols,
-                            "frame geometry must match the background");
+        check_token_geometry(m_pack, *batch);
         for (int done = 0; done < batch->n;) {
             const int k = int(std::min<long long>(batch->n - done, m_pack.max_batch));
             m_ctx.check(cvvp_highlight_rolling_push(m_ctx.get(), batch->data.data() + std::size_t(done) * batch->frame_bytes(), k,
@@ -527,30 +540,15 @@ public:
             m_ctx.check(ready);
         if (ready == 0 && !m_no_more)
             return nullptr;
-        auto out = std::make_unique<FrameBatch>();
-        out->rows = m_pack.background.rows;
-        out->cols = m_pack.background.cols;
-        out->channels = 1;
-        out->data.resize(std::size_t(m_pack.max_batch) * out->frame_bytes());
-        const bool labels = m_pack.components && m_pack.labels;
-        if (m_pack.components) {
-            out->max_comps = m_pack.max_components;
-            out->comps.resize(std::size_t(m_pack.max_batch) * m_pack.max_components);
-            out->ncomps.resize(std::size_t(m_pack.max_batch));
-        }
-        if (labels)
-            out->labels.resize(std::size_t(m_pack.max_batch) * out->frame_bytes());
+        auto out = result_batch(m_pack);
         long long first = 0, n = 0;
         m_ctx.check(cvvp_highlight_rolling_next(m_ctx.get(), out->data.data(), out->frame_bytes(), m_pack.max_batch, &first, &n,
                                                 m_pack.components ? out->comps.data() : nullptr,
                                                 m_pack.components ? out->ncomps.data() : nullptr,
-                                                labels ? out->labels.data() : nullptr, out->frame_bytes()));
+                                                out->labels.empty() ? nullptr : out->labels.data(), out->frame_bytes()));
         CVVP_ASSERT_MSG(first == m_returned, "rolling highlight results out of order");
         m_returned += n;
-        out->n = int(n);
-        out->data.resize(std::size_t(n) * out->frame_bytes());
-        if (labels)
-            out->labels.resize(std::size_t(n) * out->frame_bytes());
+        trim_result_batch(*out, n);
         return out;
     }
     // end of the stream: the last frames' windows clamp to the frames inserted

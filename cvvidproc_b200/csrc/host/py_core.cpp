@@ -923,6 +923,32 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
                 throw std::runtime_error(error);
         }
     }
+    // one step of the synchronous loop on whichever operator this run uses: insert a batch (null: end of the stream),
+    // then hand every mask that has come back to the tracker
+    auto step = [&](auto &op, std::unique_ptr<FrameBatch> batch) {
+        if (batch) {
+            h_unit.start();
+            op.Insert(std::move(batch)); // queued on the device; returns before the masks exist
+            h_unit.stop();
+            h_batch.stop();
+        } else {
+            op.NotifyNoMoreTokens(); // rolling: the last frames' windows clamp to the frames decoded
+        }
+        for (;;) {
+            h_consume.start();
+            std::unique_ptr<FrameBatch> masks = op.TryGetResult();
+            h_consume.stop();
+            if (!masks)
+                break;
+            deliver(*masks);
+        }
+    };
+    auto sync_step = [&](std::unique_ptr<FrameBatch> batch) {
+        if (roller)
+            step(*roller, std::move(batch));
+        else
+            step(*highlighter, std::move(batch));
+    };
     long long consumed = 0;
     bool eof = pipelined; // the pipelined path above has consumed the stream
     while (!eof && consumed < num_frames) {
@@ -974,37 +1000,11 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
         h_gen.stop();
         if (batch->n == 0)
             break;
-        h_unit.start();
-        if (roller)
-            roller->Insert(std::move(batch));
-        else
-            highlighter->Insert(std::move(batch)); // queued on the device; returns before the masks exist
-        h_unit.stop();
-        h_batch.stop();
         // masks that have come back meanwhile go to the tracker while the device works on the newer batches
-        for (;;) {
-            h_consume.start();
-            std::unique_ptr<FrameBatch> masks = roller ? roller->TryGetResult() : highlighter->TryGetResult();
-            h_consume.stop();
-            if (!masks)
-                break;
-            deliver(*masks);
-        }
+        sync_step(std::move(batch));
     }
-    if (highlighter || roller) { // end of stream: drain in order (token_processing_unit.h:334)
-        if (roller)
-            roller->NotifyNoMoreTokens(); // the last frames' windows clamp to the frames decoded
-        else
-            highlighter->NotifyNoMoreTokens();
-        for (;;) {
-            h_consume.start();
-            std::unique_ptr<FrameBatch> masks = roller ? roller->TryGetResult() : highlighter->TryGetResult();
-            h_consume.stop();
-            if (!masks)
-                break;
-            deliver(*masks);
-        }
-    }
+    if (highlighter || roller) // end of stream: drain in order (token_processing_unit.h:334)
+        sync_step(nullptr);
     a_consume.start();
     a_consume.stop();
     if (pack.print_timing_report) { // cv_vid_objecttrack_helpers.cpp:136-143

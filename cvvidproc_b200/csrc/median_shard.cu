@@ -439,11 +439,6 @@ __global__ void __launch_bounds__(256) shard_zero_push_kernel(const __grid_const
     __threadfence_system();
 }
 
-size_t round_up(size_t v, size_t a)
-{
-    return (v + a - 1) / a * a;
-}
-
 bool all_peers_known(const MedianShard *sh)
 {
     for (int r = 0; r < sh->world; ++r)
