@@ -73,6 +73,8 @@ def load():
         "cvvp_highlight_frames": (i32, [vp, vp, i64, sz, vp, sz]),
         "cvvp_highlight_device": (i32, [vp, vp, i64, sz, vp, sz, vp]),
         "cvvp_highlight_end": (i32, [vp]),
+        "cvvp_highlight_set_polarity": (i32, [vp, i32]),
+        "cvvp_highlight_polarity": (i32, [vp]),
         "cvvp_highlight_device_cc": (i32, [vp, vp, i64, sz, vp, sz, vp, i32, vp, vp, sz, vp]),
         "cvvp_highlight_frames_cc": (i32, [vp, vp, i64, sz, vp, sz, vp, i32, vp, vp, sz]),
         "cvvp_highlight_device_bg": (i32, [vp, vp, i64, sz, vp, sz, vp, sz, vp, i32, vp, vp, sz, vp]),
@@ -401,6 +403,16 @@ class Context:
                                                    threshold_lo, threshold_hi, min_size_hyst, min_size_threshold,
                                                    width_border))
         self._hl_shape = (h, w)
+
+    POLARITY_DARK, POLARITY_BRIGHT, POLARITY_BOTH = 0, 1, 2  # CVVP_POLARITY_*
+
+    def highlight_set_polarity(self, polarity: int):
+        """objects darker than the background (0, the default: d = max(bg - frame, 0)), brighter (1: max(frame - bg, 0))
+        or both (2: |frame - bg|); a highlight job takes it when it begins, and none may be open"""
+        self._check(self._lib.cvvp_highlight_set_polarity(self._h, polarity))
+
+    def highlight_polarity(self) -> int:
+        return int(self._lib.cvvp_highlight_polarity(self._h))
 
     def highlight_frames(self, frames: np.ndarray) -> np.ndarray:
         """frames: uint8 (n, H, W) -> masks uint8 (n, H, W) of 0/255"""

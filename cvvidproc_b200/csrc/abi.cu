@@ -799,6 +799,26 @@ int cvvp_highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, in
                            min_size_hyst, min_size_threshold);
 }
 
+int cvvp_highlight_set_polarity(cvvp_ctx *ctx, int polarity)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    if (polarity != CVVP_POLARITY_DARK && polarity != CVVP_POLARITY_BRIGHT && polarity != CVVP_POLARITY_BOTH)
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: unknown polarity %d", polarity);
+    // an open job, its queue and its rolling stream took the polarity in cvvp_highlight_begin
+    if (ctx->hl)
+        return fail(ctx, CVVP_ERR_STATE, "highlight: a highlight job is open on this context");
+    ctx->polarity = polarity;
+    return CVVP_OK;
+}
+
+int cvvp_highlight_polarity(const cvvp_ctx *ctx)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    return ctx->polarity;
+}
+
 int cvvp_highlight_frames(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, uint8_t *masks_out,
                           size_t out_stride)
 {

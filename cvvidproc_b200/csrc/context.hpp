@@ -110,6 +110,7 @@ struct cvvp_ctx {
     cvvp::HighlightQueue *hq{nullptr};
     cvvp::RollingStream *hr{nullptr};
     int percent{50}; // percentile of every background (cvvp_median_set_percentile); jobs take it when they begin
+    int polarity{CVVP_POLARITY_DARK}; // object polarity (cvvp_highlight_set_polarity); highlight jobs take it when they begin
 };
 
 namespace cvvp

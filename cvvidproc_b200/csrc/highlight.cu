@@ -6,7 +6,8 @@
 // connected-component labels and purely local rules (SURVEY.md section 9; executable spec: oracle/highlight_model.py,
 // which is held bit-exact to a cv2 restatement of the reference):
 //
-//   d  = max(bg - frame, 0)                                   (:27-29, saturating, NOT absdiff)
+//   d  = max(bg - frame, 0)                                   (:27-29, saturating, NOT absdiff; other object
+//                                                               polarities: hl_diff, cvvp_highlight_set_polarity)
 //   A  = fill(rso(open(d > th), min_size_threshold))          (:35-47)
 //   B  = fill(rso(open(hyst(d, lo, hi)), min_size_hyst))      (:54-73)
 //   out = 255 * (A | B)                                       (:77)
@@ -74,14 +75,15 @@ __device__ __forceinline__ void uf_union(uint32_t *lab, uint32_t a, uint32_t b)
 // ------------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
     diff_thresh_kernel(const uint8_t *__restrict__ frames, size_t frame_stride, const uint8_t *__restrict__ bg,
-                       size_t bg_stride, HlGeom g, const int *__restrict__ th_a, int lo, int hi, uint8_t *__restrict__ diff,
-                       uint8_t *__restrict__ mask_a, uint8_t *__restrict__ mask_u, uint8_t *__restrict__ mask_l)
+                       size_t bg_stride, HlGeom g, int polarity, const int *__restrict__ th_a, int lo, int hi,
+                       uint8_t *__restrict__ diff, uint8_t *__restrict__ mask_a, uint8_t *__restrict__ mask_u,
+                       uint8_t *__restrict__ mask_l)
 {
     const uint32_t f = blockIdx.z;
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= g.npix)
         return;
-    const int d = max(int(bg[size_t(f) * bg_stride + p]) - int(frames[size_t(f) * frame_stride + p]), 0);
+    const int d = hl_diff(bg[size_t(f) * bg_stride + p], frames[size_t(f) * frame_stride + p], polarity);
     const size_t o = size_t(f) * g.mstride + p;
     if (diff)
         diff[o] = uint8_t(d);
@@ -93,14 +95,14 @@ __global__ void __launch_bounds__(256)
 // 256-bin histogram of the difference image (only for threshold == -1, Otsu)
 __global__ void __launch_bounds__(256)
     diff_hist_kernel(const uint8_t *__restrict__ frames, size_t frame_stride, const uint8_t *__restrict__ bg,
-                     size_t bg_stride, HlGeom g, unsigned int *__restrict__ hist)
+                     size_t bg_stride, HlGeom g, int polarity, unsigned int *__restrict__ hist)
 {
     __shared__ unsigned int sh[256];
     const uint32_t f = blockIdx.z;
     sh[threadIdx.x] = 0;
     __syncthreads();
     for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < g.npix; p += gridDim.x * blockDim.x) {
-        const int d = max(int(bg[size_t(f) * bg_stride + p]) - int(frames[size_t(f) * frame_stride + p]), 0);
+        const int d = hl_diff(bg[size_t(f) * bg_stride + p], frames[size_t(f) * frame_stride + p], polarity);
         atomicAdd(&sh[d], 1u);
     }
     __syncthreads();
@@ -637,6 +639,7 @@ int highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, int hei
     st->hi = threshold_hi;
     st->min_hyst = min_size_hyst;
     st->min_th = min_size_threshold;
+    st->polarity = ctx->polarity; // the job keeps the polarity it began with
     // structuring element -> offsets relative to the anchor (kw/2, kh/2); any non-zero entry is set.  A kernel with
     // no non-zero entry is filtered by OpenCV as if only its element (0,0) were set.
     std::vector<short2> offs;
@@ -707,7 +710,8 @@ int highlight_thresholds(cvvp_ctx *ctx, HighlightState *st, const uint8_t *in, s
     }
     if (st->th == -1) {
         cudaMemsetAsync(st->d_hist, 0, size_t(nb) * 256 * sizeof(unsigned int), stream);
-        diff_hist_kernel<<<dim3(64, 1, nb), 256, 0, stream>>>(in, frame_stride, bg, bg_stride, st->g, st->d_hist);
+        diff_hist_kernel<<<dim3(64, 1, nb), 256, 0, stream>>>(in, frame_stride, bg, bg_stride, st->g, st->polarity,
+                                                              st->d_hist);
         otsu_kernel<<<(nb + 63) / 64, 64, 0, stream>>>(st->d_hist, st->g.npix, st->d_th, int(nb));
         ctx->launches += 2;
     } else {
@@ -743,8 +747,9 @@ static int highlight_pixels(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_
         Launcher L{ctx, stream, st->g, nb};
         if ((rc = highlight_thresholds(ctx, st, in, frame_stride, bg, bg_stride, nb, stream)) != CVVP_OK)
             return rc;
-        diff_thresh_kernel<<<L.per_pixel(), 256, 0, stream>>>(in, frame_stride, bg, bg_stride, st->g, st->d_th, st->lo,
-                                                              st->hi, nullptr, st->m_a, st->m_u, st->m_l);
+        diff_thresh_kernel<<<L.per_pixel(), 256, 0, stream>>>(in, frame_stride, bg, bg_stride, st->g, st->polarity,
+                                                              st->d_th, st->lo, st->hi, nullptr, st->m_a, st->m_u,
+                                                              st->m_l);
         ctx->launches += 1;
         // ---- branch A: threshold -> open -> remove small -> fill holes
         run_open(L, *st, st->m_a, st->m_t);

@@ -7,7 +7,8 @@
 // mask in HBM (the algorithmic traffic) plus L2-resident scratch:
 //
 //   bits     frame, background -> three bit images  A = d > th, U = d > hi, L = d > lo   (d = saturating bg - frame)
-//            32 pixels per thread from 128-bit loads; the byte compares are SWAR (four pixels per instruction)
+//            32 pixels per thread from 128-bit loads; the byte compares are SWAR (four pixels per instruction); the
+//            object polarity (cvvp_highlight_set_polarity) picks d = bg - frame, frame - bg or |frame - bg| per frame
 //   open     erode + dilate on bit rows: one funnel shift + AND/OR per structuring-element tap per 32 pixels
 //   label    the nodes of the union-find are the horizontal RUNS of equal bits (a few thousand per 1080p frame, not two
 //            million pixels), numbered in raster order by a two-pass block scan, so "smallest id of a component" is
@@ -105,6 +106,7 @@ struct FusedArgs {
     unsigned *queue; // [0] next frame, [1] CTAs finished
     unsigned nframes;
     int fast_io; // W % 32 == 0 and 16-byte aligned pointers / strides
+    int polarity; // CVVP_POLARITY_*: which difference image d the bits phase computes
     uint32_t smem_words; // dynamic shared memory of the CTA, in 32-bit words
     // opening in shared-memory row bands (0 rows = structuring element too large: global-memory taps instead)
     int band_rows, dy_min, dy_max, pad_words;
@@ -266,8 +268,8 @@ __device__ __forceinline__ void set_range(uint32_t *row, int x0, int x1)
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// bits: d = max(bg - frame, 0); three thresholds -> three bit images          (highlight_objects_algo.cpp:27-29, :100,
-//                                                                               :117-122)
+// bits: d = max(bg - frame, 0) (or another polarity); three thresholds -> three bit images
+//                                                             (highlight_objects_algo.cpp:27-30, :100, :117-122)
 // ------------------------------------------------------------------------------------------------------------------
 // per-byte saturating x - y (SWAR: no carries between bytes)
 __device__ __forceinline__ uint32_t sub_sat_u8x4(uint32_t x, uint32_t y)
@@ -298,9 +300,21 @@ __device__ __forceinline__ ThreshSpec make_thresh(int t)
     return s;
 }
 
+// d of four pixels in polarity POL (hl_diff): bg - frame, frame - bg (saturating), or |frame - bg| (VABSDIFF4.U8)
+template <int POL>
+__device__ __forceinline__ uint32_t diff_u8x4(uint32_t fr, uint32_t bg)
+{
+    if (POL == CVVP_POLARITY_DARK)
+        return sub_sat_u8x4(bg, fr);
+    if (POL == CVVP_POLARITY_BRIGHT)
+        return sub_sat_u8x4(fr, bg);
+    return __vabsdiffu4(fr, bg);
+}
+
 // tm: the smallest of the three thresholds (ThreshSpec of it), or force_or != 0 when one of them is negative.  Most
 // 32-pixel groups of a frame have no pixel above even the smallest threshold: one compare per four pixels settles all
 // three bit words.
+template <int POL>
 __device__ __forceinline__ void bits_of_32(const uint4 &f0, const uint4 &f1, const uint4 &b0, const uint4 &b1,
                                            const ThreshSpec &ta, const ThreshSpec &tu, const ThreshSpec &tl,
                                            const ThreshSpec &tm, uint32_t &wa, uint32_t &wu, uint32_t &wl)
@@ -312,7 +326,7 @@ __device__ __forceinline__ void bits_of_32(const uint4 &f0, const uint4 &f1, con
     uint32_t any = tm.force_or;
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
-        d[k] = sub_sat_u8x4(bk[k], fr[k]);
+        d[k] = diff_u8x4<POL>(fr[k], bk[k]);
         const uint32_t t = thm - (d[k] & ~kH);
         any |= ~((tm.t4 & ~d[k]) | (~(tm.t4 ^ d[k]) & t)) & kH; // byte MSB: d > smallest threshold
     }
@@ -342,7 +356,9 @@ __device__ __forceinline__ ThreshSpec min_thresh(int a, int b, int c)
     return make_thresh(min(a, min(b, c)));
 }
 
-__device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t *U, uint32_t *L)
+// the bits phase in polarity POL; bits_phase picks the instantiation once per frame (P.polarity is uniform)
+template <int POL>
+__device__ __forceinline__ void bits_phase_pol(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t *U, uint32_t *L)
 {
     const int tid = threadIdx.x;
     const uint8_t *fr = P.frames + size_t(f) * P.frame_stride;
@@ -377,14 +393,14 @@ __device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t
             }
             uint32_t wa = 0, wu = 0, wl = 0;
             if (v0)
-                bits_of_32(fa0, fa1, ba0, ba1, ta, tu, tl, tm, wa, wu, wl);
+                bits_of_32<POL>(fa0, fa1, ba0, ba1, ta, tu, tl, tm, wa, wu, wl);
             A[i0] = wa;
             U[i0] = wu;
             L[i0] = wl;
             if (i1 < P.nwords) {
                 wa = wu = wl = 0;
                 if (v1)
-                    bits_of_32(fb0, fb1, bb0, bb1, ta, tu, tl, tm, wa, wu, wl);
+                    bits_of_32<POL>(fb0, fb1, bb0, bb1, ta, tu, tl, tm, wa, wu, wl);
                 A[i1] = wa;
                 U[i1] = wu;
                 L[i1] = wl;
@@ -399,7 +415,7 @@ __device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t
                 const size_t o = size_t(y) * P.W;
                 const int x1 = min(32 * wx + 32, P.W);
                 for (int x = 32 * wx; x < x1; ++x) {
-                    const int d = max(int(__ldg(bg + o + x)) - int(__ldg(fr + o + x)), 0);
+                    const int d = hl_diff(__ldg(bg + o + x), __ldg(fr + o + x), POL);
                     const uint32_t b = 1u << (x & 31);
                     if (d > th_a)
                         wa |= b;
@@ -414,6 +430,16 @@ __device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t
             L[i] = wl;
         }
     }
+}
+
+__device__ void bits_phase(const FusedArgs &P, unsigned f, uint32_t *A, uint32_t *U, uint32_t *L)
+{
+    if (P.polarity == CVVP_POLARITY_DARK)
+        bits_phase_pol<CVVP_POLARITY_DARK>(P, f, A, U, L);
+    else if (P.polarity == CVVP_POLARITY_BRIGHT)
+        bits_phase_pol<CVVP_POLARITY_BRIGHT>(P, f, A, U, L);
+    else
+        bits_phase_pol<CVVP_POLARITY_BOTH>(P, f, A, U, L);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -2260,6 +2286,7 @@ int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t 
     // the common structuring elements have compile-time instantiations of the opening (CVVP_HL_NO_CT=1: run-time plan)
     P.ct_elem = (P.plan.sep && P.band_rows > 0 && !getenv("CVVP_HL_NO_CT")) ? match_ct_elem(st->h_offs) : 0;
     auto aligned16 = [](const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
+    P.polarity = st->polarity;
     P.fast_io = (P.W % 32 == 0) && aligned16(in) && aligned16(d_out) && aligned16(bg) && frame_stride % 16 == 0 &&
                 out_stride % 16 == 0 && bg_stride % 16 == 0;
     const char *dbg = getenv("CVVP_HL_DEBUG_STAGE");

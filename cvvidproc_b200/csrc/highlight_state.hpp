@@ -29,9 +29,18 @@ struct FusedScratch {
     size_t bits_bytes{0}, runs_bytes{0}, rowoff_bytes{0}; // sizes of the pooled allocations above (pool.hpp)
 };
 
+// d of one pixel in a polarity (CVVP_POLARITY_*): bg - frame, frame - bg, or |frame - bg|, saturated to 0..255
+// (highlight_objects_algo.cpp:27-30)
+__device__ __forceinline__ int hl_diff(int bg, int fr, int polarity)
+{
+    const int s = bg - fr;
+    return polarity == CVVP_POLARITY_DARK ? max(s, 0) : polarity == CVVP_POLARITY_BRIGHT ? max(-s, 0) : abs(s);
+}
+
 struct HighlightState {
     HlGeom g{};
     int th{}, lo{}, hi{}, min_hyst{}, min_th{};
+    int polarity{CVVP_POLARITY_DARK}; // the context's polarity when the job began (cvvp_highlight_set_polarity)
     int noffs{0};
     int dy_min{0}, dy_max{0}; // row range of the structuring element's taps (offsets are sorted by row, then column)
     int path{kPathFused};

@@ -309,6 +309,7 @@ struct GpuHighlightPack { // TokenProcessorPack<HighlightObjectsAlgo> :21-32
     int queue_depth{0};
     long long max_batch{0};
     SourceFormat source{}; // enabled (queue mode only): tokens are DECODED frames, prepared on the device
+    int polarity{CVVP_POLARITY_DARK}; // which difference image the masks start from (cvvp_highlight_set_polarity)
 };
 
 // What the two highlight operators below share: the job's parameters, the check of a token's geometry, and the
@@ -318,6 +319,7 @@ inline void begin_highlight(const Context &ctx, const GpuHighlightPack &p)
     CVVP_ASSERT(!p.background.empty());
     CVVP_ASSERT(!p.struct_element.empty());
     CVVP_ASSERT_MSG(p.background.channels == 1, "the highlight stage works on single-channel frames");
+    ctx.check(cvvp_highlight_set_polarity(ctx.get(), p.polarity));
     ctx.check(cvvp_highlight_begin(ctx.get(), p.background.data.data(), p.background.cols, p.background.rows,
                                    p.struct_element.data.data(), p.struct_element.cols, p.struct_element.rows, p.threshold,
                                    p.threshold_lo, p.threshold_hi, p.min_size_hyst, p.min_size_threshold, p.width_border));

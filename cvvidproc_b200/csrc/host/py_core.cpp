@@ -640,6 +640,24 @@ int background_percentile(const py::dict &kwargs)
     return int(v);
 }
 
+// kwargs["cvvp_polarity"]: CVVP_POLARITY_DARK when absent, else exactly the str "dark", "bright" or "both"
+// (RuntimeError otherwise)
+int object_polarity(const py::dict &kwargs)
+{
+    if (!kwargs.contains("cvvp_polarity"))
+        return CVVP_POLARITY_DARK;
+    py::object v = kwargs["cvvp_polarity"];
+    int polarity = -1;
+    if (PyUnicode_Check(v.ptr())) {
+        const std::string name = v.cast<std::string>();
+        polarity = name == "dark" ? CVVP_POLARITY_DARK
+                 : name == "bright" ? CVVP_POLARITY_BRIGHT
+                 : name == "both" ? CVVP_POLARITY_BOTH : -1;
+    }
+    CVVP_ASSERT_MSG(polarity >= 0, "kwargs['cvvp_polarity'] must be \"dark\", \"bright\" or \"both\"");
+    return polarity;
+}
+
 py::dict TrackObjects(const VidObjectTrackPack &pack)
 {
     // Opt-in extra of this implementation (the reference has no counterpart): kwargs["cvvp_background_window"] = W
@@ -652,6 +670,9 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     // of its upper median (P = 50).
     const int roll_window = background_window(pack.assign_objects_pack.kwargs);
     const int roll_percent = background_percentile(pack.assign_objects_pack.kwargs);
+    // kwargs["cvvp_polarity"] = "bright" finds objects brighter than the background (d = max(frame - bg, 0)), "both"
+    // objects on either side (d = |frame - bg|); "dark", the default, is the reference's d = max(bg - frame, 0).
+    const int polarity = object_polarity(pack.assign_objects_pack.kwargs);
     const bool rolling = roll_window > 0;
     FrameSource vid{pack.vid_path, pack.grayscale, pack.vid_is_grayscale};
     if (!vid.opened()) {
@@ -690,6 +711,7 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     hp.min_size_hyst = pack.highlight_objects_pack.min_size_hyst;
     hp.min_size_threshold = pack.highlight_objects_pack.min_size_threshold;
     hp.width_border = pack.highlight_objects_pack.width_border;
+    hp.polarity = polarity;
     // Opt-in extra of this implementation (the reference has no counterpart): kwargs["cvvp_components"] = True makes
     // the device label the 8-connected components of every mask and hands the callback one more keyword argument,
     // `components` = {"count", "stats" (count x 5: x, y, w, h, area -- cv2.connectedComponentsWithStats columns),

@@ -256,6 +256,24 @@ CVVP_API int cvvp_highlight_device(cvvp_ctx *ctx, const uint8_t *d_frames, long 
                                    uint8_t *d_out, size_t out_stride, void *stream);
 CVVP_API int cvvp_highlight_end(cvvp_ctx *ctx);
 
+/* Object polarity: which sign of (frame - background) counts as an object.  Every mask starts from the difference
+ * image d of a frame and its background; the reference computes d = saturate_u8(background - frame) (:27-29), which
+ * finds objects DARKER than the background.  The polarity chooses d:
+ *     CVVP_POLARITY_DARK   (0, the default)  d = max(bg - frame, 0)   the reference (:27-29)
+ *     CVVP_POLARITY_BRIGHT (1)               d = max(frame - bg, 0)   objects brighter than the background
+ *     CVVP_POLARITY_BOTH   (2)               d = |frame - bg|         cv::absdiff, commented out at :30
+ * Everything after d (thresholds, Otsu, opening, hysteresis, small-object removal, hole filling, components) is
+ * unchanged.  The polarity is a setting of the context (no counterpart in the reference): a highlight job takes it in
+ * cvvp_highlight_begin, and every call of that job (frames / device forms, the queue, the rolling stream) uses it.
+ * CVVP_ERR_INVALID for a value outside {0, 1, 2} or a NULL context; CVVP_ERR_STATE while a highlight job is open on
+ * the context (between cvvp_highlight_begin and cvvp_highlight_end). */
+#define CVVP_POLARITY_DARK 0   /* max(bg - frame, 0): the reference (default) */
+#define CVVP_POLARITY_BRIGHT 1 /* max(frame - bg, 0) */
+#define CVVP_POLARITY_BOTH 2   /* |frame - bg| (cv::absdiff) */
+CVVP_API int cvvp_highlight_set_polarity(cvvp_ctx *ctx, int polarity);
+/* the context's polarity (CVVP_POLARITY_DARK unless set), or CVVP_ERR_INVALID for a NULL context */
+CVVP_API int cvvp_highlight_polarity(const cvvp_ctx *ctx);
+
 /* ---------------------------------------------------------------------------------------------
  * components of the highlight masks (opt-in) -- the connected-component labelling that feeds the
  * object tracker.  In the reference this happens on the host inside the user's tracker callback,
