@@ -75,6 +75,8 @@ def load():
         "cvvp_highlight_end": (i32, [vp]),
         "cvvp_highlight_set_polarity": (i32, [vp, i32]),
         "cvvp_highlight_polarity": (i32, [vp]),
+        "cvvp_highlight_set_component_stats": (i32, [vp, i32]),
+        "cvvp_highlight_component_stats": (i32, [vp]),
         "cvvp_highlight_device_cc": (i32, [vp, vp, i64, sz, vp, sz, vp, i32, vp, vp, sz, vp]),
         "cvvp_highlight_frames_cc": (i32, [vp, vp, i64, sz, vp, sz, vp, i32, vp, vp, sz]),
         "cvvp_highlight_device_bg": (i32, [vp, vp, i64, sz, vp, sz, vp, sz, vp, i32, vp, vp, sz, vp]),
@@ -403,6 +405,8 @@ class Context:
                                                    threshold_lo, threshold_hi, min_size_hyst, min_size_threshold,
                                                    width_border))
         self._hl_shape = (h, w)
+        # the job's component records (cvvp_highlight_set_component_stats)
+        self._hl_dtype = self.COMPONENT_STATS_DTYPE if self.highlight_component_stats() else self.COMPONENT_DTYPE
 
     POLARITY_DARK, POLARITY_BRIGHT, POLARITY_BOTH = 0, 1, 2  # CVVP_POLARITY_*
 
@@ -413,6 +417,21 @@ class Context:
 
     def highlight_polarity(self) -> int:
         return int(self._lib.cvvp_highlight_polarity(self._h))
+
+    def highlight_set_component_stats(self, on: bool):
+        """shape and contrast statistics in every component record (COMPONENT_STATS_DTYPE) of the highlight jobs that
+        begin after this; none may be open"""
+        self._check(self._lib.cvvp_highlight_set_component_stats(self._h, int(on)))
+
+    def highlight_component_stats(self) -> bool:
+        rc = self._lib.cvvp_highlight_component_stats(self._h)
+        if rc < 0:
+            self._check(rc)
+        return rc == 1
+
+    def highlight_component_dtype(self) -> np.dtype:
+        """the records of the open job's component outputs: COMPONENT_DTYPE, or COMPONENT_STATS_DTYPE with statistics"""
+        return self._hl_dtype
 
     def highlight_frames(self, frames: np.ndarray) -> np.ndarray:
         """frames: uint8 (n, H, W) -> masks uint8 (n, H, W) of 0/255"""
@@ -429,10 +448,14 @@ class Context:
     COMPONENT_DTYPE = np.dtype([("x0", "<i4"), ("y0", "<i4"), ("x1", "<i4"), ("y1", "<i4"), ("area", "<i4"),
                                 ("first_x", "<i4"), ("first_y", "<i4"), ("reserved", "<i4"), ("sum_x", "<i8"),
                                 ("sum_y", "<i8")])
+    # numpy view of struct cvvp_component_stats: the plain record, then the shape and contrast statistics
+    COMPONENT_STATS_DTYPE = np.dtype([("c", COMPONENT_DTYPE), ("sum_xx", "<i8"), ("sum_xy", "<i8"), ("sum_yy", "<i8"),
+                                      ("sum_d", "<i8"), ("sum_dx", "<i8"), ("sum_dy", "<i8"), ("min_d", "<i4"),
+                                      ("max_d", "<i4")])
 
     def highlight_frames_cc(self, frames: np.ndarray, max_comps: int = 256, labels: bool = False):
         """frames uint8 (n, H, W) -> (masks, comps, ncomps[, labels]): the masks plus the 8-connected components of
-        every mask (structured array (n, max_comps) of COMPONENT_DTYPE, raster-first order) and, if asked, the int32
+        every mask (structured array (n, max_comps) of the job's component dtype, raster-first order) and, if asked, the int32
         label images (0 = background, k = component k of that frame)."""
         frames = np.ascontiguousarray(frames)
         if frames.dtype != np.uint8 or frames.ndim != 3 or frames.shape[1:] != self._hl_shape:
@@ -440,7 +463,7 @@ class Context:
         n = frames.shape[0]
         npix = frames.shape[1] * frames.shape[2]
         out = np.empty_like(frames)
-        comps = np.zeros((n, max_comps), self.COMPONENT_DTYPE)
+        comps = np.zeros((n, max_comps), self._hl_dtype)
         ncomps = np.zeros(n, np.int32)
         lab = np.empty(frames.shape, np.int32) if labels else None
         self._check(self._lib.cvvp_highlight_frames_cc(self._h, frames.ctypes.data, n, npix, out.ctypes.data, npix,
@@ -477,7 +500,7 @@ class Context:
         max_batch, max_comps = self._hq
         h, w = self._hl_shape
         out = np.empty((max_batch, h, w), np.uint8)
-        comps = np.zeros((max_batch, max_comps), self.COMPONENT_DTYPE) if max_comps else None
+        comps = np.zeros((max_batch, max_comps), self._hl_dtype) if max_comps else None
         ncomps = np.zeros(max_batch, np.int32) if max_comps else None
         n = C.c_longlong(0)
         self._check(self._lib.cvvp_highlight_next(self._h, out.ctypes.data, h * w, C.byref(n),
@@ -509,9 +532,9 @@ class Context:
         masks = np.frombuffer(buf, np.uint8).reshape(k, pt)[:, : h * w].reshape(k, h, w)
         if not max_comps:
             return masks
-        cbuf = (C.c_uint8 * (k * max_comps * self.COMPONENT_DTYPE.itemsize)).from_address(pc.value)
+        cbuf = (C.c_uint8 * (k * max_comps * self._hl_dtype.itemsize)).from_address(pc.value)
         nbuf = (C.c_int32 * k).from_address(pn.value)
-        return masks, np.frombuffer(cbuf, self.COMPONENT_DTYPE).reshape(k, max_comps), np.frombuffer(nbuf, np.int32)
+        return masks, np.frombuffer(cbuf, self._hl_dtype).reshape(k, max_comps), np.frombuffer(nbuf, np.int32)
 
     def highlight_view_release(self):
         self._check(self._lib.cvvp_highlight_view_release(self._h))
@@ -564,7 +587,7 @@ class Context:
         max_batch, max_comps, labels = self._hr
         h, w = self._hl_shape
         out = np.empty((max_batch, h, w), np.uint8)
-        comps = np.zeros((max_batch, max_comps), self.COMPONENT_DTYPE) if max_comps else None
+        comps = np.zeros((max_batch, max_comps), self._hl_dtype) if max_comps else None
         ncomps = np.zeros(max_batch, np.int32) if max_comps else None
         lab = np.zeros((max_batch, h, w), np.int32) if labels else None
         first, n = C.c_longlong(0), C.c_longlong(0)

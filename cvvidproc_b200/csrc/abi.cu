@@ -819,6 +819,26 @@ int cvvp_highlight_polarity(const cvvp_ctx *ctx)
     return ctx->polarity;
 }
 
+int cvvp_highlight_set_component_stats(cvvp_ctx *ctx, int on)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    if (on != 0 && on != 1)
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: component statistics must be 0 or 1, not %d", on);
+    // an open job, its queue and its rolling stream took the setting (and their record size) in cvvp_highlight_begin
+    if (ctx->hl)
+        return fail(ctx, CVVP_ERR_STATE, "highlight: a highlight job is open on this context");
+    ctx->component_stats = on;
+    return CVVP_OK;
+}
+
+int cvvp_highlight_component_stats(const cvvp_ctx *ctx)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    return ctx->component_stats;
+}
+
 int cvvp_highlight_frames(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, uint8_t *masks_out,
                           size_t out_stride)
 {

@@ -111,6 +111,7 @@ struct cvvp_ctx {
     cvvp::RollingStream *hr{nullptr};
     int percent{50}; // percentile of every background (cvvp_median_set_percentile); jobs take it when they begin
     int polarity{CVVP_POLARITY_DARK}; // object polarity (cvvp_highlight_set_polarity); highlight jobs take it when they begin
+    int component_stats{0}; // cvvp_highlight_set_component_stats; highlight jobs take it when they begin
 };
 
 namespace cvvp
@@ -179,12 +180,16 @@ int highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, int hei
                     int threshold, int threshold_lo, int threshold_hi, int min_size_hyst, int min_size_threshold);
 // optional component output of a highlight call: all pointers null = off
 struct CcOut {
-    cvvp_component *comps{nullptr}; // [frame][max_comps]
+    cvvp_component *comps{nullptr}; // [frame][max_comps] records of rec_bytes each
     int max_comps{0};
     int *ncomps{nullptr};
     int32_t *labels{nullptr}; // [frame][labels_stride] or nullptr
     size_t labels_stride{0};
+    size_t rec_bytes{sizeof(cvvp_component)}; // highlight_device_bg sets the job's (highlight_record_bytes)
 };
+// bytes of one component record of the context's highlight job: sizeof(cvvp_component_stats) while the job has
+// component statistics on (cvvp_highlight_set_component_stats), else sizeof(cvvp_component)
+size_t highlight_record_bytes(const cvvp_ctx *ctx);
 // the component arguments are complete and the job's path can label (a highlight job must exist)
 int highlight_check_cc(cvvp_ctx *ctx, long long n, const CcOut &cc);
 // frame f against the background at d_bgs + f * bg_stride (0 = one for all; d_bgs == nullptr: the job's own)
@@ -214,6 +219,7 @@ int frames_upload_prepare(cvvp_ctx *ctx, const uint8_t *frames, long long n, siz
 struct HlResults {
     size_t npix{0}, pitch{0}; // mask bytes / pitch of the masks on both sides
     int max_comps{0};         // 0: no components
+    size_t rec_bytes{0};      // bytes per component record (highlight_record_bytes of the job)
     bool labels{false};
     size_t mask_bytes{0};     // of each pooled mask buffer (pool.hpp)
     uint8_t *h_out{nullptr}, *d_out{nullptr}; // h_*: pinned
@@ -224,7 +230,8 @@ struct HlResults {
     long long n{0}; // frames of the batch
 };
 // false: out of memory (what was allocated stays for hl_results_free)
-bool hl_results_alloc(HlResults &r, long long max_batch, size_t npix, size_t pitch, int max_comps, bool labels);
+bool hl_results_alloc(HlResults &r, long long max_batch, size_t npix, size_t pitch, int max_comps, size_t rec_bytes,
+                      bool labels);
 void hl_results_free(HlResults &r);
 // the n frames' component outputs, starting at frame `first` of the batch
 CcOut hl_results_cc(const HlResults &r, long long first);

@@ -185,12 +185,14 @@ int frames_prepare_host(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_
 /* ------------------------------------------------------------------------------------------------------------------- */
 /* shared by the highlight queue and the rolling stream (highlight_rolling.cu)                                         */
 /* ------------------------------------------------------------------------------------------------------------------- */
-bool hl_results_alloc(HlResults &r, long long max_batch, size_t npix, size_t pitch, int max_comps, bool labels)
+bool hl_results_alloc(HlResults &r, long long max_batch, size_t npix, size_t pitch, int max_comps, size_t rec_bytes,
+                      bool labels)
 {
     const size_t nb = size_t(max_batch);
     r.npix = npix;
     r.pitch = pitch;
     r.max_comps = max_comps;
+    r.rec_bytes = rec_bytes;
     r.labels = labels;
     r.mask_bytes = nb * pitch;
     // the masks come from the process-wide pool: a job on the next video of the same geometry reuses them
@@ -203,9 +205,9 @@ bool hl_results_alloc(HlResults &r, long long max_batch, size_t npix, size_t pit
     if (ok)
         r.d_out = static_cast<uint8_t *>(p);
     if (max_comps > 0) {
-        ok = ok && cudaMallocHost(&r.h_comps, nb * size_t(max_comps) * sizeof(cvvp_component)) == cudaSuccess;
+        ok = ok && cudaMallocHost(&r.h_comps, nb * size_t(max_comps) * rec_bytes) == cudaSuccess;
         ok = ok && cudaMallocHost(&r.h_ncomps, nb * sizeof(int)) == cudaSuccess;
-        ok = ok && cudaMalloc(&r.d_comps, nb * size_t(max_comps) * sizeof(cvvp_component)) == cudaSuccess;
+        ok = ok && cudaMalloc(&r.d_comps, nb * size_t(max_comps) * rec_bytes) == cudaSuccess;
         ok = ok && cudaMalloc(&r.d_ncomps, nb * sizeof(int)) == cudaSuccess;
     }
     if (labels) {
@@ -237,7 +239,8 @@ CcOut hl_results_cc(const HlResults &r, long long first)
 {
     CcOut cc;
     if (r.max_comps > 0) {
-        cc.comps = r.d_comps + size_t(first) * size_t(r.max_comps);
+        cc.comps = reinterpret_cast<cvvp_component *>(reinterpret_cast<uint8_t *>(r.d_comps) +
+                                                      size_t(first) * size_t(r.max_comps) * r.rec_bytes);
         cc.max_comps = r.max_comps;
         cc.ncomps = r.d_ncomps + first;
         cc.labels = r.labels ? r.d_labels + size_t(first) * r.npix : nullptr;
@@ -253,7 +256,7 @@ int hl_results_download(cvvp_ctx *ctx, HlResults &r)
     CVVP_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->copy_out, ctx->ev_copy, 0));
     CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_out, r.d_out, n * r.pitch, cudaMemcpyDeviceToHost, ctx->copy_out));
     if (r.max_comps > 0) {
-        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_comps, r.d_comps, n * size_t(r.max_comps) * sizeof(cvvp_component),
+        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_comps, r.d_comps, n * size_t(r.max_comps) * r.rec_bytes,
                                           cudaMemcpyDeviceToHost, ctx->copy_out));
         CVVP_CUDA_OK(ctx, cudaMemcpyAsync(r.h_ncomps, r.d_ncomps, n * sizeof(int), cudaMemcpyDeviceToHost, ctx->copy_out));
     }
@@ -289,7 +292,7 @@ void hl_results_copy(const HlResults &r, uint8_t *masks, size_t mask_stride, cvv
     for (size_t i = 0; i < n; ++i)
         std::memcpy(masks + i * mask_stride, r.h_out + i * r.pitch, r.npix);
     if (r.max_comps > 0 && comps)
-        std::memcpy(comps, r.h_comps, n * size_t(r.max_comps) * sizeof(cvvp_component));
+        std::memcpy(comps, r.h_comps, n * size_t(r.max_comps) * r.rec_bytes);
     if (r.max_comps > 0 && ncomps)
         std::memcpy(ncomps, r.h_ncomps, n * sizeof(int));
     if (r.labels && labels)
@@ -439,7 +442,7 @@ int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const c
             ok = ok && dev(s.d_raw, s.b_raw, nb * q->in_pitch);
         ok = ok && dev(s.d_in, s.b_in, nb * q->pitch);
         ok = ok && cudaEventCreateWithFlags(&s.up, cudaEventDisableTiming) == cudaSuccess;
-        ok = ok && hl_results_alloc(s.res, max_batch, q->npix, q->pitch, max_comps, false);
+        ok = ok && hl_results_alloc(s.res, max_batch, q->npix, q->pitch, max_comps, highlight_record_bytes(ctx), false);
         if (!ok)
             break;
     }

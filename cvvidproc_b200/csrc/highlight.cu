@@ -28,6 +28,7 @@
 // arrays are u32 / i32 with npix + 1 entries per frame (entry npix = the FRAME node).
 #include "highlight_state.hpp"
 
+#include <cstddef>
 #include <new>
 #include <vector>
 
@@ -606,6 +607,11 @@ void highlight_release(cvvp_ctx *ctx)
     ctx->hl = nullptr;
 }
 
+size_t highlight_record_bytes(const cvvp_ctx *ctx)
+{
+    return ctx->hl && ctx->hl->component_stats ? sizeof(cvvp_component_stats) : sizeof(cvvp_component);
+}
+
 bool highlight_geometry(const cvvp_ctx *ctx, int *width, int *height)
 {
     if (!ctx->hl)
@@ -640,6 +646,7 @@ int highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, int hei
     st->min_hyst = min_size_hyst;
     st->min_th = min_size_threshold;
     st->polarity = ctx->polarity; // the job keeps the polarity it began with
+    st->component_stats = ctx->component_stats; // and its component record size (highlight_record_bytes)
     // structuring element -> offsets relative to the anchor (kw/2, kh/2); any non-zero entry is set.  A kernel with
     // no non-zero entry is filtered by OpenCV as if only its element (0,0) were set.
     std::vector<short2> offs;
@@ -823,6 +830,16 @@ static int highlight_run(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_fra
 }
 
 static_assert(sizeof(cvvp_component) == 48, "cvvp_component is part of the C ABI (include/cvvp.h, _cabi.COMPONENT_DTYPE)");
+static_assert(sizeof(cvvp_component_stats) == 104 && offsetof(cvvp_component_stats, c) == 0,
+              "cvvp_component_stats is part of the C ABI (include/cvvp.h, _cabi.COMPONENT_STATS_DTYPE)");
+
+// [p, p + (n - 1) * stride + bytes) and [q, ...) share a byte
+static bool frames_overlap(const uint8_t *p, size_t p_stride, const uint8_t *q, size_t q_stride, long long n, size_t bytes)
+{
+    const uintptr_t a0 = reinterpret_cast<uintptr_t>(p), b0 = reinterpret_cast<uintptr_t>(q);
+    const uintptr_t a1 = a0 + size_t(n - 1) * p_stride + bytes, b1 = b0 + size_t(n - 1) * q_stride + bytes;
+    return a0 < b1 && b0 < a1;
+}
 
 int highlight_check_cc(cvvp_ctx *ctx, long long n, const CcOut &cc)
 {
@@ -859,8 +876,16 @@ int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, siz
         d_bgs = st->d_bg;
         bg_stride = 0;
     }
-    return highlight_run(ctx, st, d_frames, n, frame_stride, d_bgs, bg_stride, d_out, out_stride, want_cc ? cc : CcOut(),
-                         stream);
+    CcOut job_cc = want_cc ? cc : CcOut();
+    if (want_cc && st->component_stats) {
+        // the statistics read frame and background bytes after the kernel has written the frame's mask
+        if (frames_overlap(d_out, out_stride, d_frames, frame_stride, n, st->g.npix) ||
+            frames_overlap(d_out, out_stride, d_bgs, bg_stride, n, st->g.npix))
+            return fail(ctx, CVVP_ERR_INVALID,
+                        "highlight component statistics: d_out overlaps the frames or the backgrounds");
+        job_cc.rec_bytes = sizeof(cvvp_component_stats);
+    }
+    return highlight_run(ctx, st, d_frames, n, frame_stride, d_bgs, bg_stride, d_out, out_stride, job_cc, stream);
 }
 
 template <typename T>
@@ -909,7 +934,8 @@ int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, 
             return rc;
         st->in_bytes = size_t(chunk) * pitch;
     }
-    if ((rc = grow(ctx, &st->d_comps, &st->comps_cap, size_t(chunk) * size_t(max_comps))) ||
+    const size_t rec = highlight_record_bytes(ctx);
+    if ((rc = grow(ctx, &st->d_comps, &st->comps_cap, size_t(chunk) * size_t(max_comps) * rec)) ||
         (rc = grow(ctx, &st->d_ncomps, &st->ncomps_cap, size_t(chunk))) ||
         (labels_out && (rc = grow(ctx, &st->d_labels, &st->labels_cap, size_t(chunk) * np))))
         return rc;
@@ -919,13 +945,15 @@ int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, 
         CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(st->d_in, pitch, frames + size_t(done) * frame_stride, frame_stride, np, size_t(nb),
                                             cudaMemcpyHostToDevice, s));
         rc = highlight_device_bg(ctx, st->d_in, nb, pitch, nullptr, 0, st->d_res, pitch,
-                                 CcOut{st->d_comps, max_comps, st->d_ncomps, labels_out ? st->d_labels : nullptr, np}, s);
+                                 CcOut{reinterpret_cast<cvvp_component *>(st->d_comps), max_comps, st->d_ncomps,
+                                       labels_out ? st->d_labels : nullptr, np},
+                                 s);
         if (rc != CVVP_OK)
             return rc;
         CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(masks_out + size_t(done) * out_stride, out_stride, st->d_res, pitch, np, size_t(nb),
                                             cudaMemcpyDeviceToHost, s));
-        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(comps_out + size_t(done) * max_comps, st->d_comps,
-                                          size_t(nb) * max_comps * sizeof(cvvp_component), cudaMemcpyDeviceToHost, s));
+        CVVP_CUDA_OK(ctx, cudaMemcpyAsync(reinterpret_cast<uint8_t *>(comps_out) + size_t(done) * max_comps * rec,
+                                          st->d_comps, size_t(nb) * max_comps * rec, cudaMemcpyDeviceToHost, s));
         CVVP_CUDA_OK(ctx, cudaMemcpyAsync(ncomps_out + done, st->d_ncomps, size_t(nb) * sizeof(int), cudaMemcpyDeviceToHost, s));
         if (labels_out)
             CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(labels_out + size_t(done) * labels_stride, labels_stride * sizeof(int32_t),

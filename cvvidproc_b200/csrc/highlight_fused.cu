@@ -113,9 +113,11 @@ struct FusedArgs {
     int ct_elem; // 0 = run-time plan; 1.. = the structuring element has a compile-time instantiation (open_bands_ct)
     MorphPlan plan;
     // optional component output of the final masks (cvvp_highlight_device_cc): nullptr = off
-    cvvp_component *comps; // [frame][max_comps]
+    cvvp_component *comps; // [frame][max_comps] records of rec_bytes each
     int *ncomps;           // [frame]
     int max_comps;
+    int stats;             // 1: the records are cvvp_component_stats (cvvp_highlight_set_component_stats)
+    uint32_t rec_bytes;    // sizeof(cvvp_component) or sizeof(cvvp_component_stats)
     int32_t *labels;       // [frame][labels_stride] or nullptr
     size_t labels_stride;
     unsigned long long *prof; // per-phase nanoseconds summed over frames (CVVP_HL_PROF=1), or nullptr
@@ -1718,6 +1720,94 @@ __device__ void expand_phase(const FusedArgs &P, unsigned f, const uint32_t *A, 
 // 1.. in the raster order of their first pixels (canonical labelling); per component: bounding box, area, first
 // pixel, coordinate sums (centroid = sums / area).  The label image is optional (4 bytes per pixel of output).
 // ------------------------------------------------------------------------------------------------------------------
+// Shape and contrast statistics (cvvp_component_stats) of the foreground runs, added to the records of their components.
+// The moments have closed forms per run.  The contrast sums read the run's frame and background bytes: a warp takes its
+// 32 runs one at a time and spreads each run's pixels over its lanes (four per lane and step on the 128-bit path), so
+// a frame's 1920-pixel runs (the FillHoles all-255 quirk) cost 15 steps, not 1920.  Every lane then adds its own run's
+// totals to the record.
+template <int POL, bool SM>
+__device__ void stats_runs(const FusedArgs &P, unsigned f, const View<SM> &V, uint32_t T, const uint32_t *cidx, uint8_t *recs)
+{
+    const int lane = threadIdx.x & 31;
+    const uint8_t *fr = P.frames + size_t(f) * P.frame_stride;
+    const uint8_t *bg = P.bg + size_t(f) * P.bg_stride;
+    for (uint32_t rb = threadIdx.x & ~31u; rb < T; rb += NT) { // warp-uniform: runs rb .. rb + 31
+        const uint32_t r = rb + lane;
+        int s = 0, e = -1, y = 0;
+        uint32_t kk = kNoLabel;
+        if (r < T) {
+            const uint32_t xi = V.xi(r);
+            if (run_v(xi)) {
+                s = int(run_x(xi)), y = int(run_y(xi));
+                e = int(V.end(r, V.ro(y + 1), P.W));
+                kk = ld(cidx + V.par(r));
+            }
+        }
+        const bool mine = kk < uint32_t(P.max_comps);
+        uint32_t my_sd = 0, my_mn = 0, my_mx = 0;
+        unsigned long long my_sdx = 0;
+        for (uint32_t todo = __ballot_sync(0xFFFFFFFFu, mine); todo; todo &= todo - 1u) {
+            const int src = __ffs(int(todo)) - 1;
+            const int rs = __shfl_sync(0xFFFFFFFFu, s, src), re = __shfl_sync(0xFFFFFFFFu, e, src);
+            const int ry = __shfl_sync(0xFFFFFFFFu, y, src);
+            const uint8_t *frow = fr + size_t(ry) * P.W, *brow = bg + size_t(ry) * P.W;
+            uint32_t sd = 0, mn = 255, mx = 0;
+            unsigned long long sdx = 0;
+            if (P.fast_io) { // rows start 16-byte aligned in both images: aligned words, bytes outside [rs, re] masked
+                uint32_t vmn = 0xFFFFFFFFu, vmx = 0;
+                for (int w = (rs >> 2) + lane; w <= (re >> 2); w += 32) {
+                    const int x0 = 4 * w;
+                    uint32_t keep = 0xFFFFFFFFu;
+                    if (x0 < rs)
+                        keep &= 0xFFFFFFFFu << (8 * (rs - x0));
+                    if (x0 + 3 > re)
+                        keep &= 0xFFFFFFFFu >> (8 * (x0 + 3 - re));
+                    const uint32_t d = diff_u8x4<POL>(__ldg(reinterpret_cast<const uint32_t *>(frow) + w),
+                                                      __ldg(reinterpret_cast<const uint32_t *>(brow) + w)) & keep;
+                    const uint32_t ws = __dp4a(d, 0x01010101u, 0u);
+                    sd += ws;
+                    sdx += (unsigned long long)x0 * ws + __dp4a(d, 0x03020100u, 0u);
+                    vmn = __vminu4(vmn, d | ~keep);
+                    vmx = __vmaxu4(vmx, d);
+                }
+                mn = min(min(vmn & 0xFFu, (vmn >> 8) & 0xFFu), min((vmn >> 16) & 0xFFu, vmn >> 24));
+                mx = max(max(vmx & 0xFFu, (vmx >> 8) & 0xFFu), max((vmx >> 16) & 0xFFu, vmx >> 24));
+            } else {
+                for (int x = rs + lane; x <= re; x += 32) {
+                    const uint32_t d = uint32_t(hl_diff(__ldg(brow + x), __ldg(frow + x), POL));
+                    sd += d;
+                    sdx += (unsigned long long)d * uint32_t(x);
+                    mn = min(mn, d);
+                    mx = max(mx, d);
+                }
+            }
+            sd = __reduce_add_sync(0xFFFFFFFFu, sd); // a run's sum of d is below 255 * 65536
+            mn = __reduce_min_sync(0xFFFFFFFFu, mn);
+            mx = __reduce_max_sync(0xFFFFFFFFu, mx);
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1)
+                sdx += __shfl_xor_sync(0xFFFFFFFFu, sdx, o);
+            if (lane == src)
+                my_sd = sd, my_sdx = sdx, my_mn = mn, my_mx = mx;
+        }
+        if (mine) {
+            cvvp_component_stats *c = reinterpret_cast<cvvp_component_stats *>(recs + size_t(kk) * P.rec_bytes);
+            const long long len = e - s + 1, yy = y;
+            // sum of x * x over [s, e] = F(e) - F(s - 1), F(n) = n (n + 1) (2n + 1) / 6
+            const long long se = e, ss = s - 1;
+            const long long sxx = se * (se + 1) * (2 * se + 1) / 6 - ss * (ss + 1) * (2 * ss + 1) / 6;
+            atomicAdd(reinterpret_cast<unsigned long long *>(&c->sum_xx), (unsigned long long)sxx);
+            atomicAdd(reinterpret_cast<unsigned long long *>(&c->sum_xy), (unsigned long long)(yy * ((s + e) * len / 2)));
+            atomicAdd(reinterpret_cast<unsigned long long *>(&c->sum_yy), (unsigned long long)(yy * yy * len));
+            atomicAdd(reinterpret_cast<unsigned long long *>(&c->sum_d), (unsigned long long)my_sd);
+            atomicAdd(reinterpret_cast<unsigned long long *>(&c->sum_dx), my_sdx);
+            atomicAdd(reinterpret_cast<unsigned long long *>(&c->sum_dy), (unsigned long long)yy * my_sd);
+            atomicMin(&c->min_d, int(my_mn));
+            atomicMax(&c->max_d, int(my_mx));
+        }
+    }
+}
+
 template <bool SM>
 __device__ void components_phase(const FusedArgs &P, Shared &sh, unsigned f, const View<SM> &V, uint32_t T, uint32_t *cidx)
 {
@@ -1748,7 +1838,7 @@ __device__ void components_phase(const FusedArgs &P, Shared &sh, unsigned f, con
         total += c;
     }
     uint32_t k = base + inc - cnt;
-    cvvp_component *comps = P.comps + size_t(f) * P.max_comps;
+    uint8_t *recs = reinterpret_cast<uint8_t *>(P.comps) + size_t(f) * P.max_comps * P.rec_bytes;
     for (uint32_t r = r0; r < r1; ++r) {
         const uint32_t xi = V.xi(r);
         if (run_v(xi) && V.par(r) == r) {
@@ -1760,7 +1850,13 @@ __device__ void components_phase(const FusedArgs &P, Shared &sh, unsigned f, con
                 c.first_x = int(run_x(xi)), c.first_y = int(run_y(xi));
                 c.reserved = 0;
                 c.sum_x = 0, c.sum_y = 0;
-                comps[k] = c;
+                *reinterpret_cast<cvvp_component *>(recs + size_t(k) * P.rec_bytes) = c;
+                if (P.stats) {
+                    cvvp_component_stats *cs = reinterpret_cast<cvvp_component_stats *>(recs + size_t(k) * P.rec_bytes);
+                    cs->sum_xx = cs->sum_xy = cs->sum_yy = 0;
+                    cs->sum_d = cs->sum_dx = cs->sum_dy = 0;
+                    cs->min_d = INT_MAX, cs->max_d = INT_MIN;
+                }
             }
             ++k;
         }
@@ -1788,7 +1884,7 @@ __device__ void components_phase(const FusedArgs &P, Shared &sh, unsigned f, con
         const int e = int(V.end(r, V.ro(y + 1), P.W));
         const uint32_t kk = ld(cidx + V.par(r));
         if (kk < uint32_t(P.max_comps)) {
-            cvvp_component *c = comps + kk;
+            cvvp_component *c = reinterpret_cast<cvvp_component *>(recs + size_t(kk) * P.rec_bytes);
             const int len = e - s + 1;
             atomicAdd(&c->area, len);
             atomicMin(&c->x0, s);
@@ -1803,6 +1899,14 @@ __device__ void components_phase(const FusedArgs &P, Shared &sh, unsigned f, con
             for (int x = s; x <= e; ++x)
                 row[x] = int32_t(kk + 1u);
         }
+    }
+    if (P.stats) { // uniform for the launch
+        if (P.polarity == CVVP_POLARITY_DARK)
+            stats_runs<CVVP_POLARITY_DARK>(P, f, V, T, cidx, recs);
+        else if (P.polarity == CVVP_POLARITY_BRIGHT)
+            stats_runs<CVVP_POLARITY_BRIGHT>(P, f, V, T, cidx, recs);
+        else
+            stats_runs<CVVP_POLARITY_BOTH>(P, f, V, T, cidx, recs);
     }
     __syncthreads();
 }
@@ -2294,6 +2398,8 @@ int HLF(highlight_fused_batch)(cvvp_ctx *ctx, HighlightState *st, const uint8_t 
     P.comps = cc.comps;
     P.ncomps = cc.ncomps;
     P.max_comps = cc.max_comps;
+    P.rec_bytes = uint32_t(cc.rec_bytes);
+    P.stats = cc.rec_bytes == sizeof(cvvp_component_stats);
     P.labels = cc.labels;
     P.labels_stride = cc.labels_stride;
     P.prof = nullptr;

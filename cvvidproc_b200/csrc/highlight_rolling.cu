@@ -122,7 +122,7 @@ static int get_slot(cvvp_ctx *ctx, RollingStream *r, RollSlot **out)
         return CVVP_OK;
     }
     auto s = std::make_unique<RollSlot>();
-    if (!hl_results_alloc(s->res, r->max_batch, r->npix, r->pitch, r->max_comps, r->labels)) {
+    if (!hl_results_alloc(s->res, r->max_batch, r->npix, r->pitch, r->max_comps, highlight_record_bytes(ctx), r->labels)) {
         hl_results_free(s->res);
         return fail(ctx, CVVP_ERR_NOMEM, "rolling highlight: allocation of a result slot of %lld frames failed", r->max_batch);
     }

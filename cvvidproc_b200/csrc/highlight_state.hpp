@@ -41,6 +41,7 @@ struct HighlightState {
     HlGeom g{};
     int th{}, lo{}, hi{}, min_hyst{}, min_th{};
     int polarity{CVVP_POLARITY_DARK}; // the context's polarity when the job began (cvvp_highlight_set_polarity)
+    int component_stats{0}; // the context's cvvp_highlight_set_component_stats when the job began
     int noffs{0};
     int dy_min{0}, dy_max{0}; // row range of the structuring element's taps (offsets are sorted by row, then column)
     int path{kPathFused};
@@ -60,7 +61,7 @@ struct HighlightState {
     int fused_variant{-1}; // which build of the fused kernel the job uses: 0 = 1024-thread CTAs, 1 = 256-thread CTAs, -1 = not chosen yet
     FusedScratch fs;
     // staging of the host-buffer component entry point
-    cvvp_component *d_comps{nullptr};
+    uint8_t *d_comps{nullptr}; // component records of the job's size (highlight_record_bytes)
     int *d_ncomps{nullptr};
     int32_t *d_labels{nullptr};
     size_t comps_cap{0}, ncomps_cap{0}, labels_cap{0};

@@ -48,11 +48,12 @@ struct FrameBatch {
     bool empty() const { return n == 0 || data.empty(); }
     // highlight results with the opt-in components: max_comps records and one count per frame, optional label images
     int max_comps{0};
-    std::vector<cvvp_component> comps;
+    std::size_t rec_bytes{sizeof(cvvp_component)}; // sizeof(cvvp_component_stats) when the job computes statistics
+    std::vector<std::uint8_t> comps;               // [frame][max_comps] records of rec_bytes each
     std::vector<int> ncomps;
     std::vector<std::int32_t> labels;
     int component_count(int i) const { return ncomps.empty() ? 0 : ncomps[std::size_t(i)]; }
-    const cvvp_component *components(int i) const { return comps.data() + std::size_t(i) * max_comps; }
+    cvvp_component *component_records() { return reinterpret_cast<cvvp_component *>(comps.data()); }
     const std::int32_t *label_image(int i) const { return labels.empty() ? nullptr : labels.data() + std::size_t(i) * frame_bytes(); }
 };
 
@@ -302,6 +303,7 @@ struct GpuHighlightPack { // TokenProcessorPack<HighlightObjectsAlgo> :21-32
     // opt-in extras (no counterpart in the reference's pack): 8-connected components of every mask for the tracker
     bool components{false};
     bool labels{false};
+    bool component_stats{false}; // the records are cvvp_component_stats (cvvp_highlight_set_component_stats)
     int max_components{1024};
     // queue_depth > 0: tokens are processed asynchronously, at most queue_depth batches in flight (the reference's
     // token_storage_limit, Sources/AsyncTokens/token_queue.h:209-214) of at most max_batch frames each; results come
@@ -320,6 +322,7 @@ inline void begin_highlight(const Context &ctx, const GpuHighlightPack &p)
     CVVP_ASSERT(!p.struct_element.empty());
     CVVP_ASSERT_MSG(p.background.channels == 1, "the highlight stage works on single-channel frames");
     ctx.check(cvvp_highlight_set_polarity(ctx.get(), p.polarity));
+    ctx.check(cvvp_highlight_set_component_stats(ctx.get(), p.component_stats ? 1 : 0));
     ctx.check(cvvp_highlight_begin(ctx.get(), p.background.data.data(), p.background.cols, p.background.rows,
                                    p.struct_element.data.data(), p.struct_element.cols, p.struct_element.rows, p.threshold,
                                    p.threshold_lo, p.threshold_hi, p.min_size_hyst, p.min_size_threshold, p.width_border));
@@ -339,6 +342,11 @@ inline void check_token_geometry(const GpuHighlightPack &p, const FrameBatch &b)
 
 // room for max_batch frames of masks, with components and label images when the pack asks for them; the caller reads
 // n frames into it and calls trim_result_batch
+inline std::size_t record_bytes(const GpuHighlightPack &p)
+{
+    return p.component_stats ? sizeof(cvvp_component_stats) : sizeof(cvvp_component);
+}
+
 inline std::unique_ptr<FrameBatch> result_batch(const GpuHighlightPack &p)
 {
     auto out = std::make_unique<FrameBatch>();
@@ -348,7 +356,8 @@ inline std::unique_ptr<FrameBatch> result_batch(const GpuHighlightPack &p)
     out->data.resize(std::size_t(p.max_batch) * out->frame_bytes());
     if (p.components) {
         out->max_comps = p.max_components;
-        out->comps.resize(std::size_t(p.max_batch) * p.max_components);
+        out->rec_bytes = record_bytes(p);
+        out->comps.resize(std::size_t(p.max_batch) * p.max_components * out->rec_bytes);
         out->ncomps.resize(std::size_t(p.max_batch));
         if (p.labels)
             out->labels.resize(std::size_t(p.max_batch) * out->frame_bytes());
@@ -398,12 +407,13 @@ public:
         }
         if (m_pack.components) {
             batch->max_comps = m_pack.max_components;
-            batch->comps.assign(std::size_t(batch->n) * m_pack.max_components, cvvp_component{});
+            batch->rec_bytes = record_bytes(m_pack);
+            batch->comps.assign(std::size_t(batch->n) * m_pack.max_components * batch->rec_bytes, 0);
             batch->ncomps.assign(std::size_t(batch->n), 0);
             if (m_pack.labels)
                 batch->labels.resize(std::size_t(batch->n) * batch->frame_bytes());
             m_ctx.check(cvvp_highlight_frames_cc(m_ctx.get(), batch->data.data(), batch->n, batch->frame_bytes(),
-                                                 batch->data.data(), batch->frame_bytes(), batch->comps.data(),
+                                                 batch->data.data(), batch->frame_bytes(), batch->component_records(),
                                                  m_pack.max_components, batch->ncomps.data(),
                                                  m_pack.labels ? batch->labels.data() : nullptr, batch->frame_bytes()));
         } else {
@@ -446,7 +456,7 @@ public:
         const std::uint8_t *masks{nullptr}; // mask i at masks + i * pitch
         std::size_t pitch{0};
         long long n{0};
-        const cvvp_component *comps{nullptr}; // [i * max_comps + k], null without components
+        const cvvp_component *comps{nullptr}; // [i * max_comps + k] records of record_bytes, null without components
         const int *ncomps{nullptr};
     };
     int Pending() const { return cvvp_highlight_queue_pending(m_ctx.get()); }
@@ -483,7 +493,7 @@ private:
         auto out = result_batch(m_pack); // (queue mode has no label images)
         long long n = 0;
         m_ctx.check(cvvp_highlight_next(m_ctx.get(), out->data.data(), out->frame_bytes(), &n,
-                                        m_pack.components ? out->comps.data() : nullptr,
+                                        m_pack.components ? out->component_records() : nullptr,
                                         m_pack.components ? out->ncomps.data() : nullptr));
         trim_result_batch(*out, n);
         return out;
@@ -545,7 +555,7 @@ public:
         auto out = result_batch(m_pack);
         long long first = 0, n = 0;
         m_ctx.check(cvvp_highlight_rolling_next(m_ctx.get(), out->data.data(), out->frame_bytes(), m_pack.max_batch, &first, &n,
-                                                m_pack.components ? out->comps.data() : nullptr,
+                                                m_pack.components ? out->component_records() : nullptr,
                                                 m_pack.components ? out->ncomps.data() : nullptr,
                                                 out->labels.empty() ? nullptr : out->labels.data(), out->frame_bytes()));
         CVVP_ASSERT_MSG(first == m_returned, "rolling highlight results out of order");

@@ -25,6 +25,7 @@
 
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <condition_variable>
 #include <cstdint>
 #include <cstdlib>
@@ -658,6 +659,19 @@ int object_polarity(const py::dict &kwargs)
     return polarity;
 }
 
+// kwargs["cvvp_component_stats"]: false when absent, else exactly a bool; True needs kwargs["cvvp_components"] = True
+bool component_stats(const py::dict &kwargs)
+{
+    if (!kwargs.contains("cvvp_component_stats"))
+        return false;
+    py::object v = kwargs["cvvp_component_stats"];
+    CVVP_ASSERT_MSG(py::isinstance<py::bool_>(v), "kwargs['cvvp_component_stats'] must be True or False");
+    const bool on = v.cast<bool>();
+    CVVP_ASSERT_MSG(!on || (kwargs.contains("cvvp_components") && kwargs["cvvp_components"].cast<bool>()),
+                    "kwargs['cvvp_component_stats'] needs kwargs['cvvp_components'] = True");
+    return on;
+}
+
 py::dict TrackObjects(const VidObjectTrackPack &pack)
 {
     // Opt-in extra of this implementation (the reference has no counterpart): kwargs["cvvp_background_window"] = W
@@ -673,6 +687,8 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     // kwargs["cvvp_polarity"] = "bright" finds objects brighter than the background (d = max(frame - bg, 0)), "both"
     // objects on either side (d = |frame - bg|); "dark", the default, is the reference's d = max(bg - frame, 0).
     const int polarity = object_polarity(pack.assign_objects_pack.kwargs);
+    // kwargs["cvvp_component_stats"] = True (with cvvp_components) adds shape and contrast statistics to `components`
+    const bool want_stats = component_stats(pack.assign_objects_pack.kwargs);
     const bool rolling = roll_window > 0;
     FrameSource vid{pack.vid_path, pack.grayscale, pack.vid_is_grayscale};
     if (!vid.opened()) {
@@ -717,10 +733,14 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     // `components` = {"count", "stats" (count x 5: x, y, w, h, area -- cv2.connectedComponentsWithStats columns),
     // "centroids" (count x 2), "first" (count x 2: raster-first pixel x, y)[, "labels" (int32 H x W) with
     // kwargs["cvvp_labels"] = True]}; components are numbered in the raster order of their first pixels.
+    // kwargs["cvvp_component_stats"] = True adds "moments" (count x 3 int64: m20, m11, m02), "mass" (count int64: sum of
+    // d), "weighted_centroids" (count x 2: sum(d x) / mass, sum(d y) / mass; NaN where the mass is 0) and "contrast"
+    // (count x 2 int32: min d, max d), d being the difference image the thresholds saw (cvvp_component_stats).
     const py::dict &user_kwargs = pack.assign_objects_pack.kwargs;
     const bool want_comps = user_kwargs.contains("cvvp_components") && user_kwargs["cvvp_components"].cast<bool>();
     const bool want_labels = want_comps && user_kwargs.contains("cvvp_labels") && user_kwargs["cvvp_labels"].cast<bool>();
     hp.components = want_comps;
+    hp.component_stats = want_stats;
     hp.labels = want_labels;
     if (want_comps && user_kwargs.contains("cvvp_max_components"))
         hp.max_components = std::max(1, user_kwargs["cvvp_max_components"].cast<int>());
@@ -755,6 +775,7 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     const int mrows = crop.height, mcols = crop.width;
     const std::size_t mbytes = std::size_t(mrows) * mcols;
     std::function<void()> between_frames; // pipelined path: keeps the decoder and the device fed while a batch is delivered
+    const std::size_t rec_bytes = record_bytes(hp);
     auto deliver_raw = [&](const std::uint8_t *masks, std::size_t pitch, long long n, const cvvp_component *comps_all,
                            const int *ncomps_all, int max_comps, const std::int32_t *labels_all) {
         a_batch.start();
@@ -770,7 +791,11 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
             if (want_comps) {
                 const int total = ncomps_all ? ncomps_all[i] : 0;
                 const int cnt = std::min(total, max_comps);
-                const cvvp_component *cs = comps_all + std::size_t(i) * max_comps;
+                const std::uint8_t *recs = reinterpret_cast<const std::uint8_t *>(comps_all) +
+                                           std::size_t(i) * max_comps * rec_bytes;
+                auto rec = [&](int k) -> const cvvp_component & {
+                    return *reinterpret_cast<const cvvp_component *>(recs + std::size_t(k) * rec_bytes);
+                };
                 py::array_t<std::int32_t> stats({cnt, 5});
                 py::array_t<double> cents({cnt, 2});
                 py::array_t<std::int32_t> first({cnt, 2});
@@ -778,21 +803,48 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
                 auto ce = cents.mutable_unchecked<2>();
                 auto fi = first.mutable_unchecked<2>();
                 for (int k = 0; k < cnt; ++k) {
-                    st(k, 0) = cs[k].x0;
-                    st(k, 1) = cs[k].y0;
-                    st(k, 2) = cs[k].x1 - cs[k].x0 + 1;
-                    st(k, 3) = cs[k].y1 - cs[k].y0 + 1;
-                    st(k, 4) = cs[k].area;
-                    ce(k, 0) = double(cs[k].sum_x) / double(cs[k].area);
-                    ce(k, 1) = double(cs[k].sum_y) / double(cs[k].area);
-                    fi(k, 0) = cs[k].first_x;
-                    fi(k, 1) = cs[k].first_y;
+                    const cvvp_component &c = rec(k);
+                    st(k, 0) = c.x0;
+                    st(k, 1) = c.y0;
+                    st(k, 2) = c.x1 - c.x0 + 1;
+                    st(k, 3) = c.y1 - c.y0 + 1;
+                    st(k, 4) = c.area;
+                    ce(k, 0) = double(c.sum_x) / double(c.area);
+                    ce(k, 1) = double(c.sum_y) / double(c.area);
+                    fi(k, 0) = c.first_x;
+                    fi(k, 1) = c.first_y;
                 }
                 py::dict comps;
                 comps["count"] = total;
                 comps["stats"] = stats;
                 comps["centroids"] = cents;
                 comps["first"] = first;
+                if (hp.component_stats) {
+                    py::array_t<std::int64_t> moments({cnt, 3});
+                    py::array_t<std::int64_t> mass(cnt);
+                    py::array_t<double> wcents({cnt, 2});
+                    py::array_t<std::int32_t> contrast({cnt, 2});
+                    auto mo = moments.mutable_unchecked<2>();
+                    auto ma = mass.mutable_unchecked<1>();
+                    auto wc = wcents.mutable_unchecked<2>();
+                    auto co = contrast.mutable_unchecked<2>();
+                    for (int k = 0; k < cnt; ++k) {
+                        const cvvp_component_stats &c = reinterpret_cast<const cvvp_component_stats &>(rec(k));
+                        mo(k, 0) = c.sum_xx;
+                        mo(k, 1) = c.sum_xy;
+                        mo(k, 2) = c.sum_yy;
+                        ma(k) = c.sum_d;
+                        // a component whose pixels all have d = 0 (hole filling, the all-255 quirk) has no weighted centroid
+                        wc(k, 0) = c.sum_d ? double(c.sum_dx) / double(c.sum_d) : std::nan("");
+                        wc(k, 1) = c.sum_d ? double(c.sum_dy) / double(c.sum_d) : std::nan("");
+                        co(k, 0) = c.min_d;
+                        co(k, 1) = c.max_d;
+                    }
+                    comps["moments"] = moments;
+                    comps["mass"] = mass;
+                    comps["weighted_centroids"] = wcents;
+                    comps["contrast"] = contrast;
+                }
                 if (want_labels && labels_all) {
                     py::array_t<std::int32_t> lab({mrows, mcols});
                     std::memcpy(lab.mutable_data(), labels_all + std::size_t(i) * mbytes, mbytes * sizeof(std::int32_t));
@@ -818,7 +870,8 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
         a_batch.stop();
     };
     auto deliver = [&](const FrameBatch &masks) {
-        deliver_raw(masks.data.data(), masks.frame_bytes(), masks.n, masks.comps.empty() ? nullptr : masks.comps.data(),
+        deliver_raw(masks.data.data(), masks.frame_bytes(), masks.n,
+                    masks.comps.empty() ? nullptr : reinterpret_cast<const cvvp_component *>(masks.comps.data()),
                     masks.ncomps.empty() ? nullptr : masks.ncomps.data(), masks.max_comps,
                     masks.labels.empty() ? nullptr : masks.labels.data());
     };

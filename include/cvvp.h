@@ -310,6 +310,31 @@ CVVP_API int cvvp_highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, lo
 CVVP_API int cvvp_highlight_frames_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride,
                                       uint8_t *masks_out, size_t out_stride, cvvp_component *comps_out, int max_comps,
                                       int *ncomps_out, int32_t *labels_out, size_t labels_stride);
+/* Shape and contrast statistics of the components (opt-in; no counterpart in the reference).  Over the pixels (x, y)
+ * of a component, with d the job's difference image (the polarity's d of the frame and its own background, the d
+ * the thresholds saw):
+ *     sum_xx, sum_xy, sum_yy   sum of x*x, x*y, y*y: the raw moments m20, m11, m02 of cv::moments(component mask,
+ *                              binaryImage=true); central moments and the ellipse follow from them and c's sums
+ *     sum_d                    contrast mass: sum of d (0 is possible: hole filling and the FillHoles all-255 quirk
+ *                              put pixels with d = 0 into masks)
+ *     sum_dx, sum_dy           sum of d*x, d*y: contrast-weighted centroid (sum_dx / sum_d, sum_dy / sum_d)
+ *     min_d, max_d             smallest and largest d
+ * All values are exact integers.  The setting belongs to the context, like the polarity: a highlight job takes it in
+ * cvvp_highlight_begin.  While a job has it on, EVERY cvvp_component * output of that job (cvvp_highlight_device_cc,
+ * _device_bg, _frames_cc, cvvp_highlight_next, cvvp_highlight_next_view, cvvp_highlight_rolling_next) points to an
+ * array of cvvp_component_stats, and max_comps counts those records; pass (cvvp_component *)stats (c is the first
+ * member).  The statistics read the frames and backgrounds after the masks are written, so with statistics on the
+ * device forms return CVVP_ERR_INVALID when d_out overlaps the frames or the backgrounds (no in-place output).
+ * set: 0 = off (default) or 1 = on; CVVP_ERR_INVALID for another value or a NULL context, CVVP_ERR_STATE while a
+ * highlight job is open on the context.  get: the context's setting, or CVVP_ERR_INVALID for a NULL context. */
+typedef struct cvvp_component_stats {
+    cvvp_component c;               /* exactly what the plain form returns */
+    int64_t sum_xx, sum_xy, sum_yy; /* second-order raw moments (cv::moments m20, m11, m02) */
+    int64_t sum_d, sum_dx, sum_dy;  /* contrast mass and contrast-weighted coordinate sums */
+    int32_t min_d, max_d;
+} cvvp_component_stats; /* 104 bytes */
+CVVP_API int cvvp_highlight_set_component_stats(cvvp_ctx *ctx, int on);
+CVVP_API int cvvp_highlight_component_stats(const cvvp_ctx *ctx);
 /* Device implementation used by the calls above (after cvvp_highlight_begin; both give identical masks):
  *   0 = fused (default): one persistent-CTA kernel launch per batch, run-based labelling (csrc/highlight_fused.cu)
  *   1 = per-pixel kernels (csrc/highlight.cu), ~35 launches per batch; kept as an on-device cross-check.
