@@ -75,6 +75,8 @@ def load():
         "cvvp_highlight_end": (i32, [vp]),
         "cvvp_highlight_set_polarity": (i32, [vp, i32]),
         "cvvp_highlight_polarity": (i32, [vp]),
+        "cvvp_highlight_set_channels": (i32, [vp, i32]),
+        "cvvp_highlight_channels": (i32, [vp]),
         "cvvp_highlight_set_component_stats": (i32, [vp, i32]),
         "cvvp_highlight_component_stats": (i32, [vp]),
         "cvvp_highlight_device_cc": (i32, [vp, vp, i64, sz, vp, sz, vp, i32, vp, vp, sz, vp]),
@@ -395,16 +397,21 @@ class Context:
                         threshold_hi: int, min_size_hyst: int, min_size_threshold: int, width_border: int = 0):
         bg = np.ascontiguousarray(background)
         se = np.ascontiguousarray(struct_element)
-        if bg.dtype != np.uint8 or bg.ndim != 2:
-            raise TypeError("background must be a 2-D uint8 array")
+        channels = self.highlight_channels()
+        if bg.dtype != np.uint8 or not (bg.ndim == 2 or (bg.ndim == 3 and bg.shape[2] == channels)) or \
+                (bg.ndim == 2 and channels != 1):
+            raise TypeError("background must be a uint8 array (H, W), or (H, W, C) with C the context's channels "
+                            f"({channels})")
         if se.dtype != np.uint8 or se.ndim != 2:
             raise TypeError("struct_element must be a 2-D uint8 array (cv::morphologyEx asserts CV_8U)")
-        h, w = bg.shape
+        h, w = bg.shape[:2]
         kh, kw = se.shape
         self._check(self._lib.cvvp_highlight_begin(self._h, bg.ctypes.data, w, h, se.ctypes.data, kw, kh, threshold,
                                                    threshold_lo, threshold_hi, min_size_hyst, min_size_threshold,
                                                    width_border))
         self._hl_shape = (h, w)
+        # what one frame of the job is: (H, W), or (H, W, C) for a colour job (cvvp_highlight_set_channels)
+        self._hl_frame = (h, w) if channels == 1 else (h, w, channels)
         # the job's component records (cvvp_highlight_set_component_stats)
         self._hl_dtype = self.COMPONENT_STATS_DTYPE if self.highlight_component_stats() else self.COMPONENT_DTYPE
 
@@ -417,6 +424,14 @@ class Context:
 
     def highlight_polarity(self) -> int:
         return int(self._lib.cvvp_highlight_polarity(self._h))
+
+    def highlight_set_channels(self, channels: int):
+        """channels (1..4) of the frames and backgrounds of the highlight jobs that begin after this; d is the largest
+        per-channel difference of the polarity; none may be open"""
+        self._check(self._lib.cvvp_highlight_set_channels(self._h, channels))
+
+    def highlight_channels(self) -> int:
+        return int(self._lib.cvvp_highlight_channels(self._h))
 
     def highlight_set_component_stats(self, on: bool):
         """shape and contrast statistics in every component record (COMPONENT_STATS_DTYPE) of the highlight jobs that
@@ -434,14 +449,16 @@ class Context:
         return self._hl_dtype
 
     def highlight_frames(self, frames: np.ndarray) -> np.ndarray:
-        """frames: uint8 (n, H, W) -> masks uint8 (n, H, W) of 0/255"""
+        """frames: uint8 (n, H, W) (a colour job: (n, H, W, C)) -> masks uint8 (n, H, W) of 0/255"""
         frames = np.ascontiguousarray(frames)
-        if frames.dtype != np.uint8 or frames.ndim != 3 or frames.shape[1:] != self._hl_shape:
-            raise TypeError("frames must be uint8 of shape (n, H, W) matching the background")
+        if frames.dtype != np.uint8 or frames.shape[1:] != self._hl_frame:
+            raise TypeError(f"frames must be uint8 of shape (n, {', '.join(map(str, self._hl_frame))}) matching the "
+                            "background")
         n = frames.shape[0]
         npix = frames.shape[1] * frames.shape[2]
-        out = np.empty_like(frames)
-        self._check(self._lib.cvvp_highlight_frames(self._h, frames.ctypes.data, n, npix, out.ctypes.data, npix))
+        out = np.empty(frames.shape[:3], np.uint8)
+        self._check(self._lib.cvvp_highlight_frames(self._h, frames.ctypes.data, n, int(np.prod(self._hl_frame)),
+                                                    out.ctypes.data, npix))
         return out
 
     # numpy view of struct cvvp_component (include/cvvp.h)
@@ -458,15 +475,17 @@ class Context:
         every mask (structured array (n, max_comps) of the job's component dtype, raster-first order) and, if asked, the int32
         label images (0 = background, k = component k of that frame)."""
         frames = np.ascontiguousarray(frames)
-        if frames.dtype != np.uint8 or frames.ndim != 3 or frames.shape[1:] != self._hl_shape:
-            raise TypeError("frames must be uint8 of shape (n, H, W) matching the background")
+        if frames.dtype != np.uint8 or frames.shape[1:] != self._hl_frame:
+            raise TypeError(f"frames must be uint8 of shape (n, {', '.join(map(str, self._hl_frame))}) matching the "
+                            "background")
         n = frames.shape[0]
         npix = frames.shape[1] * frames.shape[2]
-        out = np.empty_like(frames)
+        out = np.empty(frames.shape[:3], np.uint8)
         comps = np.zeros((n, max_comps), self._hl_dtype)
         ncomps = np.zeros(n, np.int32)
-        lab = np.empty(frames.shape, np.int32) if labels else None
-        self._check(self._lib.cvvp_highlight_frames_cc(self._h, frames.ctypes.data, n, npix, out.ctypes.data, npix,
+        lab = np.empty(frames.shape[:3], np.int32) if labels else None
+        self._check(self._lib.cvvp_highlight_frames_cc(self._h, frames.ctypes.data, n, int(np.prod(self._hl_frame)),
+                                                       out.ctypes.data, npix,
                                                        comps.ctypes.data, max_comps, ncomps.ctypes.data,
                                                        lab.ctypes.data if labels else None, npix))
         return (out, comps, ncomps, lab) if labels else (out, comps, ncomps)

@@ -819,6 +819,26 @@ int cvvp_highlight_polarity(const cvvp_ctx *ctx)
     return ctx->polarity;
 }
 
+int cvvp_highlight_set_channels(cvvp_ctx *ctx, int channels)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    if (channels < 1 || channels > 4)
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: channels must be in 1..4, not %d", channels);
+    // an open job, its queue and its rolling stream took the channel count (and their buffers) in cvvp_highlight_begin
+    if (ctx->hl)
+        return fail(ctx, CVVP_ERR_STATE, "highlight: a highlight job is open on this context");
+    ctx->channels = channels;
+    return CVVP_OK;
+}
+
+int cvvp_highlight_channels(const cvvp_ctx *ctx)
+{
+    if (!ctx)
+        return fail(nullptr, CVVP_ERR_INVALID, "null context");
+    return ctx->channels;
+}
+
 int cvvp_highlight_set_component_stats(cvvp_ctx *ctx, int on)
 {
     if (!ctx)

@@ -112,6 +112,7 @@ struct cvvp_ctx {
     int percent{50}; // percentile of every background (cvvp_median_set_percentile); jobs take it when they begin
     int polarity{CVVP_POLARITY_DARK}; // object polarity (cvvp_highlight_set_polarity); highlight jobs take it when they begin
     int component_stats{0}; // cvvp_highlight_set_component_stats; highlight jobs take it when they begin
+    int channels{1}; // channels of highlight frames (cvvp_highlight_set_channels); highlight jobs take it when they begin
 };
 
 namespace cvvp
@@ -195,6 +196,20 @@ int highlight_check_cc(cvvp_ctx *ctx, long long n, const CcOut &cc);
 // frame f against the background at d_bgs + f * bg_stride (0 = one for all; d_bgs == nullptr: the job's own)
 int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, size_t frame_stride, const uint8_t *d_bgs,
                         size_t bg_stride, uint8_t *d_out, size_t out_stride, const CcOut &cc, cudaStream_t stream);
+// channels of the running job's frames (cvvp_highlight_set_channels); 0: no job
+int highlight_job_channels(const cvvp_ctx *ctx);
+// Colour job: the d planes (highlight_color.cu) of n frames at src + f * frame_stride against the backgrounds at
+// d_bgs + f * bg_stride (d_bgs == nullptr: the job's own) -> d_planes + f * pitch.  row_stride == 0: contiguous frames
+// of width*height*C bytes; else frame rows row_stride bytes apart whose pixels start at pixel x0 (a crop).
+int highlight_color_d(cvvp_ctx *ctx, const uint8_t *src, long long n, size_t frame_stride, size_t row_stride, int x0,
+                      const uint8_t *d_bgs, size_t bg_stride, uint8_t *d_planes, size_t pitch, cudaStream_t stream);
+// Colour job: the masks (and components) of n d planes of highlight_color_d
+int highlight_device_planes(cvvp_ctx *ctx, const uint8_t *d_planes, long long n, size_t pitch, uint8_t *d_out,
+                            size_t out_stride, const CcOut &cc, cudaStream_t stream);
+// highlight_color.cu: d = max over the channels (2..4) of the polarity's difference, rows of row_len pixels
+int color_diff_launch(cvvp_ctx *ctx, int channels, int polarity, const uint8_t *src, long long n, size_t frame_stride,
+                      size_t row_stride, int x0, const uint8_t *bg, size_t bg_stride, uint32_t row_len, uint32_t nrows,
+                      uint8_t *dst, size_t dst_pitch, cudaStream_t stream);
 int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, size_t frame_stride, uint8_t *masks_out,
                              size_t out_stride, cvvp_component *comps_out, int max_comps, int *ncomps_out,
                              int32_t *labels_out, size_t labels_stride);

@@ -330,6 +330,14 @@ int highlight_stream_check(cvvp_ctx *ctx, const char *who, bool begun, int args_
     const int rc = frames_check_format(ctx, fmt);
     if (rc != CVVP_OK)
         return rc;
+    const int C = highlight_job_channels(ctx);
+    if (C > 1) { // a colour job takes the cropped frames as they are: its kernel computes d from all their channels
+        if (fmt->mode != CVVP_FRAMES_AS_IS || fmt->src_channels != C || fmt->crop_width != *W || fmt->crop_height != *H)
+            return fail(ctx, CVVP_ERR_INVALID,
+                        "%s: frames of a %d-channel highlight job must be CVVP_FRAMES_AS_IS with src_channels %d, cropped "
+                        "to %dx%d like the background", who, C, C, *W, *H);
+        return CVVP_OK;
+    }
     if (fmt->crop_width != *W || fmt->crop_height != *H || frames_out_bytes(*fmt) != size_t(*W) * size_t(*H))
         return fail(ctx, CVVP_ERR_INVALID,
                     "%s: prepared frames must be single-channel %dx%d like the background (cv::findContours requires 8UC1)",
@@ -356,6 +364,7 @@ struct HighlightQueue {
     long long max_batch{0};
     bool has_fmt{false};
     cvvp_frame_format fmt{};
+    bool color{false};        // a colour job: the uploaded frames go through highlight_color_d into d_in
     size_t npix{0}, pitch{0}; // prepared frame bytes / device pitch
     size_t in_bytes{0}, in_pitch{0}, in_offset{0}; // what one frame uploads (crop band or the frame) and where it starts
     size_t host_pitch{0};                          // bytes between the caller's frames in a slot's pinned input
@@ -407,6 +416,7 @@ int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const c
         q->fmt = *fmt;
     q->npix = size_t(W) * size_t(H);
     q->pitch = round_up(q->npix, 128);
+    q->color = highlight_job_channels(ctx) > 1;
     if (fmt) {
         const Band band = crop_band(*fmt);
         q->in_bytes = band.bytes;
@@ -414,10 +424,10 @@ int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const c
         q->in_offset = band.offset;
         q->host_pitch = round_up(size_t(fmt->src_width) * size_t(fmt->src_height) * size_t(fmt->src_channels), 64);
     } else {
-        q->in_bytes = q->npix;
-        q->in_pitch = q->pitch;
+        q->in_bytes = q->npix * size_t(highlight_job_channels(ctx));
+        q->in_pitch = round_up(q->in_bytes, 128);
         q->in_offset = 0;
-        q->host_pitch = q->pitch;
+        q->host_pitch = q->in_pitch;
     }
     q->slots.resize(size_t(depth));
     const size_t nb = size_t(max_batch);
@@ -438,7 +448,7 @@ int highlight_queue_begin(cvvp_ctx *ctx, int depth, long long max_batch, const c
             s.h_in = static_cast<uint8_t *>(h);
             s.b_h_in = nb * q->host_pitch;
         }
-        if (fmt)
+        if (fmt || q->color)
             ok = ok && dev(s.d_raw, s.b_raw, nb * q->in_pitch);
         ok = ok && dev(s.d_in, s.b_in, nb * q->pitch);
         ok = ok && cudaEventCreateWithFlags(&s.up, cudaEventDisableTiming) == cudaSuccess;
@@ -463,12 +473,24 @@ int highlight_queue_pending(const cvvp_ctx *ctx)
 static int launch_slot(cvvp_ctx *ctx, HighlightQueue *q, HqSlot &s, long long n)
 {
     s.res.n = n;
-    uint8_t *up_to = q->has_fmt ? s.d_raw : s.d_in;
+    uint8_t *up_to = q->has_fmt || q->color ? s.d_raw : s.d_in;
     CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(up_to, q->in_pitch, s.h_in + q->in_offset, q->host_pitch, q->in_bytes, size_t(n),
                                         cudaMemcpyHostToDevice, ctx->copy));
     CVVP_CUDA_OK(ctx, cudaEventRecord(s.up, ctx->copy));
     CVVP_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->compute, s.up, 0));
     int rc;
+    if (q->color) {
+        // one kernel makes the d planes straight from the uploaded frames (the crop of the decoded rows with a format)
+        const size_t row_stride = q->has_fmt ? size_t(q->fmt.src_width) * size_t(q->fmt.src_channels) : 0;
+        rc = highlight_color_d(ctx, s.d_raw, n, q->in_pitch, row_stride, q->has_fmt ? q->fmt.crop_x : 0, nullptr, 0, s.d_in,
+                               q->pitch, ctx->compute);
+        if (rc == CVVP_OK)
+            rc = highlight_device_planes(ctx, s.d_in, n, q->pitch, s.res.d_out, q->pitch, hl_results_cc(s.res, 0),
+                                         ctx->compute);
+        if (rc != CVVP_OK)
+            return rc;
+        return hl_results_download(ctx, s.res);
+    }
     if (q->has_fmt) {
         rc = frames_prepare_launch(ctx, s.d_raw, n, q->in_pitch, size_t(n) * q->in_pitch, q->fmt, q->fmt.crop_y, s.d_in, q->pitch,
                                    ctx->compute);

@@ -27,6 +27,7 @@
 // Layout: every kernel takes blockIdx.z = frame of the batch.  Masks are u8 0/1 (npix per frame), label / statistic
 // arrays are u32 / i32 with npix + 1 entries per frame (entry npix = the FRAME node).
 #include "highlight_state.hpp"
+#include "pool.hpp"
 
 #include <cstddef>
 #include <new>
@@ -533,10 +534,12 @@ void free_state(HighlightState *s)
     if (!s)
         return;
     void *ptrs[] = {s->d_bg, s->d_offs, s->m_a, s->m_u, s->m_l, s->m_t, s->m_out, s->lab0, s->lab1,
-                    s->st_s, s->st_e, s->st_x, s->d_th, s->d_hist, s->d_in, s->d_res, s->d_comps, s->d_ncomps, s->d_labels};
+                    s->st_s, s->st_e, s->st_x, s->d_th, s->d_hist, s->d_in, s->d_res, s->d_comps, s->d_ncomps, s->d_labels,
+                    s->d_cbg};
     for (void *p : ptrs)
         if (p)
             cudaFree(p);
+    pool_dev_free(s->d_planes, s->planes_bytes);
     fused_release(s);
     delete s;
 }
@@ -612,6 +615,11 @@ size_t highlight_record_bytes(const cvvp_ctx *ctx)
     return ctx->hl && ctx->hl->component_stats ? sizeof(cvvp_component_stats) : sizeof(cvvp_component);
 }
 
+int highlight_job_channels(const cvvp_ctx *ctx)
+{
+    return ctx->hl ? ctx->hl->channels : 0;
+}
+
 bool highlight_geometry(const cvvp_ctx *ctx, int *width, int *height)
 {
     if (!ctx->hl)
@@ -646,6 +654,12 @@ int highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, int hei
     st->min_hyst = min_size_hyst;
     st->min_th = min_size_threshold;
     st->polarity = ctx->polarity; // the job keeps the polarity it began with
+    st->channels = ctx->channels; // and its channel count
+    if (st->channels > 1) {
+        // the grey kernels read the job's d planes against a zero background, where BRIGHT gives max(d - 0, 0) = d
+        st->color_polarity = st->polarity;
+        st->polarity = CVVP_POLARITY_BRIGHT;
+    }
     st->component_stats = ctx->component_stats; // and its component record size (highlight_record_bytes)
     // structuring element -> offsets relative to the anchor (kw/2, kh/2); any non-zero entry is set.  A kernel with
     // no non-zero entry is filtered by OpenCV as if only its element (0,0) were set.
@@ -662,12 +676,17 @@ int highlight_begin(cvvp_ctx *ctx, const uint8_t *background, int width, int hei
     st->dy_min = offs.front().y;
     st->dy_max = offs.back().y;
     int rc;
-    if ((rc = dev_alloc(ctx, &st->d_bg, st->g.npix)) != CVVP_OK || (rc = dev_alloc(ctx, &st->d_offs, offs.size())) != CVVP_OK) {
+    const bool color = st->channels > 1;
+    const size_t bg_bytes = size_t(st->g.npix) * size_t(st->channels);
+    if ((rc = dev_alloc(ctx, &st->d_bg, st->g.npix)) != CVVP_OK || (rc = dev_alloc(ctx, &st->d_offs, offs.size())) != CVVP_OK ||
+        (color && (rc = dev_alloc(ctx, &st->d_cbg, bg_bytes)) != CVVP_OK)) {
         highlight_release(ctx);
         return rc;
     }
     cudaError_t e;
-    if ((e = cudaMemcpy(st->d_bg, background, st->g.npix, cudaMemcpyHostToDevice)) != cudaSuccess ||
+    if ((e = color ? cudaMemcpy(st->d_cbg, background, bg_bytes, cudaMemcpyHostToDevice) : cudaSuccess) != cudaSuccess ||
+        (e = color ? cudaMemset(st->d_bg, 0, st->g.npix) : cudaMemcpy(st->d_bg, background, st->g.npix, cudaMemcpyHostToDevice)) !=
+            cudaSuccess ||
         (e = cudaMemcpy(st->d_offs, offs.data(), offs.size() * sizeof(short2), cudaMemcpyHostToDevice)) != cudaSuccess) {
         highlight_release(ctx);
         return fail(ctx, CVVP_ERR_CUDA, "highlight: upload failed: %s", cudaGetErrorString(e));
@@ -829,15 +848,70 @@ static int highlight_run(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_fra
     return CVVP_OK;
 }
 
+// the component outputs of frames [first, ...) of cc
+static CcOut cc_from(const CcOut &cc, long long first)
+{
+    CcOut o = cc;
+    if (o.comps)
+        o.comps = reinterpret_cast<cvvp_component *>(reinterpret_cast<uint8_t *>(o.comps) +
+                                                     size_t(first) * size_t(o.max_comps) * o.rec_bytes);
+    if (o.ncomps)
+        o.ncomps += first;
+    if (o.labels)
+        o.labels += size_t(first) * o.labels_stride;
+    return o;
+}
+
+// Colour job: the d planes of a chunk of frames go into the job's scratch (highlight_color.cu), then the grey path
+// runs on them against the zero background.  Chunks hold the frames one launch keeps in flight, so that splitting
+// the call costs the kernels no occupancy; at most about 1 GB of scratch.
+static int highlight_color_run(cvvp_ctx *ctx, HighlightState *st, const uint8_t *d_frames, long long n, size_t frame_stride,
+                               const uint8_t *d_bgs, size_t bg_stride, uint8_t *d_out, size_t out_stride, const CcOut &cc,
+                               cudaStream_t stream)
+{
+    const size_t pitch = round_up(st->g.npix, 128);
+    long long chunk = use_fused(st) ? fused_frames_in_flight(ctx, st) : pick_batch(st, n);
+    const long long by_mem = (long long)((size_t(1) << 30) / pitch);
+    if (chunk > by_mem) chunk = by_mem;
+    if (chunk < 1) chunk = 1;
+    if (chunk > n) chunk = n;
+    if (st->planes_bytes < size_t(chunk) * pitch) {
+        // work queued earlier on this stream may still read the old scratch
+        CVVP_CUDA_OK(ctx, cudaStreamSynchronize(stream));
+        pool_dev_free(st->d_planes, st->planes_bytes);
+        st->d_planes = nullptr;
+        st->planes_bytes = 0;
+        void *p = nullptr;
+        if (pool_dev_alloc(&p, size_t(chunk) * pitch) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(ctx, CVVP_ERR_NOMEM, "highlight: allocation of %lld difference planes failed", chunk);
+        }
+        st->d_planes = static_cast<uint8_t *>(p);
+        st->planes_bytes = size_t(chunk) * pitch;
+    }
+    for (long long done = 0; done < n; done += chunk) {
+        const long long nb = n - done < chunk ? n - done : chunk;
+        int rc = highlight_color_d(ctx, d_frames + size_t(done) * frame_stride, nb, frame_stride, 0, 0,
+                                   d_bgs + size_t(done) * bg_stride, bg_stride, st->d_planes, pitch, stream);
+        if (rc == CVVP_OK)
+            rc = highlight_run(ctx, st, st->d_planes, nb, pitch, st->d_bg, 0, d_out + size_t(done) * out_stride, out_stride,
+                               cc_from(cc, done), stream);
+        if (rc != CVVP_OK)
+            return rc;
+    }
+    return CVVP_OK;
+}
+
 static_assert(sizeof(cvvp_component) == 48, "cvvp_component is part of the C ABI (include/cvvp.h, _cabi.COMPONENT_DTYPE)");
 static_assert(sizeof(cvvp_component_stats) == 104 && offsetof(cvvp_component_stats, c) == 0,
               "cvvp_component_stats is part of the C ABI (include/cvvp.h, _cabi.COMPONENT_STATS_DTYPE)");
 
-// [p, p + (n - 1) * stride + bytes) and [q, ...) share a byte
-static bool frames_overlap(const uint8_t *p, size_t p_stride, const uint8_t *q, size_t q_stride, long long n, size_t bytes)
+// [p, p + (n - 1) * p_stride + p_bytes) and [q, q + (n - 1) * q_stride + q_bytes) share a byte
+static bool frames_overlap(const uint8_t *p, size_t p_stride, size_t p_bytes, const uint8_t *q, size_t q_stride,
+                           size_t q_bytes, long long n)
 {
     const uintptr_t a0 = reinterpret_cast<uintptr_t>(p), b0 = reinterpret_cast<uintptr_t>(q);
-    const uintptr_t a1 = a0 + size_t(n - 1) * p_stride + bytes, b1 = b0 + size_t(n - 1) * q_stride + bytes;
+    const uintptr_t a1 = a0 + size_t(n - 1) * p_stride + p_bytes, b1 = b0 + size_t(n - 1) * q_stride + q_bytes;
     return a0 < b1 && b0 < a1;
 }
 
@@ -861,9 +935,9 @@ int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, siz
     HighlightState *st = ctx->hl;
     if (!st)
         return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
-    if (!d_frames || !d_out || n < 0 || frame_stride < st->g.npix || out_stride < st->g.npix ||
-        (bg_stride != 0 && bg_stride < st->g.npix))
-        return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments (bg_stride must be 0 or at least %u)", st->g.npix);
+    const size_t fb = size_t(st->g.npix) * size_t(st->channels); // bytes of a frame and of a background
+    if (!d_frames || !d_out || n < 0 || frame_stride < fb || out_stride < st->g.npix || (bg_stride != 0 && bg_stride < fb))
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments (bg_stride must be 0 or at least %zu)", fb);
     const bool want_cc = cc.comps || cc.ncomps || cc.labels;
     if (want_cc) {
         const int rc = highlight_check_cc(ctx, n, cc);
@@ -872,20 +946,57 @@ int highlight_device_bg(cvvp_ctx *ctx, const uint8_t *d_frames, long long n, siz
     }
     if (n == 0)
         return CVVP_OK;
+    const bool color = st->channels > 1;
     if (!d_bgs) {
-        d_bgs = st->d_bg;
+        d_bgs = color ? st->d_cbg : st->d_bg;
         bg_stride = 0;
     }
+    const size_t np = st->g.npix;
+    // a colour job's d is computed chunk by chunk ahead of the masks: a mask must not land on a frame still to be read
+    if (color && (frames_overlap(d_out, out_stride, np, d_frames, frame_stride, fb, n) ||
+                  frames_overlap(d_out, out_stride, np, d_bgs, bg_stride, fb, n)))
+        return fail(ctx, CVVP_ERR_INVALID, "highlight: d_out overlaps the frames or the backgrounds");
     CcOut job_cc = want_cc ? cc : CcOut();
     if (want_cc && st->component_stats) {
         // the statistics read frame and background bytes after the kernel has written the frame's mask
-        if (frames_overlap(d_out, out_stride, d_frames, frame_stride, n, st->g.npix) ||
-            frames_overlap(d_out, out_stride, d_bgs, bg_stride, n, st->g.npix))
+        if (frames_overlap(d_out, out_stride, np, d_frames, frame_stride, np, n) ||
+            frames_overlap(d_out, out_stride, np, d_bgs, bg_stride, np, n))
             return fail(ctx, CVVP_ERR_INVALID,
                         "highlight component statistics: d_out overlaps the frames or the backgrounds");
         job_cc.rec_bytes = sizeof(cvvp_component_stats);
     }
+    if (color)
+        return highlight_color_run(ctx, st, d_frames, n, frame_stride, d_bgs, bg_stride, d_out, out_stride, job_cc, stream);
     return highlight_run(ctx, st, d_frames, n, frame_stride, d_bgs, bg_stride, d_out, out_stride, job_cc, stream);
+}
+
+int highlight_color_d(cvvp_ctx *ctx, const uint8_t *src, long long n, size_t frame_stride, size_t row_stride, int x0,
+                      const uint8_t *d_bgs, size_t bg_stride, uint8_t *d_planes, size_t pitch, cudaStream_t stream)
+{
+    const HighlightState *st = ctx->hl;
+    if (!d_bgs) {
+        d_bgs = st->d_cbg;
+        bg_stride = 0;
+    }
+    const bool rows = row_stride != 0;
+    return color_diff_launch(ctx, st->channels, st->color_polarity, src, n, frame_stride, row_stride, x0, d_bgs, bg_stride,
+                             rows ? uint32_t(st->g.W) : st->g.npix, rows ? uint32_t(st->g.H) : 1u, d_planes, pitch, stream);
+}
+
+int highlight_device_planes(cvvp_ctx *ctx, const uint8_t *d_planes, long long n, size_t pitch, uint8_t *d_out,
+                            size_t out_stride, const CcOut &cc, cudaStream_t stream)
+{
+    HighlightState *st = ctx->hl;
+    const bool want_cc = cc.comps || cc.ncomps || cc.labels;
+    if (want_cc) {
+        const int rc = highlight_check_cc(ctx, n, cc);
+        if (rc != CVVP_OK)
+            return rc;
+    }
+    CcOut job_cc = want_cc ? cc : CcOut();
+    if (want_cc && st->component_stats)
+        job_cc.rec_bytes = sizeof(cvvp_component_stats);
+    return highlight_run(ctx, st, d_planes, n, pitch, st->d_bg, 0, d_out, out_stride, job_cc, stream);
 }
 
 template <typename T>
@@ -914,13 +1025,14 @@ int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, 
     HighlightState *st = ctx->hl;
     if (!st)
         return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
-    if (!frames || !masks_out || !comps_out || !ncomps_out || max_comps < 1 || n < 0 || frame_stride < st->g.npix ||
-        out_stride < st->g.npix || (labels_out && labels_stride < st->g.npix))
+    const size_t np = st->g.npix;
+    const size_t fb = np * size_t(st->channels); // bytes of a frame
+    if (!frames || !masks_out || !comps_out || !ncomps_out || max_comps < 1 || n < 0 || frame_stride < fb ||
+        out_stride < np || (labels_out && labels_stride < np))
         return fail(ctx, CVVP_ERR_INVALID, "highlight components: bad arguments");
     if (n == 0)
         return CVVP_OK;
-    const size_t np = st->g.npix;
-    const size_t pitch = (np + 127) & ~size_t(127);
+    const size_t pitch = round_up(fb, 128); // of the frames on the device; the masks keep it too
     long long chunk = fused_supports(st) ? fused_frames_in_flight(ctx, st) : 16;
     if (chunk > n)
         chunk = n;
@@ -942,7 +1054,7 @@ int highlight_frames_host_cc(cvvp_ctx *ctx, const uint8_t *frames, long long n, 
     cudaStream_t s = ctx->compute;
     for (long long done = 0; done < n; done += chunk) {
         const long long nb = n - done < chunk ? n - done : chunk;
-        CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(st->d_in, pitch, frames + size_t(done) * frame_stride, frame_stride, np, size_t(nb),
+        CVVP_CUDA_OK(ctx, cudaMemcpy2DAsync(st->d_in, pitch, frames + size_t(done) * frame_stride, frame_stride, fb, size_t(nb),
                                             cudaMemcpyHostToDevice, s));
         rc = highlight_device_bg(ctx, st->d_in, nb, pitch, nullptr, 0, st->d_res, pitch,
                                  CcOut{reinterpret_cast<cvvp_component *>(st->d_comps), max_comps, st->d_ncomps,
@@ -970,7 +1082,9 @@ int highlight_frames_host(cvvp_ctx *ctx, const uint8_t *frames, long long n, siz
     HighlightState *st = ctx->hl;
     if (!st)
         return fail(ctx, CVVP_ERR_STATE, "highlight: no parameters set (call cvvp_highlight_begin first)");
-    if (!frames || !masks_out || n < 0 || frame_stride < st->g.npix || out_stride < st->g.npix)
+    const size_t np = st->g.npix;
+    const size_t fb = np * size_t(st->channels); // bytes of a frame
+    if (!frames || !masks_out || n < 0 || frame_stride < fb || out_stride < np)
         return fail(ctx, CVVP_ERR_INVALID, "highlight: bad arguments");
     if (n == 0)
         return CVVP_OK;
@@ -988,8 +1102,8 @@ int highlight_frames_host(cvvp_ctx *ctx, const uint8_t *frames, long long n, siz
     } else {
         chunk = pick_batch(st, n);
     }
-    const size_t np = st->g.npix;
-    const size_t pitch = (np + 127) & ~size_t(127); // device frame pitch: keeps every frame 16-byte aligned
+    // device frame pitch: keeps every frame 16-byte aligned (the masks keep the frames' pitch)
+    const size_t pitch = round_up(fb, 128);
     const size_t need = size_t(chunk) * pitch;
     if (st->in_bytes < need) {
         if (st->d_in) cudaFree(st->d_in);
@@ -1017,7 +1131,7 @@ int highlight_frames_host(cvvp_ctx *ctx, const uint8_t *frames, long long n, siz
         uint8_t *dres = st->d_res + size_t(b) * half;
         if (idx >= 2)
             cudaStreamWaitEvent(ctx->copy, kdone[b], 0); // the kernel that read this input half has finished
-        cudaError_t e = cudaMemcpy2DAsync(din, pitch, frames + size_t(done) * frame_stride, frame_stride, np, size_t(nb),
+        cudaError_t e = cudaMemcpy2DAsync(din, pitch, frames + size_t(done) * frame_stride, frame_stride, fb, size_t(nb),
                                           cudaMemcpyHostToDevice, ctx->copy);
         if (e != cudaSuccess) {
             rc = fail(ctx, CVVP_ERR_CUDA, "highlight: H2D failed: %s", cudaGetErrorString(e));

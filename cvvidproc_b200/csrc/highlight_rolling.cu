@@ -39,7 +39,8 @@ struct RollingStream {
     cvvp_frame_format fmt{};
     int max_comps{0};
     bool labels{false};
-    size_t npix{0}, pitch{0}, in_bytes{0}; // prepared frame bytes / device pitch / bytes of one pushed frame
+    size_t npix{0}, pitch{0}, in_bytes{0}; // mask bytes / mask pitch / bytes of one pushed frame
+    size_t nelem{0}, fpitch{0};            // bytes of a prepared frame (npix * the job's channels) / its pitch in the ring
     long long ring{0};                     // frames the ring holds
     uint8_t *d_ring{nullptr}, *d_bgs{nullptr};
     size_t b_ring{0}, b_bgs{0};
@@ -91,26 +92,29 @@ int highlight_rolling_begin(cvvp_ctx *ctx, int window, long long max_batch, cons
     r->labels = labels != 0;
     r->npix = size_t(W) * size_t(H);
     r->pitch = round_up(r->npix, 128);
-    r->in_bytes = fmt ? size_t(fmt->src_width) * size_t(fmt->src_height) * size_t(fmt->src_channels) : r->npix;
+    // a colour job's ring holds colour frames, and its backgrounds are colour too (the median is element-wise)
+    r->nelem = r->npix * size_t(highlight_job_channels(ctx));
+    r->fpitch = round_up(r->nelem, 128);
+    r->in_bytes = fmt ? size_t(fmt->src_width) * size_t(fmt->src_height) * size_t(fmt->src_channels) : r->nelem;
     r->ring = (long long)window + max_batch;
     void *p = nullptr;
-    if (pool_dev_alloc(&p, size_t(r->ring) * r->pitch) != cudaSuccess) {
+    if (pool_dev_alloc(&p, size_t(r->ring) * r->fpitch) != cudaSuccess) {
         cudaGetLastError();
-        const size_t bytes = size_t(r->ring) * r->pitch;
+        const size_t bytes = size_t(r->ring) * r->fpitch;
         highlight_rolling_release(ctx);
         return fail(ctx, CVVP_ERR_NOMEM,
                     "rolling highlight: the ring of %lld frames (window %d + batch %lld, %zu bytes) does not fit on the device; "
                     "use a smaller window", (long long)window + max_batch, window, max_batch, bytes);
     }
     r->d_ring = static_cast<uint8_t *>(p);
-    r->b_ring = size_t(r->ring) * r->pitch;
-    if (pool_dev_alloc(&p, size_t(max_batch) * r->pitch) != cudaSuccess) {
+    r->b_ring = size_t(r->ring) * r->fpitch;
+    if (pool_dev_alloc(&p, size_t(max_batch) * r->fpitch) != cudaSuccess) {
         cudaGetLastError();
         highlight_rolling_release(ctx);
         return fail(ctx, CVVP_ERR_NOMEM, "rolling highlight: allocation of %lld backgrounds failed", max_batch);
     }
     r->d_bgs = static_cast<uint8_t *>(p);
-    r->b_bgs = size_t(max_batch) * r->pitch;
+    r->b_bgs = size_t(max_batch) * r->fpitch;
     return CVVP_OK;
 }
 
@@ -155,16 +159,16 @@ static int launch_ready(cvvp_ctx *ctx, RollingStream *r)
         s->first = t0;
         s->res.n = n;
         r->pending.push_back(s);
-        rc = median_roll_launch(ctx, r->d_ring, r->ring, r->pitch, r->received, r->npix, r->window, r->percent, t0, t0 + n,
-                                r->d_bgs, r->pitch, ctx->compute);
+        rc = median_roll_launch(ctx, r->d_ring, r->ring, r->fpitch, r->received, r->nelem, r->window, r->percent, t0, t0 + n,
+                                r->d_bgs, r->fpitch, ctx->compute);
         if (rc != CVVP_OK)
             return rc;
         // the frames themselves, in at most two contiguous runs of ring slots
         for (long long done = 0; done < n;) {
             const long long slot = (t0 + done) % r->ring;
             const long long k = n - done < r->ring - slot ? n - done : r->ring - slot;
-            rc = highlight_device_bg(ctx, r->d_ring + size_t(slot) * r->pitch, k, r->pitch,
-                                     r->d_bgs + size_t(done) * r->pitch, r->pitch, s->res.d_out + size_t(done) * r->pitch,
+            rc = highlight_device_bg(ctx, r->d_ring + size_t(slot) * r->fpitch, k, r->fpitch,
+                                     r->d_bgs + size_t(done) * r->fpitch, r->fpitch, s->res.d_out + size_t(done) * r->pitch,
                                      r->pitch, hl_results_cc(s->res, done), ctx->compute);
             if (rc != CVVP_OK)
                 return rc;
@@ -203,13 +207,13 @@ int highlight_rolling_push(cvvp_ctx *ctx, const uint8_t *frames, long long n, si
     for (long long done = 0; done < n;) {
         const long long slot = (r->received + done) % r->ring;
         const long long k = n - done < r->ring - slot ? n - done : r->ring - slot;
-        uint8_t *dst = r->d_ring + size_t(slot) * r->pitch;
+        uint8_t *dst = r->d_ring + size_t(slot) * r->fpitch;
         if (r->has_fmt) {
-            rc = frames_upload_prepare(ctx, frames + size_t(done) * frame_stride, k, frame_stride, r->fmt, dst, r->pitch);
+            rc = frames_upload_prepare(ctx, frames + size_t(done) * frame_stride, k, frame_stride, r->fmt, dst, r->fpitch);
             if (rc != CVVP_OK)
                 return drain_after_failure(ctx, r->failed, rc);
         } else {
-            const cudaError_t e = cudaMemcpy2DAsync(dst, r->pitch, frames + size_t(done) * frame_stride, frame_stride, r->npix,
+            const cudaError_t e = cudaMemcpy2DAsync(dst, r->fpitch, frames + size_t(done) * frame_stride, frame_stride, r->nelem,
                                                     size_t(k), cudaMemcpyHostToDevice, ctx->compute);
             if (e != cudaSuccess)
                 return drain_after_failure(ctx, r->failed,

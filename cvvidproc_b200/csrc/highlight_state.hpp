@@ -40,12 +40,21 @@ __device__ __forceinline__ int hl_diff(int bg, int fr, int polarity)
 struct HighlightState {
     HlGeom g{};
     int th{}, lo{}, hi{}, min_hyst{}, min_th{};
-    int polarity{CVVP_POLARITY_DARK}; // the context's polarity when the job began (cvvp_highlight_set_polarity)
+    // polarity of the grey kernels' difference: the context's polarity when the job began (cvvp_highlight_set_polarity),
+    // except for a colour job, whose kernels read its d planes against the zero d_bg in BRIGHT (highlight_color.cu)
+    int polarity{CVVP_POLARITY_DARK};
+    int channels{1};                    // the context's cvvp_highlight_set_channels when the job began
+    int color_polarity{CVVP_POLARITY_DARK}; // colour job: the polarity its d planes are computed in
     int component_stats{0}; // the context's cvvp_highlight_set_component_stats when the job began
     int noffs{0};
     int dy_min{0}, dy_max{0}; // row range of the structuring element's taps (offsets are sorted by row, then column)
     int path{kPathFused};
-    uint8_t *d_bg{nullptr};
+    uint8_t *d_bg{nullptr}; // the background; all zero for a colour job
+    uint8_t *d_cbg{nullptr}; // colour job: the background, npix * channels bytes
+    // colour job: d planes of a chunk of frames (pooled, pool.hpp).  Like the fused kernel's scratch, it is reused in
+    // stream order on the call's stream: work in flight on a context's highlight scratch is on one stream at a time.
+    uint8_t *d_planes{nullptr};
+    size_t planes_bytes{0};
     short2 *d_offs{nullptr};
     std::vector<short2> h_offs; // host copy of the taps
     // per-pixel path: per-batch work buffers

@@ -297,7 +297,7 @@ private:
 // ---------------------------------------------------------------------------------------------------------------------
 struct GpuHighlightPack { // TokenProcessorPack<HighlightObjectsAlgo> :21-32
     int device{-1};
-    FrameBatch background{};     // 1 frame, 1 channel
+    FrameBatch background{};     // 1 frame of `channels` channels
     FrameBatch struct_element{}; // 1 "frame" of kh x kw bytes
     int threshold{}, threshold_lo{}, threshold_hi{}, min_size_hyst{}, min_size_threshold{}, width_border{};
     // opt-in extras (no counterpart in the reference's pack): 8-connected components of every mask for the tracker
@@ -312,6 +312,7 @@ struct GpuHighlightPack { // TokenProcessorPack<HighlightObjectsAlgo> :21-32
     long long max_batch{0};
     SourceFormat source{}; // enabled (queue mode only): tokens are DECODED frames, prepared on the device
     int polarity{CVVP_POLARITY_DARK}; // which difference image the masks start from (cvvp_highlight_set_polarity)
+    int channels{1}; // channels of the frames and the background (cvvp_highlight_set_channels)
 };
 
 // What the two highlight operators below share: the job's parameters, the check of a token's geometry, and the
@@ -320,8 +321,9 @@ inline void begin_highlight(const Context &ctx, const GpuHighlightPack &p)
 {
     CVVP_ASSERT(!p.background.empty());
     CVVP_ASSERT(!p.struct_element.empty());
-    CVVP_ASSERT_MSG(p.background.channels == 1, "the highlight stage works on single-channel frames");
+    CVVP_ASSERT_MSG(p.background.channels == p.channels, "the background's channels must be the highlight stage's");
     ctx.check(cvvp_highlight_set_polarity(ctx.get(), p.polarity));
+    ctx.check(cvvp_highlight_set_channels(ctx.get(), p.channels));
     ctx.check(cvvp_highlight_set_component_stats(ctx.get(), p.component_stats ? 1 : 0));
     ctx.check(cvvp_highlight_begin(ctx.get(), p.background.data.data(), p.background.cols, p.background.rows,
                                    p.struct_element.data.data(), p.struct_element.cols, p.struct_element.rows, p.threshold,
@@ -336,7 +338,7 @@ inline void check_token_geometry(const GpuHighlightPack &p, const FrameBatch &b)
                             b.channels == p.source.fmt.src_channels,
                         "decoded frame geometry must match the source format");
     else
-        CVVP_ASSERT_MSG(b.channels == 1 && b.rows == p.background.rows && b.cols == p.background.cols,
+        CVVP_ASSERT_MSG(b.channels == p.channels && b.rows == p.background.rows && b.cols == p.background.cols,
                         "frame geometry must match the background");
 }
 
@@ -410,12 +412,14 @@ public:
             batch->rec_bytes = record_bytes(m_pack);
             batch->comps.assign(std::size_t(batch->n) * m_pack.max_components * batch->rec_bytes, 0);
             batch->ncomps.assign(std::size_t(batch->n), 0);
+            // a colour token's masks land in place at its frame stride; its labels are one int32 per pixel
+            const std::size_t npix = std::size_t(batch->rows) * batch->cols;
             if (m_pack.labels)
-                batch->labels.resize(std::size_t(batch->n) * batch->frame_bytes());
+                batch->labels.resize(std::size_t(batch->n) * npix);
             m_ctx.check(cvvp_highlight_frames_cc(m_ctx.get(), batch->data.data(), batch->n, batch->frame_bytes(),
                                                  batch->data.data(), batch->frame_bytes(), batch->component_records(),
                                                  m_pack.max_components, batch->ncomps.data(),
-                                                 m_pack.labels ? batch->labels.data() : nullptr, batch->frame_bytes()));
+                                                 m_pack.labels ? batch->labels.data() : nullptr, npix));
         } else {
             m_ctx.check(cvvp_highlight_frames(m_ctx.get(), batch->data.data(), batch->n, batch->frame_bytes(),
                                               batch->data.data(), batch->frame_bytes()));

@@ -586,17 +586,18 @@ py::object GetVideoBackground(const VidBgPack &pack)
 // ---------------------------------------------------------------------------------------------------------------------
 // TrackObjects  (cv_vid_objecttrack_helpers.cpp:153-210, :30-150; assign_objects_algo.h:94-161)
 // ---------------------------------------------------------------------------------------------------------------------
-FrameBatch to_u8_image(const py::array &src, const char *what)
+// with_channels: an (h, w, C) array is accepted too (a colour background)
+FrameBatch to_u8_image(const py::array &src, const char *what, bool with_channels = false)
 {
     CVVP_ASSERT_MSG(src.size() > 0, what);
-    CVVP_ASSERT_MSG(src.ndim() == 2, "expected a 2-D array");
+    CVVP_ASSERT_MSG(src.ndim() == 2 || (with_channels && src.ndim() == 3), "expected a 2-D array");
     CVVP_ASSERT_MSG(src.dtype().is(py::dtype::of<std::uint8_t>()), "expected a uint8 array (OpenCV asserts CV_8U here)");
     u8array a = u8array::ensure(src);
     FrameBatch b;
     b.n = 1;
     b.rows = int(a.shape(0));
     b.cols = int(a.shape(1));
-    b.channels = 1;
+    b.channels = a.ndim() == 3 ? int(a.shape(2)) : 1;
     b.data.assign(a.data(), a.data() + a.size());
     return b;
 }
@@ -672,6 +673,21 @@ bool component_stats(const py::dict &kwargs)
     return on;
 }
 
+// kwargs["cvvp_color"]: false when absent, else exactly a bool; True keeps every channel of the decoded frames, so it
+// cannot go with grayscale or vid_is_grayscale (RuntimeError otherwise)
+bool color_frames(const py::dict &kwargs, bool grayscale, bool vid_is_grayscale)
+{
+    if (!kwargs.contains("cvvp_color"))
+        return false;
+    py::object v = kwargs["cvvp_color"];
+    CVVP_ASSERT_MSG(py::isinstance<py::bool_>(v), "kwargs['cvvp_color'] must be True or False");
+    const bool on = v.cast<bool>();
+    CVVP_ASSERT_MSG(!on || (!grayscale && !vid_is_grayscale),
+                    "kwargs['cvvp_color'] = True uses the decoded frames' channels: it cannot go with grayscale or "
+                    "vid_is_grayscale");
+    return on;
+}
+
 py::dict TrackObjects(const VidObjectTrackPack &pack)
 {
     // Opt-in extra of this implementation (the reference has no counterpart): kwargs["cvvp_background_window"] = W
@@ -689,6 +705,10 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     const int polarity = object_polarity(pack.assign_objects_pack.kwargs);
     // kwargs["cvvp_component_stats"] = True (with cvvp_components) adds shape and contrast statistics to `components`
     const bool want_stats = component_stats(pack.assign_objects_pack.kwargs);
+    // kwargs["cvvp_color"] = True highlights the frames as decoded, with all their channels, against an (h, w, C)
+    // background: d is the largest per-channel difference (cvvp_highlight_set_channels), so objects that differ from
+    // the background in colour but not in grey level are found.
+    const bool color = color_frames(pack.assign_objects_pack.kwargs, pack.grayscale, pack.vid_is_grayscale);
     const bool rolling = roll_window > 0;
     FrameSource vid{pack.vid_path, pack.grayscale, pack.vid_is_grayscale};
     if (!vid.opened()) {
@@ -719,7 +739,7 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
     vid.configure();
 
     GpuHighlightPack hp;
-    hp.background = to_u8_image(bg, "background must not be empty");
+    hp.background = to_u8_image(bg, "background must not be empty", color);
     hp.struct_element = to_u8_image(pack.highlight_objects_pack.struct_element, "struct element must not be empty");
     hp.threshold = pack.highlight_objects_pack.threshold;
     hp.threshold_lo = pack.highlight_objects_pack.threshold_lo;
@@ -876,6 +896,16 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
                     masks.labels.empty() ? nullptr : masks.labels.data());
     };
 
+    // colour: the first decoded frame tells the channel count, which the background must have; checked before the
+    // operators are built
+    auto take_channels = [&](int ch) {
+        if (!color)
+            return;
+        CVVP_ASSERT_MSG(hp.background.channels == ch && bg.ndim() == 3,
+                        "kwargs['cvvp_color']: the background must be (h, w, C) with the channel count of the decoded "
+                        "frames");
+        hp.channels = ch;
+    };
     const std::vector<int> devices = device_list();
     if (rolling)
         hp.device = devices.front();
@@ -893,8 +923,10 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
             hp.queue_depth = depth;
             hp.max_batch = batch_frames;
             hp.source = vid.format_for(r, c, ch);
-            CVVP_ASSERT_MSG(hp.source.out_channels() == 1, "TrackObjects needs single-channel frames: set grayscale or "
-                                                           "vid_is_grayscale (cv::findContours requires 8UC1)");
+            take_channels(ch);
+            CVVP_ASSERT_MSG(hp.source.out_channels() == hp.channels,
+                            "TrackObjects needs single-channel frames: set grayscale or "
+                            "vid_is_grayscale (cv::findContours requires 8UC1)");
             std::vector<std::unique_ptr<GpuHighlightAlgo>> lanes; // one operator (context + queue) per device
             for (int d : devices) {
                 GpuHighlightPack lp = hp;
@@ -1045,9 +1077,12 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
                 if (device_prep) {
                     CVVP_ASSERT(r == fh && c == fw);
                     hp.source = vid.format_for(r, c, ch);
-                    CVVP_ASSERT_MSG(hp.source.out_channels() == 1,
+                    take_channels(ch);
+                    CVVP_ASSERT_MSG(hp.source.out_channels() == hp.channels,
                                     "TrackObjects needs single-channel frames: set grayscale or vid_is_grayscale "
                                     "(cv::findContours requires 8UC1)");
+                } else {
+                    take_channels(ch);
                 }
                 if (rolling)
                     roller = std::make_unique<GpuRollingHighlightAlgo>(std::move(hp), roll_window, roll_percent);
@@ -1062,8 +1097,8 @@ py::dict TrackObjects(const VidObjectTrackPack &pack)
                 batch->data.reserve(std::size_t(std::min(batch_frames, num_frames - consumed)) * r * c * ch);
             }
             if (!device_prep) {
-                CVVP_ASSERT_MSG(ch == 1, "TrackObjects needs single-channel frames: set grayscale or vid_is_grayscale "
-                                         "(cv::findContours requires 8UC1)");
+                CVVP_ASSERT_MSG(ch == hp.channels, "TrackObjects needs single-channel frames: set grayscale or "
+                                                   "vid_is_grayscale (cv::findContours requires 8UC1)");
                 CVVP_ASSERT(r == crop.height && c == crop.width);
             }
             CVVP_ASSERT(r == batch->rows && c == batch->cols && ch == batch->channels);

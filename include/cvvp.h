@@ -274,6 +274,29 @@ CVVP_API int cvvp_highlight_set_polarity(cvvp_ctx *ctx, int polarity);
 /* the context's polarity (CVVP_POLARITY_DARK unless set), or CVVP_ERR_INVALID for a NULL context */
 CVVP_API int cvvp_highlight_polarity(const cvvp_ctx *ctx);
 
+/* Colour frames (no counterpart in the reference, whose highlight stage takes 8UC1 frames only).  A job of C channels
+ * (1..4) takes frames and backgrounds of width*height*C interleaved bytes, and its difference image is the largest
+ * per-channel difference of the polarity:
+ *     d(x, y) = max over c of d_c,   d_c = the polarity's d of channel c of the background and of the frame
+ * so the thresholds stay grey levels of one channel.  Everything after d is unchanged, and C = 1 is the grey job.
+ * The channel count is a setting of the context, like the polarity: a highlight job takes it in cvvp_highlight_begin.
+ * With C > 1:
+ *   - the background of cvvp_highlight_begin is width*height*C bytes;
+ *   - frames of cvvp_highlight_frames*, cvvp_highlight_device*, of the queue and of the rolling stream without a frame
+ *     format are width*height*C bytes each, and every frame stride (and cvvp_highlight_device_bg's backgrounds and
+ *     bg_stride) is at least that;
+ *   - a frame format of the queue or of the rolling stream must be CVVP_FRAMES_AS_IS with src_channels == C
+ *     (CVVP_ERR_INVALID otherwise);
+ *   - the slots of cvvp_highlight_slot_acquire hold width*height*C bytes per frame (without a frame format);
+ *   - the device forms return CVVP_ERR_INVALID when d_out overlaps the frames or the backgrounds (d is computed
+ *     ahead of the masks, in chunks);
+ *   - masks, components, labels and records are unchanged: one byte (0 / 255) per pixel, and the statistics' d is
+ *     the d above.
+ * set: CVVP_ERR_INVALID outside 1..4 or for a NULL context, CVVP_ERR_STATE while a highlight job is open on the
+ * context.  get: the context's channel count (1 unless set), or CVVP_ERR_INVALID for a NULL context. */
+CVVP_API int cvvp_highlight_set_channels(cvvp_ctx *ctx, int channels);
+CVVP_API int cvvp_highlight_channels(const cvvp_ctx *ctx);
+
 /* ---------------------------------------------------------------------------------------------
  * components of the highlight masks (opt-in) -- the connected-component labelling that feeds the
  * object tracker.  In the reference this happens on the host inside the user's tracker callback,
